@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — scan-to-map registrations/s on B200 (BASELINE.json metric), one JSON line on stdout.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload cfg3|cfg3_leaf04|cfg1]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload cfg3|cfg3_leaf04|cfg1] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one scan-to-map registration (liogpu_scan2map: the whole Gauss-Newton loop of
@@ -24,6 +24,9 @@ Extra records in the same line (north_star's other configurations; each names it
 `cpu_baseline` (rank 0, N = 1): the CPU restatement of the reference path on the host cores — KD-tree build included
            (the reference rebuilds it every scan, mapOptmization.cpp:1846) and excluded, at numberOfCores 4 / 12 / all.
 --impl reference : that CPU path alone, same workload and sweeps, all host cores; rank 0 only.
+--dump-outputs DIR : after the timed steps, what the last one returned (pose, matP, the LM loop's results; rank 0) as
+           DIR/<name>.npy.  The sweeps, map and guesses are seeded, so two builds run with the same arguments can be
+           compared output for output.
 """
 from __future__ import annotations
 
@@ -191,6 +194,23 @@ def cpu_baseline_run(name: str, map4, scans, guesses, steps: int, warmup: int, c
 
 
 # ------------------------------------------------------------------------------------------------ GPU arm pieces
+# what liogpu_scan2map returns to its caller, without the timings and the kernels' own search statistics, so that two
+# builds can be compared output for output
+DUMP_INFO = ("status", "n_query", "iterations", "converged", "n_sel", "is_degenerate", "tie_queries", "delta_r", "delta_t",
+             "JtJ", "Jtr", "pose_hist", "nsel_hist")
+
+
+def dump_outputs(out_dir, pose, P, info):
+    """one registration's results as out_dir/<name>.npy: float32 arrays as they are, everything else as float64,
+    scalars as arrays of one element"""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"pose": pose, "matP": P}
+    arrays.update((k, info[k]) for k in DUMP_INFO)
+    for k, v in arrays.items():
+        v = np.atleast_1d(v)
+        np.save(os.path.join(out_dir, f"{k}.npy"), v if v.dtype == np.float32 else v.astype(np.float64))
+
+
 def bench_registration(torch, g, name, map4, scans, guesses, steps, warmup, flush, ext, local_rank, sampler=None):
     """-> dict with the device-resident and end-to-end numbers of one registration workload on this rank"""
     nqs = [int(sc.shape[0]) for sc in scans]
@@ -205,7 +225,7 @@ def bench_registration(torch, g, name, map4, scans, guesses, steps, warmup, flus
     g.set_local_map((dev_map.data_ptr(), map4.shape[0], 16))
 
     def step_device(k):
-        return g.scan2map((dev_scans[k].data_ptr(), nqs[k], 16), guesses[k], max_iter=MAX_ITER)[2]
+        return g.scan2map((dev_scans[k].data_ptr(), nqs[k], 16), guesses[k], max_iter=MAX_ITER)
 
     def step_host(k):
         return g.scan2map((host_recs[k].data_ptr(), nqs[k], 32), guesses[k], max_iter=MAX_ITER)[2]
@@ -222,8 +242,9 @@ def bench_registration(torch, g, name, map4, scans, guesses, steps, warmup, flus
         flush.fill_(s & 0xff)
         torch.cuda.synchronize()
         ev0.record(ext)
-        info = step_device(s % n_scans)
+        last = step_device(s % n_scans)
         ev1.record(ext)
+        info = last[2]
         ev1.synchronize()
         dev_ms.append(ev0.elapsed_time(ev1)); loop_ms.append(info["gpu_ms"]); iters.append(info["iterations"])
     launches = g.launch_count() - launches0
@@ -262,7 +283,7 @@ def bench_registration(torch, g, name, map4, scans, guesses, steps, warmup, flus
         idx_ms.append(1e3 * (time.perf_counter() - t0))
     return dict(dev_ms=dev_ms, loop_ms=loop_ms, iters=iters, e2e_ms=e2e_ms, launches=launches, nqs=nqs,
                 index_build_ms=float(np.median(idx_ms[1:])), dev_scans=dev_scans, kernel_launches=info["kernel_launches"],
-                pipe_ms=pipe_ms)
+                pipe_ms=pipe_ms, last=last)
 
 
 def profile_phases(torch, LioGpu, default_params, w, map4, dev_scans, nqs, guesses, flush, local_rank, n, **over):
@@ -533,7 +554,11 @@ def main():
     ap.add_argument("--seq-scans", type=int, default=200, help="sweeps per sequence of the cfg5 record")
     ap.add_argument("--seq-concurrency", type=int, default=0, help="sequences replayed concurrently per rank (0 = all of the rank's)")
     ap.add_argument("--only", default="", help="development: run only this extra record (cfg4 | cfg5) and print it")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write what the last timed registration returned (pose, matP, LM results) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "liogpu" or args.only):
+        ap.error("--dump-outputs writes the outputs of the GPU arm's headline workload")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world_size = int(os.environ.get("WORLD_SIZE", "1"))
@@ -547,9 +572,9 @@ def main():
     if args.impl == "reference":
         if rank != 0:
             return
-        # a step is one full CPU registration (~0.14 s on cfg3 with 16 threads): bounded so that the arm ends in
-        # well under a minute; at least 3 warm-up steps (the first parallel regions of a fresh process run slow)
-        steps = max(10, min(args.steps, 30))
+        # a step is one full CPU registration (~0.14 s on cfg3 with 16 threads); at least 3 warm-up steps (the first
+        # parallel regions of a fresh process run slow)
+        steps = args.steps
         warm = max(3, min(args.warmup, 10))
         map4, scans, guesses = make_workload(name, 0)
         cb = cpu_baseline_run(name, map4, scans, guesses, steps, warm)
@@ -611,6 +636,8 @@ def main():
     barrier()
     wall_s = time.perf_counter() - t_wall0
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *r["last"])
     kern = profile_phases(torch, LioGpu, default_params, w, map4, r["dev_scans"], r["nqs"], guesses, flush, local_rank,
                           min(args.steps, 16))
     ab = None

@@ -6,6 +6,9 @@
 2. path_small.npz : a small end-to-end case (scan, map, guess) with the oracle's outputs (VoxelGrid, one
    surfOptimization pass, the full scan2map loop).  These are ORACLE outputs, not reference outputs — the
    reference cannot be built here (parity unpinned); they guard the oracle and the CUDA path against drift.
+2b. cv2_live.npz : OpenCV's outputs (cv2) for the seeded random systems of tests/test_oracle_cv2.py
+   (test_live_cv2_random, test_normal_equations_match_cv_gemm) and for the 6x6 system of the PCL pinning kit's
+   inputs (tests/test_pcl_pin.py, pin_*), so that those comparisons run without cv2.
 3. rows_f_small.npz : the same for the widened rows (publishLocalMap, keyframe merging, loop-closure ICP, Scan
    Context, key-pose selection), again ORACLE outputs.
 """
@@ -51,6 +54,32 @@ def make_cv2():
             out[f"{name}_{k}"] = np.asarray(v)
     np.savez_compressed(os.path.join(HERE, "cv2_6x6.npz"), **out)
     print("cv2_6x6.npz:", len(cases), "cases, cv2", cv2.__version__)
+
+
+def make_cv2_live():
+    import cv2
+    sys.path.insert(0, os.path.dirname(HERE))
+    from test_oracle_cv2 import cv2_live_outputs, live_cases
+    from oracle.oracle import Oracle
+    out = {"cv2_version": np.array(cv2.__version__)}
+    for t, (A, b) in enumerate(live_cases()):
+        for name, v in cv2_live_outputs(cv2, A, b).items():
+            out[f"{name}_{t}"] = np.asarray(v)
+    rng = np.random.default_rng(1)          # the normal equations of test_normal_equations_match_cv_gemm
+    n = 5000
+    scan = rng.normal(0, 20, (n, 4)).astype(np.float32)
+    coeff = rng.normal(0, 1, (n, 4)).astype(np.float32)
+    flag = (rng.uniform(size=n) < 0.8).astype(np.uint8)
+    _, JtJ, Jtr = Oracle("port").normal_equations(scan, coeff, flag, np.array([0.01, -0.02, 0.5, 1, 2, 3], np.float32))
+    ok, X = cv2.solve(JtJ.astype(np.float32), Jtr.astype(np.float32).reshape(6, 1), flags=cv2.DECOMP_QR)
+    out.update(ne_JtJ=JtJ, ne_Jtr=Jtr, ne_ok=np.array(ok), ne_X=X[:, 0])
+    sys.path.insert(0, os.path.join(HERE, "pcl_pin"))
+    import lpin
+    inp = lpin.read(os.path.join(HERE, "pcl_pin", "pin_inputs.lpin"))
+    for name, v in cv2_live_outputs(cv2, inp["lm_A"], inp["lm_b"].reshape(-1, 1)).items():
+        out[f"pin_{name}"] = np.asarray(v)
+    np.savez_compressed(os.path.join(HERE, "cv2_live.npz"), **out)
+    print("cv2_live.npz: 60 systems, the normal equations and the pin kit's system, cv2", cv2.__version__)
 
 
 def make_path():

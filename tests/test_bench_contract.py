@@ -5,6 +5,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -22,7 +23,7 @@ def run_bench(*args, timeout=600):
 
 def test_reference_arm_line():
     d = run_bench("--impl", "reference", "--workload", "cfg1", "--steps", "1", "--warmup", "1")
-    assert BASE_KEYS <= set(d) and d["impl"] == "reference"
+    assert BASE_KEYS <= set(d) and d["impl"] == "reference" and d["steps"] == 1
     assert d["metric"] == "scan2map_registrations_per_sec" and d["unit"] == "registrations/s" and d["higher_is_better"] is True
     assert d["value"] > 0 and d["vs_baseline"] is None and d["data"] == "synthetic" and "workload" in d["config"]
     cb = d["cpu_baseline"]
@@ -48,3 +49,33 @@ def test_gpu_arm_line():
     cb = d["cpu_baseline"]
     assert cb["value"] > 0 and cb["cores"] >= 1 and cb["kind"] == "port"
     assert set(d["clocks"]) >= {"sm_mhz", "sm_max_mhz", "reasons"}
+
+
+@pytest.mark.gpu
+def test_gpu_arm_dump_outputs(tmp_path):
+    """--dump-outputs writes what the last timed registration returned: the same bytes from run to run, and the same
+    bytes as one registration of that sweep outside the bench"""
+    from bench import MAX_ITER, WORKLOADS, make_workload
+    from lio_slam_b200.liogpu import LioGpu, default_params
+    runs = []
+    for k in range(2):
+        out = tmp_path / f"run{k}"
+        d = run_bench("--workload", "cfg1", "--steps", "3", "--warmup", "1", "--no-extras", "--no-cpu-baseline",
+                      "--dump-outputs", str(out))
+        assert d["steps"] == 3
+        runs.append({f[:-4]: np.load(out / f) for f in os.listdir(out)})
+    a, b = runs
+    assert set(a) == {"pose", "matP", "status", "n_query", "iterations", "converged", "n_sel", "is_degenerate",
+                      "tie_queries", "delta_r", "delta_t", "JtJ", "Jtr", "pose_hist", "nsel_hist"}
+    assert sum(v.nbytes for v in a.values()) <= 64 << 20
+    for name, v in a.items():
+        assert v.dtype in (np.float32, np.float64), name
+        assert v.dtype == b[name].dtype and v.shape == b[name].shape and v.tobytes() == b[name].tobytes(), name
+    w = WORKLOADS["cfg1"]
+    map4, scans, guesses = make_workload("cfg1", 0)
+    g = LioGpu(default_params(n_scan=w["beams"], horizon_scan=w["cols"], surrounding_keyframe_map_leaf_size=w["map_leaf"]))
+    g.set_local_map(map4)
+    pose, P, info = g.scan2map(scans[2], guesses[2], max_iter=MAX_ITER)   # step 2 of 3 registers sweep 2
+    g.close()
+    assert np.array_equal(pose.view(np.uint32), a["pose"].view(np.uint32)) and np.array_equal(P, a["matP"])
+    assert a["iterations"].tolist() == [info["iterations"]] and np.array_equal(a["pose_hist"], info["pose_hist"])

@@ -49,30 +49,60 @@ def test_normal_equations_match_cv_gemm(oracle):
     nsel, JtJ, Jtr = oracle.normal_equations(scan, coeff, flag, pose)
     assert nsel == int(flag.sum())
     assert np.allclose(JtJ, JtJ.T, rtol=0, atol=0)
+    # JtJ = At*A cannot be rebuilt without the rows: check symmetry + a round trip through cv::solve(QR), against the
+    # outputs make_golden.py stored and, when cv2 is importable, against the library itself
+    L = np.load(os.path.join(os.path.dirname(__file__), "golden", "cv2_live.npz"))
+    assert np.array_equal(JtJ, L["ne_JtJ"]) and np.array_equal(Jtr, L["ne_Jtr"])
+    wants = [(bool(L["ne_ok"]), L["ne_X"])]
+    cv2 = import_cv2()
+    if cv2 is not None:
+        ok, X = cv2.solve(JtJ.astype(np.float32), Jtr.astype(np.float32).reshape(6, 1), flags=cv2.DECOMP_QR)
+        wants.append((ok, X[:, 0]))
+    ok2, X2 = oracle.cv_solve6_qr(JtJ.astype(np.float32), Jtr.astype(np.float32))
+    for ok, X in wants:
+        assert ok == ok2 and biteq(X, X2)
+
+
+def import_cv2():
     try:
         import cv2
+        return cv2
     except ImportError:
-        pytest.skip("cv2 not importable")
-    # rebuild matA / matB exactly as LMOptimization does, through the oracle's own Jacobian rows: JtJ = At*A
-    # cannot be rebuilt without the rows, so check symmetry + a cv2 solve round trip instead
-    ok, X = cv2.solve(JtJ.astype(np.float32), Jtr.astype(np.float32).reshape(6, 1), flags=cv2.DECOMP_QR)
-    ok2, X2 = oracle.cv_solve6_qr(JtJ.astype(np.float32), Jtr.astype(np.float32))
-    assert ok == ok2 and biteq(X[:, 0], X2)
+        return None
 
 
-def test_live_cv2_random(oracle):
-    cv2 = pytest.importorskip("cv2")
+def live_cases():
+    """the seeded systems of test_live_cv2_random (tests/golden/make_golden.py stores OpenCV's outputs for them)"""
     rng = np.random.default_rng(77)
     for t in range(60):
         n = int(rng.integers(60, 2000))
         A = (rng.normal(size=(n, 6)) * rng.uniform(0.05, 20, size=6)).astype(np.float32)
-        AtA = cv2.gemm(np.ascontiguousarray(A.T), A, 1.0, None, 0.0)
-        Atb = cv2.gemm(np.ascontiguousarray(A.T), rng.normal(size=(n, 1)).astype(np.float32), 1.0, None, 0.0)
-        ok, X = cv2.solve(AtA, Atb, flags=cv2.DECOMP_QR)
-        ok2, X2 = oracle.cv_solve6_qr(AtA, Atb[:, 0])
-        assert ok == ok2 and biteq(X[:, 0], X2)
-        _, E, V = cv2.eigen(AtA)
-        W2, V2 = oracle.cv_eigen6(AtA)
-        assert biteq(E[:, 0], W2) and biteq(V, V2)
-        _, Vi = cv2.invert(V, flags=cv2.DECOMP_LU)
-        assert biteq(Vi, oracle.cv_inv6(V)[1])
+        yield A, rng.normal(size=(n, 1)).astype(np.float32)
+
+
+def cv2_live_outputs(cv2, A, b):
+    AtA = cv2.gemm(np.ascontiguousarray(A.T), A, 1.0, None, 0.0)
+    Atb = cv2.gemm(np.ascontiguousarray(A.T), b, 1.0, None, 0.0)
+    ok, X = cv2.solve(AtA, Atb, flags=cv2.DECOMP_QR)
+    _, E, V = cv2.eigen(AtA)
+    _, Vi = cv2.invert(V, flags=cv2.DECOMP_LU)
+    return dict(AtA=AtA, Atb=Atb[:, 0], ok=ok, X=X[:, 0], E=E[:, 0], V=V, Vi=Vi)
+
+
+def test_live_cv2_random(oracle):
+    """the oracle against OpenCV on 60 seeded random systems: against the outputs make_golden.py stored
+    (cv2_live.npz) and, when cv2 is importable, against the library itself"""
+    L = np.load(os.path.join(os.path.dirname(__file__), "golden", "cv2_live.npz"))
+    cv2 = import_cv2()
+    for t, (A, b) in enumerate(live_cases()):
+        AtA = (A.astype(np.float64).T @ A.astype(np.float64)).astype(np.float32)
+        assert biteq(AtA, L[f"AtA_{t}"]), t                   # the stored outputs belong to these inputs
+        wants = [{k: L[f"{k}_{t}"] for k in ("AtA", "Atb", "ok", "X", "E", "V", "Vi")}]
+        if cv2 is not None:
+            wants.append(cv2_live_outputs(cv2, A, b))
+        for w in wants:
+            ok2, X2 = oracle.cv_solve6_qr(w["AtA"], w["Atb"])
+            assert bool(w["ok"]) == ok2 and biteq(w["X"], X2)
+            W2, V2 = oracle.cv_eigen6(w["AtA"])
+            assert biteq(w["E"], W2) and biteq(w["V"], V2)
+            assert biteq(w["Vi"], oracle.cv_inv6(w["V"])[1])

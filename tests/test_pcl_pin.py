@@ -110,9 +110,15 @@ def test_icp_matches_pcl(oracle, pin):
     assert abs(r["fitness_score"] - out["icp_meta"][1]) <= 1e-6 * max(1.0, out["icp_meta"][1])
 
 
-@pinned
-def test_opencv_6x6_pieces_match_opencv_cpp(oracle, pin):
-    inp, out = pin
+def test_opencv_6x6_pieces_match_opencv_cpp(oracle):
+    """the kit's fixture when it is present, else OpenCV's outputs for the same system stored by
+    tests/golden/make_golden.py (Python cv2 calls the same cv::gemm / cv::solve / cv::eigen / cv::invert)"""
+    inp = lpin.read(INP)
+    if os.path.exists(OUT):
+        out = lpin.read(OUT)
+    else:
+        G = np.load(os.path.join(HERE, "golden", "cv2_live.npz"))
+        out = {"cv_AtA": G["pin_AtA"], "cv_x": G["pin_X"], "cv_E": G["pin_E"], "cv_V": G["pin_V"], "cv_Vinv": G["pin_Vi"]}
     A, b = inp["lm_A"], inp["lm_b"]
     AtA = (A.astype(np.float64).T @ A.astype(np.float64)).astype(np.float32)   # what oracle::normal_equations computes
     assert np.array_equal(bits(AtA), bits(out["cv_AtA"])), "AtA differs from cv::gemm (f64 accumulation rounded once)"
