@@ -295,6 +295,68 @@ int liogpu_make_scancontext(liogpu_ctx* ctx, const void* xyzi, int n, int stride
                             double max_radius, double desc[LIOGPU_SC_NUM_RING * LIOGPU_SC_NUM_SECTOR],
                             double ringkey[LIOGPU_SC_NUM_RING], double sectorkey[LIOGPU_SC_NUM_SECTOR]);
 
+/* ---- loop-closure detection (SURVEY §8 row f3): SCManager::detectLoopClosureID (include/Scancontext.cpp) over a
+ * descriptor store kept in the context, and the key-pose radius detector detectLoopClosureDistance (MO ~1271-1300).
+ * SCManager's constants (include/Scancontext.h); defaults by liogpu_default_sc_params are SC-LIO-SAM's Scancontext.h,
+ * which liorf vendors: NUM_EXCLUDE_RECENT 30, NUM_CANDIDATES_FROM_TREE 3, TREE_MAKING_PERIOD_ 30, SEARCH_RATIO 0.1,
+ * SC_DIST_THRES 0.2 (and historyKeyframeSearchTimeDiff 30.0 in utility.h for the radius detector).  They are taken
+ * from the public sources as remembered, not checked against the reference tree. */
+#define LIOGPU_SC_MAX_CANDIDATES 32
+typedef struct liogpu_sc_params {
+  int    num_exclude_recent;        /* NUM_EXCLUDE_RECENT        (>= 0)      */
+  int    num_candidates_from_tree;  /* NUM_CANDIDATES_FROM_TREE  (1..LIOGPU_SC_MAX_CANDIDATES) */
+  int    tree_making_period;        /* TREE_MAKING_PERIOD_       (>= 1)      */
+  double search_ratio;              /* SEARCH_RATIO              (0, 1]      */
+  double sc_dist_thres;             /* SC_DIST_THRES                         */
+  int    reserved[4];
+} liogpu_sc_params;
+
+typedef struct liogpu_sc_info {     /* everything detectLoopClosureID computes on the way */
+  int    n_stored, n_searchable;    /* polarcontexts_.size(), size of the tree's snapshot */
+  int    tree_rebuilt;              /* this call rebuilt the snapshot (counter % period == 0) */
+  int    n_candidates;              /* min(num_candidates_from_tree, n_searchable) */
+  int    candidates[LIOGPU_SC_MAX_CANDIDATES];        /* kNN order */
+  float  candidate_key_d2[LIOGPU_SC_MAX_CANDIDATES];  /* ring-key distance, nanoflann L2 (f32) */
+  double candidate_dist[LIOGPU_SC_MAX_CANDIDATES];    /* distanceBtnScanContext().first */
+  int    candidate_shift[LIOGPU_SC_MAX_CANDIDATES];   /* ... .second */
+  int    nn_idx, nn_align;          /* best candidate and its shift, also when it is not a loop (-1 / 0 when the
+                                       call returned early) */
+  double min_dist;                  /* 1e7 (the reference's initial value) when nothing was scored */
+  int    knn_ties;                  /* ring-key distances equal across the k-th boundary or inside the set */
+  float  gpu_ms;
+  int    reserved[4];
+} liogpu_sc_info;
+
+void liogpu_default_sc_params(liogpu_sc_params* p);
+/* polarcontexts_ / invkeys / vkeys .push_back (makeAndSaveScancontextAndKeys, Scancontext.cpp:228-243) for n
+ * descriptors as liogpu_make_scancontext returns them (row-major [ring][sector], f64, 1200 each; host or device memory).
+ * The keys are derived on the device with the same code as liogpu_make_scancontext, so they are bit-equal to the ones it
+ * returns. */
+int liogpu_sc_add(liogpu_ctx* ctx, const double* descs, int n);
+/* drop every stored descriptor and reset the tree counter (a fresh SCManager); liogpu_keyframe_clear does not touch the
+ * store */
+int liogpu_sc_clear(liogpu_ctx* ctx);
+/* SCManager::detectLoopClosureID on the newest stored descriptor, with the reference's tree-snapshot state kept in the
+ * context.  loop_id = -1 when there is no loop; yaw_diff_rad as the reference returns it; info may be NULL.  With fewer
+ * than num_exclude_recent + 1 stored descriptors: LIOGPU_OK, loop_id = -1, yaw 0, counter not advanced (the reference's
+ * early return).  Candidates are the exact k nearest ring keys of the snapshot in (distance, index) order; the
+ * reference's KD-tree may order equal distances differently (counted in knn_ties). */
+int liogpu_sc_detect_loop(liogpu_ctx* ctx, const liogpu_sc_params* p, int* loop_id, float* yaw_diff_rad,
+                          liogpu_sc_info* info);
+/* Offline: the results of n_calls detectLoopClosureID calls of a FRESH SCManager (counter 0) made when it held
+ * store_sizes[j] descriptors (non-decreasing, each <= the stored count).  Bit-equal to clearing a store, adding the
+ * same descriptors and calling liogpu_sc_detect_loop at those sizes.  Does not change the context's online counter.
+ * yaw_diff_rad and min_dist may be NULL. */
+int liogpu_sc_detect_loops(liogpu_ctx* ctx, const liogpu_sc_params* p, const int* store_sizes, int n_calls,
+                           int* loop_ids, float* yaw_diff_rad, double* min_dist);
+/* detectLoopClosureDistance (MO ~1271-1300) minus the loopIndexContainer check, which stays with the caller:
+ * among the key poses strictly within search_radius of the newest one (FLANN: d2 < (float)(r*r), sorted by
+ * distance, ties by lower index), the first whose |time - time_laser_info_cur| > time_diff; -1 if none or if it
+ * is the newest itself.  Same key-pose / time arguments as liogpu_extract_nearby. */
+int liogpu_detect_loop_distance(liogpu_ctx* ctx, const void* key_poses3d, int n_key, int stride3d,
+                                const void* key_times, int time_stride, double time_laser_info_cur,
+                                float search_radius, float time_diff, int* loop_key_pre);
+
 /* ---- key-pose selection (SURVEY §8 row f4): extractNearby (MO:1519-1554) + the guard of extractCloud (MO:1562).
  * key_poses3d = cloudKeyPoses3D->points (x, y, z, intensity = keyframe index; n_key records of stride3d bytes),
  * key_times = the `time` field of cloudKeyPoses6D->points (n_key doubles, time_stride bytes apart: 8 for a plain

@@ -236,7 +236,8 @@ int liogpu_create(liogpu_ctx** out, const liogpu_params* params) {
                       &c.fail_buf, &c.prev_nn, &c.hopeless, &c.fz_rows, &c.fz_left, &c.fz_lb, &c.fz_probe, &c.tile_plan,
                       &c.tile_hist, &c.tile_pts, &c.tile_out, &c.dbg_idx, &c.dbg_d2, &c.dbg_coeff, &c.dbg_flag, &c.dbg_tie,
                       &c.imu_tab, &c.dsk_flags, &c.dsk_scan, &c.lm_flag, &c.lm_pos, &c.lm_a, &c.lm_b, &c.lm_md, &c.lm_left,
-                      &c.lm_out, &c.lm_stats, &c.sor_setup, &c.sor_sorted, &c.sor_cell_start, &c.kf_tab};
+                      &c.lm_out, &c.lm_stats, &c.sor_setup, &c.sor_sorted, &c.sor_cell_start, &c.kf_tab,
+                      &c.sc_q, &c.sc_part, &c.sc_cand, &c.sc_out};
     for (DevBuf* b : bufs) { b->stream = c.stream; b->async = true; }
   }
   // scratch hint of allocateMemory (mapOptmization.cpp:333-335)
@@ -263,8 +264,9 @@ void liogpu_destroy(liogpu_ctx* ctx) {
                     &c.vox_setup, &c.grid_setup, &c.minmax, &c.lm_state, &c.partials, &c.block_counter, &c.misc,
                     &c.fail_buf, &c.prev_nn, &c.hopeless, &c.fz_rows, &c.fz_left, &c.fz_lb, &c.fz_probe, &c.tile_plan, &c.tile_hist, &c.tile_pts, &c.tile_out, &c.dbg_idx, &c.dbg_d2, &c.dbg_coeff, &c.dbg_flag, &c.dbg_tie, &c.imu_tab, &c.dsk_flags, &c.dsk_scan,
                     &c.lm_flag, &c.lm_pos, &c.lm_a, &c.lm_b, &c.lm_md, &c.lm_left, &c.lm_out, &c.lm_stats, &c.sor_setup,
-                    &c.sor_sorted, &c.sor_cell_start};
+                    &c.sor_sorted, &c.sor_cell_start, &c.sc_q, &c.sc_part, &c.sc_cand, &c.sc_out};
   for (DevBuf* b : bufs) b->release();
+  sc_release(&c);
   for (auto& kv : c.keyframes) kv.second.first.release();
   for (void* slab : c.kf_slabs) cudaFree(slab);
   if (c.h_pinned) cudaFreeHost(c.h_pinned);
@@ -747,6 +749,146 @@ int liogpu_extract_nearby(liogpu_ctx* ctx, const void* key_poses3d, int n_key, i
   for (int i = 0; i < n_key; ++i) std::memcpy(&times[i], (const char*)key_times + (size_t)i * time_stride, sizeof(double));
   return extract_nearby_dev(c, c->lm_a.as<float4>(), n_key, times.data(), time_laser_info_cur, search_radius, density_leaf,
                             ids_out, cap_ids, n_ids);
+}
+
+void liogpu_default_sc_params(liogpu_sc_params* p) {
+  if (!p) return;
+  std::memset(p, 0, sizeof(*p));
+  p->num_exclude_recent = 30;        // Scancontext.h: NUM_EXCLUDE_RECENT
+  p->num_candidates_from_tree = 3;   // NUM_CANDIDATES_FROM_TREE
+  p->tree_making_period = 30;        // TREE_MAKING_PERIOD_
+  p->search_ratio = 0.1;             // SEARCH_RATIO
+  p->sc_dist_thres = 0.2;            // SC_DIST_THRES
+}
+
+int liogpu_sc_add(liogpu_ctx* ctx, const double* descs, int n) {
+  NvtxRange nvtx_range_(__func__);
+  int rc = enter(ctx);
+  if (rc) return rc;
+  Ctx* c = &ctx->c;
+  if (!descs || n <= 0 || (long long)c->sc.count + n > 0x7fffffffLL) { c->err = "liogpu_sc_add: bad arguments"; return LIOGPU_E_INVALID; }
+  return sc_add_dev(c, descs, n);
+}
+
+int liogpu_sc_clear(liogpu_ctx* ctx) {
+  NvtxRange nvtx_range_(__func__);
+  int rc = enter(ctx);
+  if (rc) return rc;
+  Ctx* c = &ctx->c;
+  c->sc.count = 0;  // the arrays stay with the context and are filled again (freeing would synchronise the device)
+  c->sc.counter = 0;
+  c->sc.snap = 0;
+  c->last_ms = 0.f;
+  return LIOGPU_OK;
+}
+
+static bool sc_params_ok(const liogpu_sc_params* p) {
+  return p && p->num_exclude_recent >= 0 && p->num_candidates_from_tree >= 1 &&
+         p->num_candidates_from_tree <= LIOGPU_SC_MAX_CANDIDATES && p->tree_making_period >= 1 && p->search_ratio > 0.0 &&
+         p->search_ratio <= 1.0 && !std::isnan(p->sc_dist_thres);
+}
+static int sc_search_radius(const liogpu_sc_params* p) {  // SEARCH_RADIUS = round(0.5 * SEARCH_RATIO * cols)
+  return (int)std::round(0.5 * p->search_ratio * LIOGPU_SC_NUM_SECTOR);
+}
+
+int liogpu_sc_detect_loop(liogpu_ctx* ctx, const liogpu_sc_params* p, int* loop_id, float* yaw_diff_rad, liogpu_sc_info* info) {
+  NvtxRange nvtx_range_(__func__);
+  int rc = enter(ctx);
+  if (rc) return rc;
+  Ctx* c = &ctx->c;
+  if (!sc_params_ok(p) || !loop_id || !yaw_diff_rad) { c->err = "liogpu_sc_detect_loop: bad arguments"; return LIOGPU_E_INVALID; }
+  liogpu_sc_info local_info;
+  if (!info) info = &local_info;
+  std::memset(info, 0, sizeof(*info));
+  ScStore& st = c->sc;
+  info->n_stored = st.count;
+  info->nn_idx = -1;
+  info->min_dist = 10000000.0;
+  *loop_id = -1;
+  *yaw_diff_rad = 0.f;
+  c->last_ms = 0.f;
+  if (st.count < p->num_exclude_recent + 1) {  // early return: the counter does not advance
+    info->n_searchable = st.snap;
+    return LIOGPU_OK;
+  }
+  const bool rebuild = st.counter % p->tree_making_period == 0;
+  const int snap = rebuild ? st.count - p->num_exclude_recent : st.snap;
+  std::vector<int2> qm(1, make_int2(st.count - 1, snap));
+  ScQueryOut out;
+  rc = sc_detect_dev(c, qm, p->num_candidates_from_tree, sc_search_radius(p), p->sc_dist_thres, &out, info);
+  if (rc) return rc;
+  st.snap = snap;
+  st.counter++;
+  info->n_searchable = snap;
+  info->tree_rebuilt = rebuild ? 1 : 0;
+  info->n_candidates = out.n_cand;
+  info->nn_idx = out.nn_idx;
+  info->nn_align = out.nn_align;
+  info->min_dist = out.min_dist;
+  info->knn_ties = out.ties;
+  info->gpu_ms = c->last_ms;
+  *loop_id = out.loop_id;
+  *yaw_diff_rad = out.yaw;
+  return LIOGPU_OK;
+}
+
+int liogpu_sc_detect_loops(liogpu_ctx* ctx, const liogpu_sc_params* p, const int* store_sizes, int n_calls, int* loop_ids,
+                           float* yaw_diff_rad, double* min_dist) {
+  NvtxRange nvtx_range_(__func__);
+  int rc = enter(ctx);
+  if (rc) return rc;
+  Ctx* c = &ctx->c;
+  bool ok = sc_params_ok(p) && store_sizes && loop_ids && n_calls > 0;
+  for (int j = 0; ok && j < n_calls; ++j)
+    ok = store_sizes[j] >= 0 && store_sizes[j] <= c->sc.count && (j == 0 || store_sizes[j] >= store_sizes[j - 1]);
+  if (!ok) { c->err = "liogpu_sc_detect_loops: bad arguments"; return LIOGPU_E_INVALID; }
+  // the snapshot schedule of a fresh SCManager: which calls search, and over which prefix
+  std::vector<int2> qm;
+  std::vector<int> slot((size_t)n_calls, -1);
+  long long counter = 0;
+  int snap = 0;
+  for (int j = 0; j < n_calls; ++j) {
+    const int size = store_sizes[j];
+    if (size < p->num_exclude_recent + 1) continue;  // early return, counter untouched
+    if (counter % p->tree_making_period == 0) snap = size - p->num_exclude_recent;
+    ++counter;
+    slot[j] = (int)qm.size();
+    qm.push_back(make_int2(size - 1, snap));
+  }
+  std::vector<ScQueryOut> out(qm.size());
+  c->last_ms = 0.f;
+  if (!qm.empty()) {
+    rc = sc_detect_dev(c, qm, p->num_candidates_from_tree, sc_search_radius(p), p->sc_dist_thres, out.data(), nullptr);
+    if (rc) return rc;
+  }
+  for (int j = 0; j < n_calls; ++j) {
+    const int s = slot[j];
+    loop_ids[j] = s < 0 ? -1 : out[s].loop_id;
+    if (yaw_diff_rad) yaw_diff_rad[j] = s < 0 ? 0.f : out[s].yaw;
+    if (min_dist) min_dist[j] = s < 0 ? 10000000.0 : out[s].min_dist;
+  }
+  return LIOGPU_OK;
+}
+
+int liogpu_detect_loop_distance(liogpu_ctx* ctx, const void* key_poses3d, int n_key, int stride3d, const void* key_times,
+                                int time_stride, double time_laser_info_cur, float search_radius, float time_diff,
+                                int* loop_key_pre) {
+  NvtxRange nvtx_range_(__func__);
+  int rc = enter(ctx);
+  if (rc) return rc;
+  Ctx* c = &ctx->c;
+  if (!loop_key_pre || n_key <= 0 || !key_poses3d || !key_times || time_stride < 8 || !(search_radius > 0.f) ||
+      std::isnan(time_diff) || key_poses3d == LIOGPU_DEVICE_RESIDENT || key_poses3d == LIOGPU_UPLOADED_SCAN || !stride_ok(stride3d)) {
+    c->err = "liogpu_detect_loop_distance: bad arguments";
+    return LIOGPU_E_INVALID;
+  }
+  *loop_key_pre = -1;
+  rc = load_cloud(c, key_poses3d, n_key, stride3d, c->lm_a);  // the key-pose upload of liogpu_extract_nearby
+  if (rc) return rc;
+  std::vector<double> times((size_t)n_key);
+  for (int i = 0; i < n_key; ++i) std::memcpy(&times[i], (const char*)key_times + (size_t)i * time_stride, sizeof(double));
+  return detect_loop_distance_dev(c, c->lm_a.as<float4>(), n_key, times.data(), time_laser_info_cur, search_radius, time_diff,
+                                  loop_key_pre);
 }
 
 int liogpu_set_local_map(liogpu_ctx* ctx, const void* xyzi, int n, int stride) {

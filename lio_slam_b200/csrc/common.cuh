@@ -107,6 +107,26 @@ struct LmDevState {
   int main_finalized_iter;  // two-kernel path: value of `iter` after the main kernel's last block ran the tail itself
 };
 
+// ---- loop-closure detection (loopdetect.cu) ----
+// SCManager's descriptor store (polarcontexts_ and its keys), one entry per liogpu_sc_add-ed descriptor: the f64
+// descriptor [SC_BINS], the f32 ring key [20], the f64 sector key [60] and the f64 column norms [60], in four arrays of
+// `cap` entries.  Grows geometrically (stream-ordered, contents carried over); emptied but kept by liogpu_sc_clear.
+struct ScStore {
+  double* desc = nullptr;
+  float* rkey = nullptr;
+  double* vkey = nullptr;
+  double* cnorm = nullptr;
+  int count = 0, cap = 0;
+  long long counter = 0;  // tree_making_period_conter
+  int snap = 0;           // size of the tree's snapshot (a prefix of the store)
+};
+// result of one detectLoopClosureID query, as the device leaves it
+struct ScQueryOut {
+  int n_cand, ties, nn_idx, nn_align, loop_id;
+  float yaw;
+  double min_dist;
+};
+
 // host-visible context
 struct Ctx {
   liogpu_params prm;
@@ -169,6 +189,9 @@ struct Ctx {
   cudaStream_t copy_stream = nullptr;
   struct Upload { DevBuf raw; cudaEvent_t ev = nullptr; int n = 0, stride = 0; bool valid = false; } upload[2];
   int upload_head = 0, upload_count = 0;  // FIFO: a consumer takes the OLDEST pending upload
+  // loop-closure detection: the descriptor store and the per-call scratch (queries, partial top-k lists, candidates)
+  ScStore sc;
+  DevBuf sc_q, sc_part, sc_cand, sc_out;
 };
 
 #define LIOGPU_CUDA_OK(ctx, expr)                                                        \
@@ -211,6 +234,12 @@ int extract_nearby_dev(Ctx* c, const float4* key3d, int n, const double* h_times
                        float density, int* ids, int cap, int* n_ids);
 // --- scancontext.cu
 int scancontext_dev(Ctx* c, const float4* pts, int n, double lidar_height, double max_radius, double* h_out);
+// --- loopdetect.cu
+int sc_add_dev(Ctx* c, const double* descs, int n);
+void sc_release(Ctx* c);
+int sc_detect_dev(Ctx* c, const std::vector<int2>& qm, int k, int R, double thres, ScQueryOut* h_out, liogpu_sc_info* info);
+int detect_loop_distance_dev(Ctx* c, const float4* key3d, int n, const double* h_times, double time_cur, float radius,
+                             float time_diff, int* loop_key_pre);
 // --- icp.cu
 int icp_align_dev(Ctx* c, const float4* src, int ns, const float4* tgt, int nt, const liogpu_icp_params* prm,
                   float final_T[16], liogpu_icp_info* info);

@@ -6,15 +6,13 @@
 // f32, f64 ceil), height z + LIDAR_HEIGHT narrowed to f32, atomicMax on an order-preserving integer image of the
 // float into a 20 x 60 table in shared memory, one global atomicMax per occupied bin and block.  A one-block
 // epilogue kernel turns the table into doubles (empty bins -> 0) and forms the row / column means.
-#include "common.cuh"
+#include "scancontext.cuh"
 
 #include <math_constants.h>
 
 namespace liogpu {
 
 namespace {
-
-constexpr int SC_RING = LIOGPU_SC_NUM_RING, SC_SECTOR = LIOGPU_SC_NUM_SECTOR, SC_BINS = SC_RING * SC_SECTOR;
 
 __device__ __forceinline__ unsigned sc_f2ord(float f) {
   const unsigned u = __float_as_uint(f);
@@ -74,16 +72,7 @@ sc_keys_kernel(const unsigned* __restrict__ table, double* __restrict__ out) {
   }
   __syncthreads();
   const int k = threadIdx.x;
-  if (k < SC_RING) {
-    double s = 0.0;
-    for (int c = 0; c < SC_SECTOR; ++c) s += d[k * SC_SECTOR + c];
-    out[SC_BINS + k] = s / SC_SECTOR;
-  } else if (k < SC_RING + SC_SECTOR) {
-    const int c = k - SC_RING;
-    double s = 0.0;
-    for (int r = 0; r < SC_RING; ++r) s += d[r * SC_SECTOR + c];
-    out[SC_BINS + SC_RING + c] = s / SC_RING;
-  }
+  if (k < SC_RING + SC_SECTOR) out[SC_BINS + k] = sc_key(d, k);
 }
 
 }  // namespace

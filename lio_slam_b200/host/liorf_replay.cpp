@@ -44,7 +44,9 @@ extern "C" void liorf_worker_destroy(liorf_worker* w) {
 extern "C" int liorf_worker_replay(liorf_worker* w, const liorf_replay_options* options, const liorf_sweep* sweeps, int n,
                                    float* poses_out, int* iters_out, int* nds_out, liorf_replay_stats* stats, char* err, int err_len) {
   if (!w) return LIOGPU_E_INVALID;
-  const int rc = liogpu_keyframe_clear(w->ctx);  // a new sequence starts with an empty map
+  int rc = liogpu_keyframe_clear(w->ctx);  // a new sequence starts with an empty map
+  if (rc < 0) return rc;
+  rc = liogpu_sc_clear(w->ctx);            // ... and a fresh SCManager
   if (rc < 0) return rc;
   return replay_impl(&w->params, w->ctx, options, sweeps, n, poses_out, iters_out, nds_out, stats, err, err_len);
 }
@@ -73,6 +75,7 @@ static int replay_impl(const liogpu_params* params, liogpu_ctx* borrowed, const 
     if (opt.keyframe_angle > 0.f) MO.surroundingkeyframeAddingAngleThreshold = opt.keyframe_angle;
     if (opt.search_radius > 0.f) MO.surroundingKeyframeSearchRadius = opt.search_radius;
     if (opt.density > 0.f) MO.surroundingKeyframeDensity = opt.density;
+    MO.detectLoopDistanceOnDevice = true;  // the replay runs both detectors through the library
     const unsigned long long launches0 = liogpu_launch_count(MO.context());
     const Clock::time_point t_all = Clock::now();
     int last_map_n = -1;
@@ -115,6 +118,17 @@ static int replay_impl(const liogpu_params* params, liogpu_ctx* borrowed, const 
       t0 = Clock::now();
       if (MO.saveFrame()) {                                              // saveKeyFramesAndFactor (:2085), gate :1909-1928
         MO.saveKeyFrameResident();
+        if (MO.lastStatus < 0) { rc = MO.lastStatus; break; }
+        if (opt.loop_detection_every > 0) {                              // :2151-2166
+          MO.makeAndSaveScancontextAndKeys();
+          if (MO.lastStatus < 0) { rc = MO.lastStatus; break; }
+        }
+      }
+      if (opt.loop_detection_every > 0 && (s + 1) % opt.loop_detection_every == 0 && !MO.cloudKeyPoses3D.empty()) {
+        int cur = -1, pre = -1;                                          // loopClosureThread: RS, then SC
+        if (MO.detectLoopClosureDistance(&cur, &pre)) ++st.loops_rs;
+        if (MO.lastStatus < 0) { rc = MO.lastStatus; break; }
+        if (MO.detectLoopClosureID().first != -1) ++st.loops_sc;
         if (MO.lastStatus < 0) { rc = MO.lastStatus; break; }
       }
       if (opt.publish_local_map) {

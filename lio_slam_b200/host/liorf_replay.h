@@ -28,7 +28,11 @@ typedef struct liorf_replay_options {
   int publish_local_map;          /* also run publishLocalMap after every scan (MO:504) */
   float keyframe_dist, keyframe_angle; /* surroundingkeyframeAddingDistThreshold / AngleThreshold (UT:312-313); 0 = 1.0 / 0.2 */
   float search_radius, density;   /* surroundingKeyframeSearchRadius / Density (UT:315-316); 0 = 50 / 2 */
-  int reserved[6];
+  int loop_detection_every;       /* 0 = off; N = every N sweeps, after the keyframe step, run detectLoopClosureDistance and
+                                     detectLoopClosureID (the 1 Hz loopClosureThread at 10 Hz sweeps: N = 10); a Scan
+                                     Context descriptor is then saved at every keyframe.  Both run through the library
+                                     (liogpu_detect_loop_distance, liogpu_sc_detect_loop).  The registration is unchanged. */
+  int reserved[5];
 } liorf_replay_options;
 
 typedef struct liorf_replay_stats {
@@ -40,7 +44,8 @@ typedef struct liorf_replay_stats {
   double loop_gpu_ms;              /* device time of the LM loops, summed */
   long long h2d_bytes, d2h_bytes;  /* sweep uploads / pose + state read-backs */
   unsigned long long gpu_launches;
-  int reserved[4];
+  int loops_sc, loops_rs;          /* loop_detection_every: detections of detectLoopClosureID / detectLoopClosureDistance */
+  int reserved[2];
 } liorf_replay_stats;
 
 /* poses_out: n x 6 floats (transformTobeMapped after every scan); iters_out, nds_out: n ints (LM iterations,
@@ -51,7 +56,8 @@ int liorf_replay_sequence(const liogpu_params* params, const liorf_replay_option
                           int err_len);
 
 /* A mapping worker = one liogpu context (one GPU, one stream) that replays sequence after sequence: the context, its
- * pinned staging memory and its device buffers are created once and reused (liogpu_keyframe_clear between sequences),
+ * pinned staging memory and its device buffers are created once and reused (liogpu_keyframe_clear and liogpu_sc_clear
+ * between sequences),
  * as a batch-mapping service would do.  One worker per host thread. */
 typedef struct liorf_worker liorf_worker;
 liorf_worker* liorf_worker_create(const liogpu_params* params, char* err, int err_len);

@@ -31,10 +31,12 @@ mapOptimization::mapOptimization(const liogpu_params& params) : params_(params) 
   const int st = liogpu_create(&ctx_, &params_);  // allocateMemory (mapOptmization.cpp:316-349)
   if (st != LIOGPU_OK) throw std::runtime_error("liogpu_create failed (no sm_100 GPU? there is no CPU fallback)");
   liogpu_default_local_map_params(&localMapParams);  // utility.h:219-229
+  liogpu_default_sc_params(&scParams);
 }
 mapOptimization::mapOptimization(const liogpu_params& params, liogpu_ctx* borrowed) : ctx_(borrowed), owns_ctx_(false), params_(params) {
   if (!ctx_) throw std::runtime_error("mapOptimization: null context");
   liogpu_default_local_map_params(&localMapParams);
+  liogpu_default_sc_params(&scParams);
 }
 mapOptimization::~mapOptimization() { if (owns_ctx_) liogpu_destroy(ctx_); }
 const char* mapOptimization::lastError() const { return liogpu_last_error(ctx_); }
@@ -299,6 +301,71 @@ bool mapOptimization::loopClosureICP(int loopKeyCur, int loopKeyPre, float corre
   if (lastStatus < 0) return false;
   if (!lastIcpInfo.converged || lastIcpInfo.fitness_score > historyKeyframeFitnessScore) return false;  // :1123
   if (noiseScore) *noiseScore = (float)lastIcpInfo.fitness_score;                   // :1145
+  return true;
+}
+
+void mapOptimization::makeAndSaveScancontextAndKeys() {
+  double desc[LIOGPU_SC_NUM_RING * LIOGPU_SC_NUM_SECTOR], ringkey[LIOGPU_SC_NUM_RING], sectorkey[LIOGPU_SC_NUM_SECTOR];
+  // LIDAR_HEIGHT 2.0, PC_MAX_RADIUS 80.0 (Scancontext.h); the resident cloud is read in place and stays valid
+  lastStatus = liogpu_make_scancontext(ctx_, LIOGPU_DEVICE_RESIDENT, 0, 16, 2.0, 80.0, desc, ringkey, sectorkey);
+  if (lastStatus < 0) return;
+  lastStatus = liogpu_sc_add(ctx_, desc, 1);
+}
+
+std::pair<int, float> mapOptimization::detectLoopClosureID() {
+  int loop_id = -1;
+  float yaw = 0.f;
+  lastStatus = liogpu_sc_detect_loop(ctx_, &scParams, &loop_id, &yaw, &lastScInfo);
+  if (lastStatus < 0) return {-1, 0.f};
+  return {loop_id, yaw};
+}
+
+bool mapOptimization::detectLoopClosureDistance(int* latestID, int* closestID) {
+  if (cloudKeyPoses3D.empty()) return false;
+  const int loopKeyCur = (int)cloudKeyPoses3D.size() - 1;
+  if (loopIndexContainer.find(loopKeyCur) != loopIndexContainer.end()) return false;  // :1277-1279
+  int loopKeyPre = -1;
+  if (detectLoopDistanceOnDevice) {
+    lastStatus = liogpu_detect_loop_distance(ctx_, cloudKeyPoses3D.data(), (int)cloudKeyPoses3D.size(), sizeof(PointType),
+                                             &cloudKeyPoses6D[0].time, sizeof(PointTypePose), timeLaserInfoCur,
+                                             historyKeyframeSearchRadius, historyKeyframeSearchTimeDiff, &loopKeyPre);
+    if (lastStatus < 0) return false;
+  } else {  // radiusSearch (d2 < (float)(r*r), by distance, ties by index), then the first old enough (:1282-1291)
+    const PointType& last = cloudKeyPoses3D.back();
+    const float r2 = (float)((double)historyKeyframeSearchRadius * (double)historyKeyframeSearchRadius);
+    float best = 0.f;
+    for (int i = 0; i < (int)cloudKeyPoses3D.size(); ++i) {
+      const PointType& p = cloudKeyPoses3D[i];
+      float d2 = 0.f, d = last.x - p.x;
+      d2 += d * d; d = last.y - p.y;
+      d2 += d * d; d = last.z - p.z;
+      d2 += d * d;
+      if (!(d2 < r2) || !(std::fabs(cloudKeyPoses6D[i].time - timeLaserInfoCur) > (double)historyKeyframeSearchTimeDiff)) continue;
+      if (loopKeyPre < 0 || d2 < best) { loopKeyPre = i; best = d2; }
+    }
+  }
+  if (loopKeyPre == -1 || loopKeyCur == loopKeyPre) return false;
+  *latestID = loopKeyCur;
+  *closestID = loopKeyPre;
+  return true;
+}
+
+bool mapOptimization::performSCLoopClosure(int* loopKeyCur, int* loopKeyPre, float correctionLidarFrame[16], float* noiseScore) {
+  if (cloudKeyPoses3D.empty()) return false;
+  const std::pair<int, float> detectResult = detectLoopClosureID();
+  if (detectResult.first == -1) return false;
+  *loopKeyCur = (int)cloudKeyPoses3D.size() - 1;
+  *loopKeyPre = detectResult.first;
+  if (!loopClosureICP(*loopKeyCur, *loopKeyPre, correctionLidarFrame, noiseScore)) return false;
+  loopIndexContainer[*loopKeyCur] = *loopKeyPre;
+  return true;
+}
+
+bool mapOptimization::performRSLoopClosure(int* loopKeyCur, int* loopKeyPre, float correctionLidarFrame[16], float* noiseScore) {
+  if (cloudKeyPoses3D.empty()) return false;
+  if (!detectLoopClosureDistance(loopKeyCur, loopKeyPre)) return false;
+  if (!loopClosureICP(*loopKeyCur, *loopKeyPre, correctionLidarFrame, noiseScore)) return false;
+  loopIndexContainer[*loopKeyCur] = *loopKeyPre;
   return true;
 }
 

@@ -10,6 +10,7 @@
 #pragma once
 #include <cmath>
 #include <cstdint>
+#include <map>
 #include <string>
 #include <vector>
 
@@ -93,6 +94,13 @@ class mapOptimization {
   // loop closure (utility.h:315, 321-324)
   float historyKeyframeSearchRadius = 10.0f, historyKeyframeFitnessScore = 0.3f, loopClosureICPSurfLeafSize = 0.3f;
   int historyKeyframeSearchNum = 25;
+  float historyKeyframeSearchTimeDiff = 30.0f;  // utility.h
+  liogpu_sc_params scParams;                    // SCManager's constants (Scancontext.h)
+  liogpu_sc_info lastScInfo{};
+  std::map<int, int> loopIndexContainer;        // loop closures already made: loopKeyCur -> loopKeyPre
+  // detectLoopClosureDistance through liogpu_detect_loop_distance instead of the host loop.  Off by default: on a B200
+  // the host loop was faster at every measured size up to 10^5 key poses (profiles/r03_loop_detection.jsonl)
+  bool detectLoopDistanceOnDevice = false;
   liogpu_icp_info lastIcpInfo{};
   liogpu_s2m_info lastInfo{};
   int lastStatus = 0;
@@ -116,6 +124,21 @@ class mapOptimization {
   // the cloud / ICP part of performRSLoopClosure (:1098-1125): false when a guard rejects the closure;
   // correctionLidarFrame = icp.getFinalTransformation() (row-major 4x4), noiseScore = icp.getFitnessScore()
   bool loopClosureICP(int loopKeyCur, int loopKeyPre, float correctionLidarFrame[16], float* noiseScore);
+  // ---- loop-closure detection (the loop context of INTEGRATION.md); descriptors are stored in this node's context ----
+  // scManager.makeAndSaveScancontextAndKeys(*thisSurfKeyFrame) (:2151-2166) on the keyframe's cloud as
+  // saveKeyFrameResident leaves it (the downsampled sweep, SCInputType::SINGLE_SCAN_FEAT) -> liogpu_make_scancontext +
+  // liogpu_sc_add
+  void makeAndSaveScancontextAndKeys();
+  // scManager.detectLoopClosureID() -> liogpu_sc_detect_loop: {loop id or -1, yaw difference (rad)}
+  std::pair<int, float> detectLoopClosureID();
+  // detectLoopClosureDistance (:1271-1300) -> liogpu_detect_loop_distance; false when there is no candidate or the
+  // newest key pose already closed a loop (loopIndexContainer)
+  bool detectLoopClosureDistance(int* latestID, int* closestID);
+  // performSCLoopClosure / performRSLoopClosure (:1187-1268 / :1086-1185): detection -> loopClosureICP.  Instead of
+  // queueing a GTSAM factor they return the pair and the correction (icp.getFinalTransformation()); true when a
+  // closure passed every guard (it is then recorded in loopIndexContainer).
+  bool performSCLoopClosure(int* loopKeyCur, int* loopKeyPre, float correctionLidarFrame[16], float* noiseScore);
+  bool performRSLoopClosure(int* loopKeyCur, int* loopKeyPre, float correctionLidarFrame[16], float* noiseScore);
   void publishLocalMap();                                // :2442-2541 -> liogpu_publish_local_map (fills localMapCloud)
   const char* lastError() const;
   liogpu_ctx* context() { return ctx_; }

@@ -78,13 +78,31 @@ class TileInfo(C.Structure):
                 ("reserved", C.c_int * 3)]
 
 
+LIOGPU_SC_MAX_CANDIDATES = 32
+
+
+class ScParams(C.Structure):
+    _fields_ = [("num_exclude_recent", C.c_int), ("num_candidates_from_tree", C.c_int), ("tree_making_period", C.c_int),
+                ("search_ratio", C.c_double), ("sc_dist_thres", C.c_double), ("reserved", C.c_int * 4)]
+
+
+class ScInfo(C.Structure):
+    _fields_ = [("n_stored", C.c_int), ("n_searchable", C.c_int), ("tree_rebuilt", C.c_int), ("n_candidates", C.c_int),
+                ("candidates", C.c_int * LIOGPU_SC_MAX_CANDIDATES), ("candidate_key_d2", C.c_float * LIOGPU_SC_MAX_CANDIDATES),
+                ("candidate_dist", C.c_double * LIOGPU_SC_MAX_CANDIDATES),
+                ("candidate_shift", C.c_int * LIOGPU_SC_MAX_CANDIDATES), ("nn_idx", C.c_int), ("nn_align", C.c_int),
+                ("min_dist", C.c_double), ("knn_ties", C.c_int), ("gpu_ms", C.c_float), ("reserved", C.c_int * 4)]
+
+
 EXPORTS = ["liogpu_abi_version", "liogpu_default_params", "liogpu_create", "liogpu_destroy", "liogpu_last_error",
            "liogpu_host_alloc", "liogpu_host_free", "liogpu_deskew", "liogpu_transform_cloud",
            "liogpu_voxel_downsample", "liogpu_keyframe_put", "liogpu_keyframe_clear", "liogpu_keyframe_count",
            "liogpu_build_local_map", "liogpu_set_local_map", "liogpu_local_map_size", "liogpu_scan2map",
            "liogpu_downsample_scan2map", "liogpu_surf_optimization", "liogpu_last_gpu_ms", "liogpu_launch_count",
            "liogpu_stream", "liogpu_resident_size", "liogpu_default_local_map_params", "liogpu_publish_local_map", "liogpu_merge_keyframes", "liogpu_default_icp_params", "liogpu_icp_align", "liogpu_make_scancontext", "liogpu_extract_nearby",
-           "liogpu_scan2map_trace", "liogpu_voxel_tile", "liogpu_upload_scan_async", "liogpu_fetch_result"]
+           "liogpu_scan2map_trace", "liogpu_voxel_tile", "liogpu_upload_scan_async", "liogpu_fetch_result",
+           "liogpu_default_sc_params", "liogpu_sc_add", "liogpu_sc_clear", "liogpu_sc_detect_loop", "liogpu_sc_detect_loops",
+           "liogpu_detect_loop_distance"]
 
 RESIDENT = "resident"   # LIOGPU_DEVICE_RESIDENT: the cloud the context kept in HBM (include/liogpu.h)
 UPLOADED = "uploaded"   # LIOGPU_UPLOADED_SCAN: the sweep liogpu_upload_scan_async put on its way
@@ -138,6 +156,16 @@ def load_library() -> C.CDLL:
                                             C.c_void_p, C.c_void_p]
     lib.liogpu_extract_nearby.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_double,
                                           C.c_float, C.c_float, C.c_void_p, C.c_int, C.POINTER(C.c_int)]
+    lib.liogpu_default_sc_params.argtypes = [C.POINTER(ScParams)]
+    lib.liogpu_default_sc_params.restype = None
+    lib.liogpu_sc_add.argtypes = [C.c_void_p, C.c_void_p, C.c_int]
+    lib.liogpu_sc_clear.argtypes = [C.c_void_p]
+    lib.liogpu_sc_detect_loop.argtypes = [C.c_void_p, C.POINTER(ScParams), C.POINTER(C.c_int), C.POINTER(C.c_float),
+                                          C.POINTER(ScInfo)]
+    lib.liogpu_sc_detect_loops.argtypes = [C.c_void_p, C.POINTER(ScParams), C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
+                                           C.c_void_p]
+    lib.liogpu_detect_loop_distance.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_double,
+                                                C.c_float, C.c_float, C.POINTER(C.c_int)]
     lib.liogpu_default_icp_params.argtypes = [C.POINTER(IcpParams), C.c_float]
     lib.liogpu_default_icp_params.restype = None
     lib.liogpu_icp_align.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int,
@@ -175,6 +203,16 @@ def local_map_params(**over) -> LocalMapParams:
     load_library().liogpu_default_local_map_params(C.byref(p))
     for k, v in over.items():
         setattr(p, k, v)
+    return p
+
+
+def sc_params(**over) -> ScParams:
+    """SCManager's constants (Scancontext.h) with keyword overrides; `num_candidates` is accepted for
+    num_candidates_from_tree."""
+    p = ScParams()
+    load_library().liogpu_default_sc_params(C.byref(p))
+    for k, v in over.items():
+        setattr(p, "num_candidates_from_tree" if k == "num_candidates" else k, v)
     return p
 
 
@@ -412,6 +450,52 @@ class LioGpu:
                                                         C.c_float(radius), C.c_float(density), ids.ctypes.data, ids.shape[0],
                                                         C.byref(n_ids)))
         return ids[: n_ids.value].copy(), st
+
+    def sc_add(self, descs) -> None:
+        """makeAndSaveScancontextAndKeys for descriptors as make_scancontext returns them: (20, 60) or (n, 20, 60) f64."""
+        d = np.ascontiguousarray(descs, np.float64).reshape(-1, 1200)
+        self._check(self.lib.liogpu_sc_add(self.h, d.ctypes.data, d.shape[0]))
+
+    def sc_clear(self) -> None:
+        self._check(self.lib.liogpu_sc_clear(self.h))
+
+    def sc_detect_loop(self, params: "ScParams | None" = None, **over):
+        """SCManager::detectLoopClosureID on the newest stored descriptor -> (loop_id, yaw_diff_rad, info dict)."""
+        prm = params if params is not None else sc_params(**over)
+        loop_id = C.c_int(0)
+        yaw = C.c_float(0)
+        info = ScInfo()
+        self._check(self.lib.liogpu_sc_detect_loop(self.h, C.byref(prm), C.byref(loop_id), C.byref(yaw), C.byref(info)))
+        n = info.n_candidates
+        d = dict(n_stored=info.n_stored, n_searchable=info.n_searchable, tree_rebuilt=info.tree_rebuilt, n_candidates=n,
+                 candidates=np.array(info.candidates[:n], np.int32),
+                 candidate_key_d2=np.array(info.candidate_key_d2[:n], np.float32),
+                 candidate_dist=np.array(info.candidate_dist[:n], np.float64),
+                 candidate_shift=np.array(info.candidate_shift[:n], np.int32), nn_idx=info.nn_idx, nn_align=info.nn_align,
+                 min_dist=info.min_dist, knn_ties=info.knn_ties, gpu_ms=info.gpu_ms)
+        return loop_id.value, np.float32(yaw.value), d
+
+    def sc_detect_loops(self, store_sizes, params: "ScParams | None" = None, **over):
+        """detectLoopClosureID of a fresh SCManager at each store size -> (loop_ids, yaw_diff_rad, min_dist)."""
+        prm = params if params is not None else sc_params(**over)
+        sizes = np.ascontiguousarray(store_sizes, np.int32)
+        n = sizes.shape[0]
+        ids = np.zeros(max(n, 1), np.int32)
+        yaw = np.zeros(max(n, 1), np.float32)
+        md = np.zeros(max(n, 1), np.float64)
+        self._check(self.lib.liogpu_sc_detect_loops(self.h, C.byref(prm), sizes.ctypes.data, n, ids.ctypes.data,
+                                                    yaw.ctypes.data, md.ctypes.data))
+        return ids[:n].copy(), yaw[:n].copy(), md[:n].copy()
+
+    def detect_loop_distance(self, key3d, key_time, time_cur: float, radius: float = 10.0, time_diff: float = 30.0) -> int:
+        """detectLoopClosureDistance (mapOptmization.cpp ~1271-1300) without the loopIndexContainer check -> id or -1."""
+        ptr, n, stride, keep = _cloud_args(key3d)
+        key_time = np.ascontiguousarray(key_time, np.float64)
+        assert key_time.shape[0] == n
+        out = C.c_int(-1)
+        self._check(self.lib.liogpu_detect_loop_distance(self.h, ptr, n, stride, key_time.ctypes.data, 8, C.c_double(time_cur),
+                                                         C.c_float(radius), C.c_float(time_diff), C.byref(out)))
+        return out.value
 
     def upload_scan_async(self, cloud) -> None:
         """liogpu_upload_scan_async: the buffer must stay alive until the call that consumes UPLOADED returns."""

@@ -22,7 +22,8 @@ class Sweep(C.Structure):
 
 class ReplayOptions(C.Structure):
     _fields_ = [("select_key_poses_on_device", C.c_int), ("publish_local_map", C.c_int), ("keyframe_dist", C.c_float),
-                ("keyframe_angle", C.c_float), ("search_radius", C.c_float), ("density", C.c_float), ("reserved", C.c_int * 6)]
+                ("keyframe_angle", C.c_float), ("search_radius", C.c_float), ("density", C.c_float),
+                ("loop_detection_every", C.c_int), ("reserved", C.c_int * 5)]
 
 
 class ReplayStats(C.Structure):
@@ -30,7 +31,8 @@ class ReplayStats(C.Structure):
                 ("lm_iterations", C.c_int), ("map_points_last", C.c_int), ("wall_ms", C.c_double),
                 ("deskew_ms", C.c_double), ("nearby_ms", C.c_double), ("register_ms", C.c_double),
                 ("keyframe_ms", C.c_double), ("loop_gpu_ms", C.c_double), ("h2d_bytes", C.c_longlong),
-                ("d2h_bytes", C.c_longlong), ("gpu_launches", C.c_ulonglong), ("reserved", C.c_int * 4)]
+                ("d2h_bytes", C.c_longlong), ("gpu_launches", C.c_ulonglong), ("loops_sc", C.c_int), ("loops_rs", C.c_int),
+                ("reserved", C.c_int * 2)]
 
 
 _lib = None
