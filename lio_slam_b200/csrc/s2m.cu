@@ -21,9 +21,8 @@
 //     convergence test (:1784-1835), next iteration's transform
 //   lm_matp_kernel    iteration 0's Jacobi eigen-decomposition + matP on a second stream when a rigorous
 //     certificate has already decided isDegenerate = false
-//   A/B variants of the main kernel (LIOGPU_MAIN, bit-identical results, all measured slower: DESIGN.md §4):
-//     s2m_main_pw_kernel (persistent warps), s2m_wc.cuh (warp-cooperative candidate evaluation), s2m_split.cuh
-//     (search in one wave + fit kernel); s2m_fused.cuh is the whole loop as one cooperative launch (params.s2m_path = 2)
+//   s2m_fused.cuh is the whole loop as one cooperative launch (params.s2m_path = 2).  Other main kernels (persistent
+//   warps, warp-cooperative candidate evaluation, search and fit split) were measured slower: DESIGN.md §4.
 //
 // The pose, matP, isDegenerate and the iteration counter stay in HBM (LmDevState); the host enqueues a chunk of
 // iterations back to back and reads the 2.5 KB state once — a launch that finds `done` set returns immediately.
@@ -44,9 +43,9 @@ namespace liogpu {
 #define S2M_MINBLOCKS_CFG 4
 #endif
 constexpr int S2M_THREADS = S2M_THREADS_CFG;
-// The leftover kernel turns the main kernel's per-block (per-chunk) leftover counts into segment offsets itself, in
-// shared memory, when the table fits; the main kernels then end without a ticket and without the serial scan their last
-// block used to run (4 rounds on the fixed grid, 29 on the per-chunk table of the persistent-warp kernel).
+// The leftover kernel turns the main kernel's per-block leftover counts into segment offsets itself, in shared memory,
+// when the table fits; the main kernel then ends without a ticket and without the serial scan of its last block (which
+// still runs for sweeps of more than (LEFT_OFF_CAP - 1) x S2M_THREADS points).
 constexpr int LEFT_OFF_CAP = 8192;
 constexpr int S2M_SUMS = 32;  // 21 (upper AtA) + 6 (AtB) + nsel + ties, padded to 32
 
@@ -84,23 +83,6 @@ struct Top5 {
       rej = fminf(rej, d);
     }
   }
-  // The list already holds real map points (the previous iteration's neighbours): a candidate that IS one of them is
-  // skipped — it neither enters twice nor counts as a rejected candidate.
-  __device__ __forceinline__ void offer_seeded(float d, int id) {
-    const u64 key = (((u64)__float_as_uint(d)) << 32) | (u64)(unsigned)id;
-    if (key < k4) {
-      if (key == k0 || key == k1 || key == k2 || key == k3) return;
-      rej = fminf(rej, __uint_as_float((unsigned)(k4 >> 32)));
-      u64 lo;
-      k4 = key;
-      lo = min(k3, k4); k4 = max(k3, k4); k3 = lo;
-      lo = min(k2, k3); k3 = max(k2, k3); k2 = lo;
-      lo = min(k1, k2); k2 = max(k1, k2); k1 = lo;
-      lo = min(k0, k1); k1 = max(k0, k1); k0 = lo;
-    } else if (key != k4) {
-      rej = fminf(rej, d);
-    }
-  }
   __device__ __forceinline__ float d(const u64 k) const { return __uint_as_float((unsigned)(k >> 32)); }
   __device__ __forceinline__ int i(const u64 k) const { return (int)(unsigned)(k & 0xffffffffull); }
   __device__ __forceinline__ bool tie() const {
@@ -121,12 +103,10 @@ __device__ __forceinline__ int zigzag(int k) { return (k & 1) ? -((k + 1) >> 1) 
 
 // Exact 5 nearest map points of q among those closer than sqrt(gate_d2), ascending (d2, map index).
 // On return t.d(t.k4) < gate_d2 iff at least 5 such points exist (then the answer is exact).
-// PRESET: t already holds five real map points closer than sqrt(gate_d2) (in order); the walk skips them when it meets them.
-template <bool PRESET = false>
 __device__ __forceinline__ void grid_knn5(const float4 q, const GridParams& g, const float gate_d2,
                                           const float4* __restrict__ map_sorted,
                                           const uint32_t* __restrict__ cell_start, Top5& t) {
-  if (!PRESET) t.init(gate_d2);
+  t.init(gate_d2);
   const float s2 = 2.0f * g.slack;
   const float reach = sqrtf(gate_d2) * 1.000001f + s2;
   int zmin = (int)floorf((q.z - reach - g.oz) * g.inv_h), zmax = (int)floorf((q.z + reach - g.oz) * g.inv_h);
@@ -170,17 +150,10 @@ __device__ __forceinline__ void grid_knn5(const float4 q, const GridParams& g, c
         const float4 p1 = __ldg(map_sorted + min(j + 1, last));
         const float4 p2 = __ldg(map_sorted + min(j + 2, last));
         const float4 p3 = __ldg(map_sorted + min(j + 3, last));
-        if (PRESET) {
-          t.offer_seeded(l2_simple(q, p0), __float_as_int(p0.w));
-          if (j + 1 < e) t.offer_seeded(l2_simple(q, p1), __float_as_int(p1.w));
-          if (j + 2 < e) t.offer_seeded(l2_simple(q, p2), __float_as_int(p2.w));
-          if (j + 3 < e) t.offer_seeded(l2_simple(q, p3), __float_as_int(p3.w));
-        } else {
-          t.offer(l2_simple(q, p0), __float_as_int(p0.w));
-          if (j + 1 < e) t.offer(l2_simple(q, p1), __float_as_int(p1.w));
-          if (j + 2 < e) t.offer(l2_simple(q, p2), __float_as_int(p2.w));
-          if (j + 3 < e) t.offer(l2_simple(q, p3), __float_as_int(p3.w));
-        }
+        t.offer(l2_simple(q, p0), __float_as_int(p0.w));
+        if (j + 1 < e) t.offer(l2_simple(q, p1), __float_as_int(p1.w));
+        if (j + 2 < e) t.offer(l2_simple(q, p2), __float_as_int(p2.w));
+        if (j + 3 < e) t.offer(l2_simple(q, p3), __float_as_int(p3.w));
       }
     }
   }
@@ -192,10 +165,6 @@ __device__ __forceinline__ void grid_knn5(const float4 q, const GridParams& g, c
 // where it runs ~30 times per warp at 5 of 32 lanes; the five are selected afterwards with all lanes in step.  The bound
 // is not tightened during the walk (nothing to gain when it is tight from the start).  Returns the number of candidates
 // inside the bound; more than S2M_COLLECT_CAP means the list overflowed (the caller repeats with the insertion walk).
-#ifndef S2M_GATE1_WIDEN_CFG
-#define S2M_GATE1_WIDEN_CFG 1.0f
-#endif
-constexpr float S2M_GATE1_WIDEN = S2M_GATE1_WIDEN_CFG;  // (radius factor)^2 of the unseeded search in the main kernel
 #ifndef S2M_COLLECT_CAP_CFG
 #define S2M_COLLECT_CAP_CFG 16
 #endif
@@ -261,11 +230,10 @@ __device__ __forceinline__ int grid_knn5_collect(const float4 q, const GridParam
 // and the rows are then walked centre-out with the usual pruning against the running 5th-best distance.
 // The x range of a row is fixed from the initial bound (a superset of what the tightened bound would give);
 // the extra candidates cost one compare each.  Returns false when the box is larger (caller falls back).
-template <bool PRESET = false>
 __device__ __forceinline__ bool grid_knn5_box9(const float4 q, const GridParams& g, const float gate_d2,
                                                const float4* __restrict__ map_sorted,
                                                const uint32_t* __restrict__ cell_start, Top5& t) {
-  if (!PRESET) t.init(gate_d2);
+  t.init(gate_d2);
   const float s2 = 2.0f * g.slack;
   const float reach = sqrtf(gate_d2) * 1.000001f + s2;
   int zmin = (int)floorf((q.z - reach - g.oz) * g.inv_h), zmax = (int)floorf((q.z + reach - g.oz) * g.inv_h);
@@ -316,17 +284,10 @@ __device__ __forceinline__ bool grid_knn5_box9(const float4 q, const GridParams&
       const float4 p1 = __ldg(map_sorted + min(j + 1, last));
       const float4 p2 = __ldg(map_sorted + min(j + 2, last));
       const float4 p3 = __ldg(map_sorted + min(j + 3, last));
-      if (PRESET) {
-        t.offer_seeded(l2_simple(q, p0), __float_as_int(p0.w));
-        if (j + 1 < e) t.offer_seeded(l2_simple(q, p1), __float_as_int(p1.w));
-        if (j + 2 < e) t.offer_seeded(l2_simple(q, p2), __float_as_int(p2.w));
-        if (j + 3 < e) t.offer_seeded(l2_simple(q, p3), __float_as_int(p3.w));
-      } else {
-        t.offer(l2_simple(q, p0), __float_as_int(p0.w));
-        if (j + 1 < e) t.offer(l2_simple(q, p1), __float_as_int(p1.w));
-        if (j + 2 < e) t.offer(l2_simple(q, p2), __float_as_int(p2.w));
-        if (j + 3 < e) t.offer(l2_simple(q, p3), __float_as_int(p3.w));
-      }
+      t.offer(l2_simple(q, p0), __float_as_int(p0.w));
+      if (j + 1 < e) t.offer(l2_simple(q, p1), __float_as_int(p1.w));
+      if (j + 2 < e) t.offer(l2_simple(q, p2), __float_as_int(p2.w));
+      if (j + 3 < e) t.offer(l2_simple(q, p3), __float_as_int(p3.w));
     }
   }
   return true;
@@ -937,11 +898,8 @@ struct S2mArgs {
   const float* T_override;
   SurfDebugOut dbg;
   int mode;
-  int main_blocks;         // partial rows of the main phase
-  int seg_blocks;          // leftover segments (= main_blocks except for the split search kernel's smaller blocks)
+  int main_blocks;         // main kernel blocks: partial rows of the main phase and leftover segments
   float collect_move;      // metres: a warp collects when most of its seeded points moved less than this (see main_point)
-  int seg_stride;          // slots per segment of fail_seg (S2M_THREADS, or 32 for the persistent-warp main kernel)
-  unsigned* queue;         // chunk queue head of the persistent-warp main kernel
   int* prev_nn;            // [5][nq] neighbours found by the previous iteration (-1: none), SoA
   float4* hopeless;        // [nq] (x,y,z of the point when it was found hopeless, w = 1) or w = 0
 };
@@ -1013,16 +971,9 @@ __device__ __forceinline__ void main_point(const S2mArgs& A, const float* sT, co
     const float4 sel = apply_T(sT, ori);
     Top5 t;
     const bool dense = A.g.gate1_d2 < A.g.gate_d2;     // phase-1 gate active (cell edge = its radius)
-    // An unseeded point searches a somewhat wider ball than the phase-1 radius: the walk is centre-out and pruned against the
-    // running 5th distance, so only the few points without five neighbours inside the phase-1 radius pay for it, and most
-    // of them are settled here instead of by a warp-cooperative full-gate search in the leftover kernel.
-    float gate_use = fminf(A.g.gate1_d2 * S2M_GATE1_WIDEN, A.g.gate_d2);
+    float gate_use = fminf(A.g.gate1_d2, A.g.gate_d2);
     const float gate1_use = gate_use;
     bool can_search = dense, is_seeded = false, skip = false;
-#ifdef S2M_PRESET_SEEDS
-    float sd[5] = {0.f, 0.f, 0.f, 0.f, 0.f};
-    int sp[5] = {0, 0, 0, 0, 0};
-#endif
     if (s_iter > 0) {
       // Seeded search: the five neighbours of the previous iteration are real map points, so their
       // largest distance to the moved query bounds the true 5th-neighbour distance.  Searching inside
@@ -1048,10 +999,6 @@ __device__ __forceinline__ void main_point(const S2mArgs& A, const float* sT, co
           can_search = true;
           is_seeded = true;
           ++seeded;
-#ifdef S2M_PRESET_SEEDS
-          sd[0] = d0; sd[1] = d1; sd[2] = d2; sd[3] = d3; sd[4] = d4;
-          sp[0] = p0; sp[1] = p1; sp[2] = p2; sp[3] = p3; sp[4] = p4;
-#endif
         }
       }
     }
@@ -1060,7 +1007,6 @@ __device__ __forceinline__ void main_point(const S2mArgs& A, const float* sT, co
     //   otherwise -> the insertion walk that tightens its bound as it goes (after a large step the seeds' bound is loose:
     //   collecting then costs 130 us instead of 77).
     bool use_collect = false;
-#ifndef S2M_NO_COLLECT
     if (s_iter > 0 && dense) {
       const float range = sqrtf(ori.x * ori.x + ori.y * ori.y + ori.z * ori.z);
       const unsigned act = __activemask();
@@ -1068,17 +1014,6 @@ __device__ __forceinline__ void main_point(const S2mArgs& A, const float* sT, co
       const unsigned mt = __ballot_sync(act, is_seeded && step_t + step_r * range < A.collect_move);
       use_collect = 4 * __popc(mt) >= 3 * __popc(ms);
     }
-#endif
-    bool preset = false;
-#ifdef S2M_PRESET_SEEDS
-    // A/B: the five seeds enter the list up front and the walk skips them when it meets them (grid_knn5<true>).  Measured
-    // on this kernel: -2 us on a late iteration (where collecting wins by 12), +8 us on the iteration after a large step.
-    if (is_seeded && !use_collect) {
-      t.init(gate_use);
-      t.offer(sd[0], sp[0]); t.offer(sd[1], sp[1]); t.offer(sd[2], sp[2]); t.offer(sd[3], sp[3]); t.offer(sd[4], sp[4]);
-      preset = true;
-    }
-#endif
     if (skip) {
       t.init(A.g.gate_d2);  // "not found": flag false, no seeds for the next iteration, marker kept
       need2 = false;
@@ -1099,13 +1034,8 @@ __device__ __forceinline__ void main_point(const S2mArgs& A, const float* sT, co
         // dense map: the row-by-row walk (x ranges tightened as the bound shrinks) executes fewer instructions
         // and the kernel is issue bound; sparse map (1 m cells, few points per row): the search is latency
         // bound and the all-rows-at-once variant wins
-        if (preset) {
-          if (dense || !grid_knn5_box9<true>(sel, A.g, gate_use, A.map_sorted, A.cell_start, t))
-            grid_knn5<true>(sel, A.g, gate_use, A.map_sorted, A.cell_start, t);
-        } else {
-          if (dense || !grid_knn5_box9(sel, A.g, gate_use, A.map_sorted, A.cell_start, t))
-            grid_knn5(sel, A.g, gate_use, A.map_sorted, A.cell_start, t);
-        }
+        if (dense || !grid_knn5_box9(sel, A.g, gate_use, A.map_sorted, A.cell_start, t))
+          grid_knn5(sel, A.g, gate_use, A.map_sorted, A.cell_start, t);
       }
       need2 = !is_seeded && !(t.d(t.k4) < gate1_use);
     } else {
@@ -1197,7 +1127,7 @@ s2m_main_kernel(const S2mArgs A) {
     for (int w = 0; w < S2M_THREADS / 32; ++w) nf += s_wfail[w];
     A.block_nfail[blockIdx.x] = nf;
   }
-  if (A.seg_blocks + 1 <= LEFT_OFF_CAP) return;  // the leftover kernel derives the offsets itself
+  if (A.main_blocks + 1 <= LEFT_OFF_CAP) return;  // the leftover kernel derives the offsets itself
   __threadfence();
   __syncthreads();
   if (tid == 0) s_last = (atomicAdd(A.ticket, 1u) == gridDim.x - 1);
@@ -1234,106 +1164,6 @@ s2m_main_kernel(const S2mArgs A) {
   }
 }
 
-// Persistent-warp variant of s2m_main_kernel (round 2, VERDICT lever (i)): the grid is sized to residency and every
-// WARP pulls 32-point chunks from an atomic queue until the sweep is exhausted, so no SM idles while work remains (the
-// fixed grid leaves 23 % of the SM-cycles idle: 900 CTAs on 592 slots).  MEASURED SLOWER than the fixed grid (config 3:
-// 88 vs 78 us per launch; 16-beam shape 21 vs 20): kept for A/B (LIOGPU_MAIN=pw), not the default.  A chunk's 27 sums go to its own partial row and
-// its leftovers to its own segment (both indexed by the chunk, so the result does not depend on which warp took it);
-// the last CTA to finish turns the per-chunk leftover counts into offsets, exactly as the fixed-grid kernel does per block.
-__global__ void __launch_bounds__(S2M_THREADS, S2M_MINBLOCKS_CFG)
-s2m_main_pw_kernel(const S2mArgs A) {
-  __shared__ float sT[12];
-  __shared__ LmTrig sTrig;
-  __shared__ float rows[S2M_THREADS][8];
-  __shared__ u64 s_list[S2M_COLLECT_CAP][S2M_THREADS];
-  __shared__ float s_step[2];
-  __shared__ int s_iter, s_done0;
-  __shared__ bool s_last;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  cudaGridDependencySynchronize();
-  if (tid < 12) sT[tid] = A.T_override ? A.T_override[tid] : A.st->T[tid];
-  if (tid == 32) {
-    sTrig.srx = A.st->trig[0]; sTrig.crx = A.st->trig[1]; sTrig.sry = A.st->trig[2];
-    sTrig.cry = A.st->trig[3]; sTrig.srz = A.st->trig[4]; sTrig.crz = A.st->trig[5];
-  }
-  if (tid == 64) { s_done0 = A.st->done; s_iter = A.mode == 0 ? A.st->iter : 0; }
-  if (tid == 96) { s_step[0] = A.st->delta_t * 0.01f; s_step[1] = A.st->delta_r * 0.01745329f; }  // last step: metres, radians
-  __syncthreads();
-  if (A.mode == 0 && s_done0) return;
-  const int nchunks = A.main_blocks;
-  const RowAcc ra = row_acc_of(lane);
-  for (;;) {
-    int c = 0;
-    if (lane == 0) c = (int)atomicAdd(A.queue, 1u);
-    c = __shfl_sync(0xffffffffu, c, 0);
-    if (c >= nchunks) break;
-    const int i = c * 32 + lane;
-    float row[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-    float rhs = 0.f;
-    bool flag = false, tie = false, need2 = false;
-    int seeded = 0;
-    if (i < A.nq) main_point(A, sT, sTrig, s_iter, i, row, rhs, flag, tie, need2, seeded, &s_list[0][tid], s_step[0], s_step[1]);
-    const unsigned fm = __ballot_sync(0xffffffffu, need2);
-    if (need2) A.fail_seg[(size_t)c * 32 + __popc(fm & ((1u << lane) - 1u))] = i;
-    if (lane == 0) A.block_nfail[c] = __popc(fm);
-    const int w_ties = __popc(__ballot_sync(0xffffffffu, flag && tie));
-    const int w_seed = __popc(__ballot_sync(0xffffffffu, seeded != 0));
-#pragma unroll
-    for (int k = 0; k < 6; ++k) rows[tid][k] = row[k];
-    rows[tid][6] = rhs;
-    rows[tid][7] = flag ? 1.f : 0.f;
-    __syncwarp();
-    double acc = 0.0;
-    if (ra.live) {
-#pragma unroll 8
-      for (int r = 0; r < 32; ++r) {
-        const float* rr = rows[warp * 32 + r];
-        acc += (double)rr[ra.a] * (double)rr[ra.b];
-      }
-    }
-    if (lane == 28) acc = (double)w_ties;
-    if (lane == 29) acc = (double)w_seed;
-    A.partials_main[(size_t)c * S2M_SUMS + lane] = acc;
-    __syncwarp();
-  }
-  if (nchunks + 1 <= LEFT_OFF_CAP) return;  // offsets: leftover kernel; queue head: reset there too
-  __threadfence();
-  __syncthreads();
-  if (tid == 0) s_last = (atomicAdd(A.ticket, 1u) == gridDim.x - 1);
-  __syncthreads();
-  if (!s_last) return;
-  // ---- last CTA: exclusive scan of the per-chunk leftover counts -> fail_off (chunk order) ----
-  __threadfence();
-  __shared__ int s_wsum[S2M_THREADS / 32];
-  __shared__ int s_carry;
-  if (tid == 0) s_carry = 0;
-  __syncthreads();
-  for (int b0 = 0; b0 < nchunks; b0 += S2M_THREADS) {
-    const int b = b0 + tid;
-    const int cnt = b < nchunks ? __ldcg(A.block_nfail + b) : 0;
-    int incl = cnt;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const int v = __shfl_up_sync(0xffffffffu, incl, o);
-      if (lane >= o) incl += v;
-    }
-    if (lane == 31) s_wsum[warp] = incl;
-    __syncthreads();
-    int base = s_carry;
-    for (int w = 0; w < warp; ++w) base += s_wsum[w];
-    if (b < nchunks) A.fail_off[b] = base + incl - cnt;
-    __syncthreads();
-    if (tid == S2M_THREADS - 1) s_carry = base + incl;
-    __syncthreads();
-  }
-  if (tid == 0) {
-    A.fail_off[nchunks] = s_carry;
-    *A.fail_total = s_carry;
-    *A.ticket = 0u;
-    *A.queue = 0u;
-  }
-}
-
 constexpr int LEFT_THREADS = 256;
 __global__ void __launch_bounds__(LEFT_THREADS, 2)
 s2m_left_kernel(const S2mArgs A) {
@@ -1356,19 +1186,18 @@ s2m_left_kernel(const S2mArgs A) {
     sTrig.cry = A.st->trig[3]; sTrig.srz = A.st->trig[4]; sTrig.crz = A.st->trig[5];
     s_ties = 0;
   }
-  const bool off_in_smem = A.seg_blocks + 1 <= LEFT_OFF_CAP;
+  const bool off_in_smem = A.main_blocks + 1 <= LEFT_OFF_CAP;
   if (tid == 64) { s_done0 = A.st->done; s_iter0 = A.st->iter; s_total0 = off_in_smem ? 0 : *A.fail_total; }
-  if (tid == 96 && blockIdx.x == 0) *A.queue = 0u;  // chunk queue of the persistent-warp main kernel
   // The offsets of the leftover segments (exclusive scan of the main kernel's per-block counts), computed HERE by every
   // block in shared memory: every thread sums a contiguous slice of the counts (all loads in flight), one block-wide scan
   // of the 256 slice sums, then the slice's prefixes are written out.  The binary search below runs on shared memory.
   __shared__ int s_off[LEFT_OFF_CAP];
   __shared__ int s_wsum[LEFT_THREADS / 32];
   if (off_in_smem) {
-    for (int k = tid; k < A.seg_blocks; k += LEFT_THREADS) s_off[k] = __ldcg(A.block_nfail + k);  // one round trip
+    for (int k = tid; k < A.main_blocks; k += LEFT_THREADS) s_off[k] = __ldcg(A.block_nfail + k);  // one round trip
     __syncthreads();
-    const int per = (A.seg_blocks + LEFT_THREADS - 1) / LEFT_THREADS;
-    const int k0 = min(tid * per, A.seg_blocks), k1 = min(k0 + per, A.seg_blocks);
+    const int per = (A.main_blocks + LEFT_THREADS - 1) / LEFT_THREADS;
+    const int k0 = min(tid * per, A.main_blocks), k1 = min(k0 + per, A.main_blocks);
     int sum = 0;
     for (int k = k0; k < k1; ++k) sum += s_off[k];
     int incl = sum;
@@ -1382,7 +1211,7 @@ s2m_left_kernel(const S2mArgs A) {
     int run = incl - sum;
     for (int w = 0; w < warp; ++w) run += s_wsum[w];
     for (int k = k0; k < k1; ++k) { const int v = s_off[k]; s_off[k] = run; run += v; }
-    if (tid == LEFT_THREADS - 1) { s_off[A.seg_blocks] = run; s_total0 = run; }
+    if (tid == LEFT_THREADS - 1) { s_off[A.main_blocks] = run; s_total0 = run; }
   }
   __syncthreads();
   if (A.mode == 0 && s_done0) return;
@@ -1417,13 +1246,13 @@ s2m_left_kernel(const S2mArgs A) {
         if (all_points) {
           mine = e;
         } else {  // leftover e lives in the segment of the main block whose offset range contains it
-          int lo = 0, hi = A.seg_blocks;  // invariant: fail_off[lo] <= e < fail_off[hi]
+          int lo = 0, hi = A.main_blocks;  // invariant: fail_off[lo] <= e < fail_off[hi]
           while (hi - lo > 1) {
             const int mid = (lo + hi) >> 1;
             const int v = off_in_smem ? s_off[mid] : __ldg(A.fail_off + mid);
             if (v <= e) lo = mid; else hi = mid;
           }
-          mine = A.fail_seg[(size_t)lo * A.seg_stride + (e - (off_in_smem ? s_off[lo] : __ldg(A.fail_off + lo)))];
+          mine = A.fail_seg[(size_t)lo * S2M_THREADS + (e - (off_in_smem ? s_off[lo] : __ldg(A.fail_off + lo)))];
         }
       }
       float4 ori = make_float4(0.f, 0.f, 0.f, 0.f), sel = ori;
@@ -1528,8 +1357,6 @@ s2m_left_kernel(const S2mArgs A) {
 }
 
 }  // namespace liogpu
-#include "s2m_wc.cuh"
-#include "s2m_split.cuh"
 #include "s2m_fused.cuh"
 namespace liogpu {
 
@@ -1537,11 +1364,10 @@ namespace liogpu {
 // as the previous one drains (its last block is still reducing / solving the 6x6 system) and waits in
 // cudaGridDependencySynchronize(), which hides the launch latency between dependent kernels.
 template <class K>
-static cudaError_t launch_pdl(K kernel, int blocks, int threads, cudaStream_t stream, const S2mArgs& A, size_t smem = 0) {
+static cudaError_t launch_pdl(K kernel, int blocks, int threads, cudaStream_t stream, const S2mArgs& A) {
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3((unsigned)blocks);
   cfg.blockDim = dim3((unsigned)threads);
-  cfg.dynamicSmemBytes = smem;
   cfg.stream = stream;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
@@ -1556,66 +1382,17 @@ static int check_grid(Ctx* c) {
   return LIOGPU_OK;
 }
 
-// device scratch shared by both entry points
-// CTAs of the persistent-warp main kernel: every resident slot, but no more warps than chunks
-static int pw_grid_size(Ctx* c, int nchunks) {
-  static int per_sm = 0;
-  if (per_sm == 0) {
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, s2m_main_pw_kernel, S2M_THREADS, 0) != cudaSuccess || per_sm < 1) per_sm = 1;
-  }
-  const int full = per_sm * c->sm_count;
-  const int need = div_up(nchunks, S2M_THREADS / 32);
-  return need < full ? (need > 0 ? need : 1) : full;
-}
-
-// LIOGPU_MAIN = fixed | pw | wc | wc1 | split selects the main kernel for A/B runs: the thread-per-point walk on a fixed grid, the
-// same on persistent warps, the warp-cooperative candidate evaluation (s2m_wc.cuh) for every iteration, or for the
-// seeded iterations only (iteration 0 on the fixed grid).
-static int main_variant_env() {
-  static const int env = [] {
-    const char* e = getenv("LIOGPU_MAIN");
-    if (!e) return -1;
-    if (!strcmp(e, "fixed")) return 0;
-    if (!strcmp(e, "pw")) return 1;
-    if (!strcmp(e, "wc")) return 2;
-    if (!strcmp(e, "wc1")) return 3;
-    if (!strcmp(e, "split")) return 4;
-    return -1;
-  }();
-  return env;
-}
-static bool use_pw_main(const Ctx* c) {
-  (void)c;
-  return main_variant_env() == 1;  // the fixed grid measured faster than persistent warps (104 vs 117 us per iteration, config 3)
-}
-// the warp-cooperative kernel needs the dense-map grid (cell edge = phase-1 radius: a ball touches at most 3 x 3 rows)
-static bool use_wc_main(const Ctx* c, bool first_iteration) {
-  const int v = main_variant_env();
-  if (!(c->grid.gate1_d2 < c->grid.gate_d2)) return false;
-  return v == 2 || (v == 3 && !first_iteration);
-}
-// the split path packs two flag bits into a neighbour index and lets the leftover kernel scan the per-block leftover counts
-// in shared memory: maps below 2^29 points, sweeps below 64 x 8191 points, dense-map grid
-static bool use_split_main(const Ctx* c, int n) {
-  return main_variant_env() == 4 && c->n_map < (1 << 29) && div_up(n, SEARCH_THREADS) + 1 <= LEFT_OFF_CAP;
-}
-static cudaError_t wc_prepare() {
-  static const cudaError_t rc = cudaFuncSetAttribute(s2m_main_wc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)WC_SMEM_BYTES);
-  return rc;
-}
-
+// device scratch shared by both entry points.  fail_buf: fail_seg[main_blocks][S2M_THREADS] | fail_off[main_blocks + 1] |
+// block_nfail[main_blocks] | fail_total[1]; block_counter: word 0 the main kernel's ticket, word 1 the leftover kernel's.
 static int prepare_args(Ctx* c, const float4* scan4, int n, S2mArgs& A, int& main_blocks, int& left_blocks) {
-  const bool pw = use_pw_main(c);
-  const bool split = use_split_main(c, n);
-  main_blocks = pw ? div_up(n, 32) : div_up(n, S2M_THREADS);  // partial rows: per chunk or per block
-  const int seg = pw ? 32 : (split ? SEARCH_THREADS : S2M_THREADS);  // leftover segments: per chunk / search block / block
-  const int seg_blocks = div_up(n, seg);
+  A = S2mArgs{};
+  main_blocks = div_up(n, S2M_THREADS);
   // two CTAs per SM: a leftover point is a serial chain of dependent look-ups (~5 us), so they are spread
   // over as many resident warps as possible (one point per warp up to 2368 points)
   left_blocks = c->sm_count * 2;
   LIOGPU_CUDA_OK(c, c->lm_state.reserve(sizeof(LmDevState)));
   LIOGPU_CUDA_OK(c, c->partials.reserve(((size_t)main_blocks + left_blocks) * S2M_SUMS * sizeof(double)));
-  LIOGPU_CUDA_OK(c, c->fail_buf.reserve(((size_t)seg_blocks * seg + 2 * (size_t)seg_blocks + 64) * sizeof(int)));
+  LIOGPU_CUDA_OK(c, c->fail_buf.reserve(((size_t)main_blocks * S2M_THREADS + 2 * (size_t)main_blocks + 64) * sizeof(int)));
   if (!c->block_counter.p) {
     LIOGPU_CUDA_OK(c, c->block_counter.reserve(64));
     LIOGPU_CUDA_OK(c, cudaMemsetAsync(c->block_counter.p, 0, 64, c->stream));
@@ -1628,16 +1405,13 @@ static int prepare_args(Ctx* c, const float4* scan4, int n, S2mArgs& A, int& mai
   A.partials_left = A.partials_main + (size_t)main_blocks * S2M_SUMS;
   int* fb = c->fail_buf.as<int>();
   A.fail_seg = fb;
-  A.seg_stride = seg;
-  A.seg_blocks = seg_blocks;
   // LIOGPU_COLLECT_MOVE (metres) overrides the threshold of the collecting walk: 0 = never collect, a huge value = every
   // seeded iteration collects (tests/test_gpu_variants.py uses both to exercise the list-overflow fallback)
   static const float collect_move = [] { const char* e = getenv("LIOGPU_COLLECT_MOVE"); return e ? (float)atof(e) : S2M_COLLECT_MOVE; }();
   A.collect_move = collect_move;
-  A.queue = c->block_counter.as<unsigned>() + 4;
-  A.fail_off = fb + (size_t)seg_blocks * seg;
-  A.block_nfail = A.fail_off + seg_blocks + 1;
-  A.fail_total = A.block_nfail + seg_blocks;
+  A.fail_off = fb + (size_t)main_blocks * S2M_THREADS;
+  A.block_nfail = A.fail_off + main_blocks + 1;
+  A.fail_total = A.block_nfail + main_blocks;
   A.ticket = c->block_counter.as<unsigned>();
   LIOGPU_CUDA_OK(c, c->prev_nn.reserve((size_t)5 * (size_t)(n > 0 ? n : 1) * sizeof(int)));
   A.prev_nn = c->prev_nn.as<int>();
@@ -1843,9 +1617,6 @@ static int scan2map_legacy_dev(Ctx* c, const float4* scan4, int n, float pose_io
   // chunk of 5 spends two launch pairs of ~5 us per scan on nothing — was tried: a misprediction costs a second host
   // round trip, and the batch-mapping throughput moved by +0.5 % (6,362 vs 6,331 scans/s, 8 workers on one GPU).)
   const int S2M_CHUNK = 5;
-  const bool pw = use_pw_main(c);
-  const int pw_grid = pw_grid_size(c, main_blocks);
-  LIOGPU_CUDA_OK(c, wc_prepare());
   int launched = 0;
   float prof_main_ms = 0.f, prof_left_ms = 0.f;
   int prof_main_n = 0, prof_left_n = 0;
@@ -1862,15 +1633,7 @@ static int scan2map_legacy_dev(Ctx* c, const float4* scan4, int n, float pose_io
     for (int it = 0; it < todo; ++it) {
       const bool first = launched + it == 0;
       if (prof) LIOGPU_CUDA_OK(c, cudaEventRecord(c->prof_ev[3 * it], c->stream));
-      if (two_phase || !first) {
-        if (pw) LIOGPU_CUDA_OK(c, launch_pdl(s2m_main_pw_kernel, pw_grid, S2M_THREADS, c->stream, A));
-        else if (use_split_main(c, n)) {
-          LIOGPU_CUDA_OK(c, launch_pdl(s2m_search_kernel, A.seg_blocks, SEARCH_THREADS, c->stream, A));
-          LIOGPU_CUDA_OK(c, launch_pdl(s2m_fit_kernel, main_blocks, S2M_THREADS, c->stream, A));
-          c->launches++;
-        } else if (use_wc_main(c, first)) LIOGPU_CUDA_OK(c, launch_pdl(s2m_main_wc_kernel, main_blocks, S2M_THREADS, c->stream, A, WC_SMEM_BYTES));
-        else LIOGPU_CUDA_OK(c, launch_pdl(s2m_main_kernel, main_blocks, S2M_THREADS, c->stream, A));
-      }
+      if (two_phase || !first) LIOGPU_CUDA_OK(c, launch_pdl(s2m_main_kernel, main_blocks, S2M_THREADS, c->stream, A));
       if (prof) LIOGPU_CUDA_OK(c, cudaEventRecord(c->prof_ev[3 * it + 1], c->stream));
       LIOGPU_CUDA_OK(c, launch_pdl(s2m_left_kernel, left_blocks, LEFT_THREADS, c->stream, A));
       if (prof) LIOGPU_CUDA_OK(c, cudaEventRecord(c->prof_ev[3 * it + 2], c->stream));
@@ -1952,17 +1715,7 @@ int surf_optimization_dev(Ctx* c, const float4* scan4, int n, const float* pose6
                        c->dbg_flag.as<unsigned char>(), c->dbg_tie.as<unsigned char>()};
   A.mode = 1;
   LIOGPU_CUDA_OK(c, cudaEventRecord(c->ev0, c->stream));
-  if (A.g.gate1_d2 < A.g.gate_d2) {
-    if (use_pw_main(c)) s2m_main_pw_kernel<<<pw_grid_size(c, main_blocks), S2M_THREADS, 0, c->stream>>>(A);
-    else if (use_split_main(c, n)) {
-      s2m_search_kernel<<<A.seg_blocks, SEARCH_THREADS, 0, c->stream>>>(A);
-      s2m_fit_kernel<<<main_blocks, S2M_THREADS, 0, c->stream>>>(A);
-      c->launches++;
-    } else if (use_wc_main(c, false)) {
-      LIOGPU_CUDA_OK(c, wc_prepare());
-      s2m_main_wc_kernel<<<main_blocks, S2M_THREADS, WC_SMEM_BYTES, c->stream>>>(A);
-    } else s2m_main_kernel<<<main_blocks, S2M_THREADS, 0, c->stream>>>(A);
-  }
+  if (A.g.gate1_d2 < A.g.gate_d2) s2m_main_kernel<<<main_blocks, S2M_THREADS, 0, c->stream>>>(A);
   s2m_left_kernel<<<left_blocks, LEFT_THREADS, 0, c->stream>>>(A);
   c->launches += 2;
   LIOGPU_CUDA_OK(c, cudaGetLastError());

@@ -293,8 +293,19 @@ def test_full_size_config4_voxel_5M(gpu, oracle):
 
 
 def test_large_scale_1p2M_queries_1p4M_map(oracle):
-    # beyond BASELINE sizes: 1.2 M sweep points (more than 4096 thread blocks: the leftover kernel's segment-offset
-    # table no longer fits its shared-memory fast path) against a 1.4 M-point map; spot-checked against the oracle
+    # 1.2 M points = 4,688 main-kernel blocks: the leftover kernel derives the segment offsets in shared memory
+    large_scale_registration(oracle, 1_200_000)
+
+
+def test_large_scale_2p4M_queries_1p4M_map(oracle):
+    # above 2,096,896 points (more than LEFT_OFF_CAP - 1 = 8191 main-kernel blocks of 256) the leftover kernel's
+    # segment-offset table no longer fits its shared memory: the main kernel's last block scans the offsets into global
+    # memory and the leftover kernel reads them there
+    large_scale_registration(oracle, 2_400_000)
+
+
+def large_scale_registration(oracle, n_q):
+    # beyond BASELINE sizes: n_q sweep points against a 1.4 M-point map; spot-checked against the oracle
     from lio_slam_b200.liogpu import LioGpu
     rng = np.random.default_rng(77)
 
@@ -309,7 +320,7 @@ def test_large_scale_1p2M_queries_1p4M_map(oracle):
     try:
         map4, _ = g.voxel_downsample(raw, 0.2)
         assert map4.shape[0] > 1_000_000
-        q = np.column_stack([surfaces(1_200_000, 0.02), np.ones(1_200_000)]).astype(np.float32)
+        q = np.column_stack([surfaces(n_q, 0.02), np.ones(n_q)]).astype(np.float32)
         q = q[rng.permutation(q.shape[0])]
         pose = np.array([0.002, -0.003, 0.004, 0.05, -0.04, 0.02], np.float32)
         g.set_local_map(map4)
@@ -327,7 +338,8 @@ def test_large_scale_1p2M_queries_1p4M_map(oracle):
         pose_g, _, info = g.scan2map(q, pose)
         assert info["iterations"] == ref_info["iterations"] and np.array_equal(info["nsel_hist"], ref_info["nsel_hist"])
         assert np.abs(pose_g[:3] - ref_pose[:3]).max() <= 1e-5 and np.abs(pose_g[3:] - ref_pose[3:]).max() <= 1e-4
-        print("1.2M x", map4.shape[0], "iterations", info["iterations"], "gpu loop ms", info["gpu_ms"], "bit-equal pose", np.array_equal(pose_g, ref_pose))
+        print(n_q, "x", map4.shape[0], "iterations", info["iterations"], "gpu loop ms", info["gpu_ms"], "bit-equal pose", np.array_equal(pose_g, ref_pose),
+              "leftovers per iteration", info["leftover_hist"].tolist())
     finally:
         g.close()
 
