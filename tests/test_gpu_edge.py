@@ -138,9 +138,7 @@ def test_deskew_corner_cases(oracle, world):
                               kw["lidar_min_left"], kw["lidar_min_right"], kw["lidar_max_range"], kw["lidar_max_intensity"])
             want = oracle.deskew(sc, dp, t_scan, *imu, enabled)
             got, st = g.deskew(sc, t_scan, *imu, enabled)
-            assert got.shape == want.shape
-            if want.shape[0]:
-                assert np.abs(got - want).max() <= 1e-5
+            assert biteq(got, want)
             return want.shape[0]
         finally:
             g.close()
@@ -156,6 +154,88 @@ def test_deskew_corner_cases(oracle, world):
     assert run(base, (imu_t, rx, ry, rz), t_scan=t0 - 10.0) > 0
     # empty input
     assert run(base, (imu_t, rx, ry, rz), sc=scan[:0]) == 0
+
+
+DESKEW_BASE = dict(n_scan=32, downsample_rate=1, point_filter_num=1, lidar_min_front=2.0, lidar_min_back=10.0,
+                   lidar_min_left=2.0, lidar_min_right=2.0, lidar_max_range=100.0, lidar_max_intensity=90.0)
+
+
+def deskew_vs_oracle(oracle, scan, t_scan, imu, enabled=True, **over):
+    """liogpu_deskew on a fresh context and oracle.deskew with the same parameters -> (gpu, oracle); bit-equal"""
+    from lio_slam_b200.liogpu import LioGpu
+    from oracle.oracle import DeskewParams
+    kw = dict(DESKEW_BASE, **over)
+    g = LioGpu(**kw)
+    try:
+        want = oracle.deskew(scan, DeskewParams(*kw.values()), t_scan, *imu, enabled)
+        got, st = g.deskew(scan, t_scan, *imu, enabled)
+    finally:
+        g.close()
+    assert st == 0 and biteq(got, want)
+    return got, want
+
+
+def test_deskew_first_survivor_in_a_later_block(oracle, world):
+    """the first surviving point fixes transStartInverse for the whole sweep; the flag kernel finds it with atomicMin.
+    Here points 0..4999 fail the range gate or the crop box, so it sits in block 19 (5,001 with point_filter_num 3)"""
+    scan = synth.make_scan(world, synth.path_pose(2.5), 32, seed=41, cols=900).copy()
+    for f in ("x", "y", "z"):
+        scan[f][:2500] *= np.float32(1000.0)    # beyond lidarMaxRange
+        scan[f][2500:5000] *= np.float32(1e-3)  # inside the vehicle's crop box
+    t0 = 300.0
+    imu = synth.make_imu_table(t0, seed=4)
+    got, want = deskew_vs_oracle(oracle, scan, t0, imu, point_filter_num=3)
+    p = synth.to_packed(scan)
+    rng_ok = np.sqrt((p[:, :3].astype(np.float64) ** 2).sum(axis=1)) <= 100.0
+    x, y = p[:, 0], p[:, 1]
+    crop = (y < 2.0) & (-10.0 < y) & (x < 2.0) & (-2.0 < x)
+    survives = rng_ok & ~crop & (p[:, 3] <= 90.0) & (np.arange(p.shape[0]) % 3 == 0)
+    first = int(np.argmax(survives))
+    assert first >= 19 * 256 and want.shape[0] > 1000
+    # the first survivor is deskewed by its own rotation and transStartInverse: the identity up to rounding
+    assert np.abs(want[0, :3] - p[first, :3]).max() <= 1e-5 * np.abs(p[first, :3]).max()
+
+
+def test_deskew_permuted_sweep(oracle, world):
+    """point order that is not column-major: the first survivor and every point's IMU row come from arbitrary places"""
+    scan = synth.make_scan(world, synth.path_pose(4.0), 32, seed=42, cols=900)
+    scan = scan[np.random.default_rng(6).permutation(scan.shape[0])]
+    t0 = 301.0
+    got, want = deskew_vs_oracle(oracle, scan, t0, synth.make_imu_table(t0, seed=5), point_filter_num=2)
+    assert want.shape[0] > 5000
+
+
+def test_deskew_imu_table_at_its_limit(oracle, world):
+    """2,000 IMU rows (imuQueLength), the sweep over the last ten, so findRotation scans about 1,990 rows per point;
+    2,001 rows are refused"""
+    from lio_slam_b200.liogpu import E_INVALID, LioGpu, LioGpuError
+    rng = np.random.default_rng(12)
+    dt, t0 = 0.01, 500.0
+    t = t0 - 1990 * dt + dt * np.arange(2000)                 # the last row at t0 + 0.09, inside the 0.1 s sweep
+    rates = np.c_[0.2 * np.sin(2 * np.pi * 0.3 * t), 0.2 * np.cos(2 * np.pi * 0.2 * t), 0.6 + rng.normal(0, 1e-3, 2000)]
+    rot = np.vstack([np.zeros(3), np.cumsum(rates[1:] * dt, axis=0)])
+    imu = (t, rot[:, 0].copy(), rot[:, 1].copy(), rot[:, 2].copy())
+    scan = synth.make_scan(world, synth.path_pose(5.0), 32, seed=43, cols=900)
+    got, want = deskew_vs_oracle(oracle, scan, t0, imu)
+    assert want.shape[0] > 5000
+    longer = tuple(np.r_[a[:1] - (dt if k == 0 else 0.0), a] for k, a in enumerate(imu))
+    assert longer[0].shape[0] == 2001
+    g = LioGpu(**DESKEW_BASE)
+    try:
+        with pytest.raises(LioGpuError) as e:
+            g.deskew(scan, t0, *longer, True)
+        assert e.value.status == E_INVALID
+    finally:
+        g.close()
+
+
+def test_deskew_enabled_without_imu_rows(oracle, world):
+    """n_imu == 0 with deskew on: imuAvailable is false, so the points pass through the crop and decimation unchanged"""
+    scan = synth.make_scan(world, synth.path_pose(6.0), 32, seed=44, cols=600)
+    empty = tuple(np.zeros(0, np.float64) for _ in range(4))
+    got, want = deskew_vs_oracle(oracle, scan, 700.0, empty, point_filter_num=2)
+    off, _ = deskew_vs_oracle(oracle, scan, 700.0, synth.make_imu_table(700.0, seed=1), enabled=False, point_filter_num=2)
+    assert want.shape[0] > 1000 and biteq(got, off)
 
 
 def test_context_reuse_and_errors(gpu, oracle, small_case):

@@ -335,13 +335,33 @@ def test_deskew_parity(oracle, world, cfg):
                           kw["lidar_max_intensity"])
         want = oracle.deskew(scan, dp, t0, imu_t, rx, ry, rz, True)
         got, st = g.deskew(scan, t0, imu_t, rx, ry, rz, True)
-        assert got.shape == want.shape and want.shape[0] > 1000
-        assert np.abs(got - want).max() <= 1e-5
-        print("deskew bit-equal:", np.array_equal(bits(got), bits(want)), "survivors", want.shape[0], "of", scan.shape[0])
+        assert want.shape[0] > 1000
+        assert_biteq(got, want, "deskew")
         # deskewFlag == -1 / no IMU: crop + decimation only, points unchanged
         want0 = oracle.deskew(scan, dp, t0, imu_t, rx, ry, rz, False)
         got0, _ = g.deskew(scan, t0, imu_t, rx, ry, rz, False)
         assert_biteq(got0, want0, "passthrough")
+    finally:
+        g.close()
+
+
+@pytest.mark.parametrize("beams", [64, 128])
+def test_deskew_full_sweep_parity(oracle, world, beams):
+    """a whole 1800-column sweep (115,200 / 230,400 points, 450 / 900 blocks of the flag and apply kernels)"""
+    from lio_slam_b200.liogpu import LioGpu
+    from oracle.oracle import DeskewParams
+    kw = dict(n_scan=beams, downsample_rate=1, point_filter_num=1, lidar_min_front=2.0, lidar_min_back=10.0,
+              lidar_min_left=2.0, lidar_min_right=2.0, lidar_max_range=100.0, lidar_max_intensity=90.0)
+    g = LioGpu(**kw)
+    try:
+        scan = synth.make_scan(world, synth.path_pose(3.0), beams, seed=78, cols=1800)
+        assert scan.shape[0] == beams * 1800
+        t0 = 1700000000.75
+        imu = synth.make_imu_table(t0, seed=9)
+        want = oracle.deskew(scan, DeskewParams(*kw.values()), t0, *imu, True)
+        got, st = g.deskew(scan, t0, *imu, True)
+        assert st == 0 and want.shape[0] > scan.shape[0] // 2
+        assert_biteq(got, want, f"deskew {beams}-beam sweep")
     finally:
         g.close()
 
