@@ -285,6 +285,30 @@ int liogpu_icp_align(liogpu_ctx* ctx, const void* source_xyzi, int n_source, int
                      const void* target_xyzi, int n_target, int target_stride, const liogpu_icp_params* params,
                      float final_transformation[16], liogpu_icp_info* info);
 
+typedef struct liogpu_loop_icp_result {
+  int   n_source, n_target;              /* cureKeyframeCloud / prevKeyframeCloud after downSizeFilterICP (MO:1102-1103) */
+  int   source_overflow, target_overflow;  /* VoxelGrid overflow guard (q4) fired on that submap */
+  int   rejected_by_size;                /* n_source < 300 || n_target < 1000 (MO:1104): ICP not run, icp zeroed, T = I */
+  float final_transformation[16];        /* icp.getFinalTransformation(), row-major */
+  liogpu_icp_info icp;                   /* as liogpu_icp_align fills it; icp.gpu_ms = 0 (per-pair device time is not
+                                            separable) */
+  int   reserved[4];
+} liogpu_loop_icp_result;
+
+/* loopFindNearKeyframes (MO:1360-1383) for both ends of n_pairs candidate pairs, followed by the ICP of MO:1104-1123 for
+ * each pair.  Keyframe ids are indices into key_pose6s (n_key x 6, cloudKeyPoses6D: roll, pitch, yaw, x, y, z).  The
+ * window [key - search_num, key + search_num] is clamped to [0, n_key).  key_cur uses search_num 0, key_pre uses
+ * search_num, and both submaps are voxelised at icp_leaf (loopClosureICPSurfLeafSize, > 0).  Every key must lie in
+ * [0, n_key) (LIOGPU_E_INVALID) and every id of every window must have been put (LIOGPU_E_NO_KEYFRAME); both are checked
+ * before any work is done.  The submaps never leave the device.  One params struct for all pairs.  results[j] are
+ * bit-equal to liogpu_merge_keyframes of the two windows followed by liogpu_icp_align on the results, whatever the
+ * batch around pair j.  The registration's local map and index and the resident cloud are left untouched.
+ * The acceptance test of MO:1123 (converged && fitness <= historyKeyframeFitnessScore) stays with the caller.
+ * liogpu_last_gpu_ms covers the whole call. */
+int liogpu_loop_closure_icp_batch(liogpu_ctx* ctx, const int* key_cur, const int* key_pre, int n_pairs,
+                                  const float* key_pose6s, int n_key, int search_num, float icp_leaf,
+                                  const liogpu_icp_params* params, liogpu_loop_icp_result* results);
+
 /* SCManager::makeScancontext (include/Scancontext.cpp:151-195) and the ring / sector keys (:198-225) that
  * makeAndSaveScancontextAndKeys stores at every keyframe (MO:2151-2166).  desc is the 20 x 60 MatrixXd, row-major
  * [ring][sector]; lidar_height = LIDAR_HEIGHT (Scancontext.h:80: 2.0), max_radius = PC_MAX_RADIUS (:84: 80.0).

@@ -4,6 +4,7 @@
 #include "common.cuh"
 
 #include <cmath>
+#include <cstdlib>
 #include <cstring>
 #include <new>
 
@@ -237,7 +238,7 @@ int liogpu_create(liogpu_ctx** out, const liogpu_params* params) {
                       &c.tile_hist, &c.tile_pts, &c.tile_out, &c.dbg_idx, &c.dbg_d2, &c.dbg_coeff, &c.dbg_flag, &c.dbg_tie,
                       &c.imu_tab, &c.dsk_flags, &c.dsk_scan, &c.lm_flag, &c.lm_pos, &c.lm_a, &c.lm_b, &c.lm_md, &c.lm_left,
                       &c.lm_out, &c.lm_stats, &c.sor_setup, &c.sor_sorted, &c.sor_cell_start, &c.kf_tab,
-                      &c.sc_q, &c.sc_part, &c.sc_cand, &c.sc_out};
+                      &c.sc_q, &c.sc_part, &c.sc_cand, &c.sc_out, &c.lc_src, &c.lc_tgt, &c.lc_tab};
     for (DevBuf* b : bufs) { b->stream = c.stream; b->async = true; }
   }
   // scratch hint of allocateMemory (mapOptmization.cpp:333-335)
@@ -264,7 +265,8 @@ void liogpu_destroy(liogpu_ctx* ctx) {
                     &c.vox_setup, &c.grid_setup, &c.minmax, &c.lm_state, &c.partials, &c.block_counter, &c.misc,
                     &c.fail_buf, &c.prev_nn, &c.hopeless, &c.fz_rows, &c.fz_left, &c.fz_lb, &c.fz_probe, &c.tile_plan, &c.tile_hist, &c.tile_pts, &c.tile_out, &c.dbg_idx, &c.dbg_d2, &c.dbg_coeff, &c.dbg_flag, &c.dbg_tie, &c.imu_tab, &c.dsk_flags, &c.dsk_scan,
                     &c.lm_flag, &c.lm_pos, &c.lm_a, &c.lm_b, &c.lm_md, &c.lm_left, &c.lm_out, &c.lm_stats, &c.sor_setup,
-                    &c.sor_sorted, &c.sor_cell_start, &c.sc_q, &c.sc_part, &c.sc_cand, &c.sc_out};
+                    &c.sor_sorted, &c.sor_cell_start, &c.sc_q, &c.sc_part, &c.sc_cand, &c.sc_out, &c.lc_src, &c.lc_tgt,
+                    &c.lc_tab};
   for (DevBuf* b : bufs) b->release();
   sc_release(&c);
   for (auto& kv : c.keyframes) kv.second.first.release();
@@ -700,6 +702,145 @@ int liogpu_icp_align(liogpu_ctx* ctx, const void* source_xyzi, int n_source, int
   rc = load_cloud(c, target_xyzi, n_target, target_stride, c->lm_out);
   if (rc) return rc;
   return icp_align_dev(c, c->lm_b.as<float4>(), n_source, c->lm_out.as<float4>(), n_target, params, final_transformation, info);
+}
+
+}  // extern "C"
+
+namespace {
+
+// grows `b` to `need` bytes keeping its first `used` bytes (stream-ordered, like DevBuf::reserve)
+int reserve_keep(Ctx* c, DevBuf& b, size_t need, size_t used) {
+  if (need <= b.cap) return LIOGPU_OK;
+  const size_t want = need + need / 2 + 4096;
+  void* np_ = nullptr;
+  LIOGPU_CUDA_OK(c, cudaMallocAsync(&np_, want, c->stream));
+  if (used) LIOGPU_CUDA_OK(c, cudaMemcpyAsync(np_, b.p, used, cudaMemcpyDeviceToDevice, c->stream));
+  if (b.p) LIOGPU_CUDA_OK(c, cudaFreeAsync(b.p, c->stream));
+  b.p = np_;
+  b.cap = want;
+  return LIOGPU_OK;
+}
+
+// loopFindNearKeyframes (MO:1360-1383) for the window [key - search_num, key + search_num] ∩ [0, n_key): the
+// liogpu_merge_keyframes pipeline (transform + concatenate + VoxelGrid), the result appended to `arena` at record `used`
+int loop_submap(Ctx* c, int key, int search_num, const float* key_pose6s, int n_key, float leaf, DevBuf& arena, int used,
+                int* m, bool* overflow) {
+  *m = 0;
+  *overflow = false;
+  std::vector<int> ids;
+  std::vector<float> poses;
+  const long long lo = (long long)key - search_num, hi = (long long)key + search_num;
+  for (long long k = lo < 0 ? 0 : lo; k <= hi && k < n_key; ++k) {
+    ids.push_back((int)k);
+    poses.insert(poses.end(), key_pose6s + 6 * k, key_pose6s + 6 * k + 6);
+  }
+  KfTables t;
+  int rc = stage_keyframes(c, "liogpu_loop_closure_icp_batch", ids.data(), poses.data(), (int)ids.size(), t);
+  if (rc || t.total == 0) return rc;
+  const int total = (int)t.total;
+  LIOGPU_CUDA_OK(c, c->lm_a.reserve(t.total * sizeof(float4)));
+  LIOGPU_CUDA_OK(c, launch_transform_multi(c, t.srcs, t.offs, (int)ids.size(), t.poses, t.T12, (long long)total, c->lm_a.as<float4>()));
+  rc = voxel_downsample_dev(c, c->lm_a.as<float4>(), total, leaf, c->lm_out, m, overflow);
+  if (rc) return rc;
+  if (*m == 0) return LIOGPU_OK;
+  rc = reserve_keep(c, arena, ((size_t)used + *m) * sizeof(float4), (size_t)used * sizeof(float4));
+  if (rc) return rc;
+  LIOGPU_CUDA_OK(c, cudaMemcpyAsync(arena.as<float4>() + used, c->lm_out.p, (size_t)*m * sizeof(float4),
+                                    cudaMemcpyDeviceToDevice, c->stream));
+  return LIOGPU_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int liogpu_loop_closure_icp_batch(liogpu_ctx* ctx, const int* key_cur, const int* key_pre, int n_pairs,
+                                  const float* key_pose6s, int n_key, int search_num, float icp_leaf,
+                                  const liogpu_icp_params* params, liogpu_loop_icp_result* results) {
+  NvtxRange nvtx_range_(__func__);
+  int rc = enter(ctx);
+  if (rc) return rc;
+  Ctx* c = &ctx->c;
+  if (n_pairs < 0 || (n_pairs > 0 && (!key_cur || !key_pre || !key_pose6s || !results)) || n_key < 0 || search_num < 0 ||
+      !(icp_leaf > 0.f) || !params || params->max_iterations < 1 || !(params->max_correspondence_distance > 0.f)) {
+    c->err = "liogpu_loop_closure_icp_batch: bad arguments";
+    return LIOGPU_E_INVALID;
+  }
+  for (int j = 0; j < n_pairs; ++j) {
+    if (key_cur[j] < 0 || key_cur[j] >= n_key || key_pre[j] < 0 || key_pre[j] >= n_key) {
+      c->err = "liogpu_loop_closure_icp_batch: key outside [0, n_key)";
+      return LIOGPU_E_INVALID;
+    }
+    const long long lo = (long long)key_pre[j] - search_num, hi = (long long)key_pre[j] + search_num;
+    bool ok = c->keyframes.count(key_cur[j]) != 0;
+    for (long long k = lo < 0 ? 0 : lo; ok && k <= hi && k < n_key; ++k) ok = c->keyframes.count((int)k) != 0;
+    if (!ok) { c->err = "liogpu_loop_closure_icp_batch: unknown keyframe id"; return LIOGPU_E_NO_KEYFRAME; }
+  }
+  for (int j = 0; j < n_pairs; ++j) {
+    std::memset(&results[j], 0, sizeof(results[j]));
+    for (int q = 0; q < 16; ++q) results[j].final_transformation[q] = (q % 5 == 0) ? 1.f : 0.f;
+  }
+  // Pairs go to the device in groups that keep the submaps (and with them the index and per-point buffers) under a
+  // fixed size; every pair's result is independent of the group it lands in.  LIOGPU_LOOP_ICP_GROUP caps the pairs of
+  // a group (tests use it to split small batches).
+  constexpr long long GROUP_POINTS = 1ll << 25;
+  int group_pairs = 1024;
+  if (const char* e = getenv("LIOGPU_LOOP_ICP_GROUP")) {
+    const int v = atoi(e);
+    if (v > 0 && v < group_pairs) group_pairs = v;
+  }
+  LIOGPU_CUDA_OK(c, cudaEventRecord(c->ev0, c->stream));
+  std::vector<int> members, so{0}, to{0};
+  std::vector<float> T;
+  std::vector<liogpu_icp_info> info;
+  auto flush = [&]() -> int {
+    const int n = (int)members.size();
+    if (n == 0) return LIOGPU_OK;
+    T.resize((size_t)n * 16);
+    info.assign(n, liogpu_icp_info{});
+    int r = icp_batch_dev(c, c->lc_src.as<float4>(), so.data(), c->lc_tgt.as<float4>(), to.data(), n, params,
+                          reinterpret_cast<float(*)[16]>(T.data()), info.data());
+    if (r) return r;
+    for (int g = 0; g < n; ++g) {
+      liogpu_loop_icp_result& res = results[members[g]];
+      std::memcpy(res.final_transformation, &T[(size_t)g * 16], 16 * sizeof(float));
+      res.icp = info[g];
+    }
+    members.clear();
+    so.assign(1, 0);
+    to.assign(1, 0);
+    return LIOGPU_OK;
+  };
+  for (int j = 0; j < n_pairs; ++j) {
+    liogpu_loop_icp_result& res = results[j];
+    int ms = 0, mt = 0;
+    bool os = false, ot = false;
+    rc = loop_submap(c, key_cur[j], 0, key_pose6s, n_key, icp_leaf, c->lc_src, so.back(), &ms, &os);       // MO:1102
+    if (rc) return rc;
+    rc = loop_submap(c, key_pre[j], search_num, key_pose6s, n_key, icp_leaf, c->lc_tgt, to.back(), &mt, &ot);  // MO:1103
+    if (rc) return rc;
+    res.n_source = ms;
+    res.n_target = mt;
+    res.source_overflow = os ? 1 : 0;
+    res.target_overflow = ot ? 1 : 0;
+    if (ms < 300 || mt < 1000) {  // MO:1104; the submaps just appended are overwritten by the next pair
+      res.rejected_by_size = 1;
+      continue;
+    }
+    members.push_back(j);
+    so.push_back(so.back() + ms);
+    to.push_back(to.back() + mt);
+    if ((int)members.size() >= group_pairs || (long long)so.back() + to.back() >= GROUP_POINTS) {
+      rc = flush();
+      if (rc) return rc;
+    }
+  }
+  rc = flush();
+  if (rc) return rc;
+  LIOGPU_CUDA_OK(c, cudaEventRecord(c->ev1, c->stream));
+  LIOGPU_CUDA_OK(c, cudaStreamSynchronize(c->stream));
+  cudaEventElapsedTime(&c->last_ms, c->ev0, c->ev1);
+  return LIOGPU_OK;
 }
 
 int liogpu_make_scancontext(liogpu_ctx* ctx, const void* xyzi, int n, int stride, double lidar_height, double max_radius,

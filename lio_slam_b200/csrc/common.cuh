@@ -192,6 +192,9 @@ struct Ctx {
   // loop-closure detection: the descriptor store and the per-call scratch (queries, partial top-k lists, candidates)
   ScStore sc;
   DevBuf sc_q, sc_part, sc_cand, sc_out;
+  // batched loop-closure ICP: the group's source / target submaps (packed float4, one segment per pair) and its
+  // device tables (per-pair offsets, grids, ICP states, reduce partials)
+  DevBuf lc_src, lc_tgt, lc_tab;
 };
 
 #define LIOGPU_CUDA_OK(ctx, expr)                                                        \
@@ -243,6 +246,11 @@ int detect_loop_distance_dev(Ctx* c, const float4* key3d, int n, const double* h
 // --- icp.cu
 int icp_align_dev(Ctx* c, const float4* src, int ns, const float4* tgt, int nt, const liogpu_icp_params* prm,
                   float final_T[16], liogpu_icp_info* info);
+// n pairs at once: pair p's source is src[src_off[p] .. src_off[p+1]), its target tgt[tgt_off[p] .. tgt_off[p+1])
+// (offsets in records, n + 1 entries each, every segment non-empty).  Each pair's result is bit-equal to icp_align_dev
+// on its two segments.
+int icp_batch_dev(Ctx* c, const float4* src, const int* src_off, const float4* tgt, const int* tgt_off, int n,
+                  const liogpu_icp_params* prm, float (*final_T)[16], liogpu_icp_info* info);
 // --- s2m.cu
 int scan2map_dev(Ctx* c, const float4* scan4, int n, float pose_io[6], float matP_io[36], int* degenerate_io,
                  int max_iter, liogpu_s2m_info* info);

@@ -401,6 +401,355 @@ icp_reduce_kernel(const IcpArgs A) {
   }
 }
 
+// ---- many pairs at once (liogpu_loop_closure_icp_batch) ----
+// Every pair keeps its own IcpDevState and its own grid; the search gives each point the same nearest target point as
+// the single-pair kernels (the search is exact, ties go to the lower target index, whatever the grid), and the reduction
+// sums each pair in the exact order of icp_reduce_kernel, so every pair's result is bit-equal to icp_align_dev.
+// The targets of all pairs share one sorted array: key = cell_base[pair] + the cell inside the pair's grid, so a pair's
+// points form one contiguous run and cell_start + cell_base[pair] is that pair's cell_start.
+
+struct IcpbCounters {
+  unsigned n_brute[2];  // exhaustive-search list of the current launch (parity), the other one is cleared for the next
+  int live;             // pairs not yet done
+  int pad;
+};
+
+struct IcpbArgs {
+  const float4* src;        // sources of all pairs, concatenated
+  float4* cur;              // input_transformed, same indexing
+  const float4* tgt;        // targets of all pairs, concatenated
+  const float4* sorted;     // targets in (pair, cell) order, w = bits(index inside the pair's target)
+  const uint32_t* cs;       // cell_start over the concatenated cells
+  const int* sp;            // [n + 1] source offsets
+  const int* tp;            // [n + 1] target offsets
+  const int* rp;            // [n + 1] reduce-block offsets
+  const unsigned* cell_base;
+  const GridParams* gp;
+  IcpDevState* st;
+  IcpbCounters* cnt;
+  int* nn_idx;
+  float* nn_d2;
+  uint32_t* brute;          // [ns] points left to the exhaustive search
+  double* partials;         // [rp[n]][ICP_SUMS]
+  int n, ns;
+  int fitness;
+  int par;                  // launch parity: which n_brute counter this launch uses
+};
+
+// segment of element i: the last p with off[p] <= i (segments are non-empty)
+__device__ __forceinline__ int find_seg(const int* __restrict__ off, int n, int i) {
+  int lo = 0, hi = n - 1;
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (__ldg(off + mid) <= i) lo = mid; else hi = mid - 1;
+  }
+  return lo;
+}
+
+// block per pair: bounding box and finite count of its target, then grid_setup_kernel's choice of grid
+constexpr int BB_THREADS = 256;
+__global__ void __launch_bounds__(BB_THREADS)
+icpb_grid_kernel(const float4* __restrict__ tgt, const int* __restrict__ tp, float cell, unsigned max_cells,
+                 GridParams* __restrict__ gp) {
+  __shared__ float s_mn[3][BB_THREADS / 32], s_mx[3][BB_THREADS / 32];
+  __shared__ int s_cnt[BB_THREADS / 32];
+  const int p = blockIdx.x;
+  float mn[3] = {CUDART_INF_F, CUDART_INF_F, CUDART_INF_F}, mx[3] = {-CUDART_INF_F, -CUDART_INF_F, -CUDART_INF_F};
+  int cnt = 0;
+  for (int t = tp[p] + (int)threadIdx.x; t < tp[p + 1]; t += BB_THREADS) {
+    const float4 q = tgt[t];
+    if (!(isfinite(q.x) && isfinite(q.y) && isfinite(q.z))) continue;
+    mn[0] = fminf(mn[0], q.x); mn[1] = fminf(mn[1], q.y); mn[2] = fminf(mn[2], q.z);
+    mx[0] = fmaxf(mx[0], q.x); mx[1] = fmaxf(mx[1], q.y); mx[2] = fmaxf(mx[2], q.z);
+    ++cnt;
+  }
+  for (int o = 16; o > 0; o >>= 1) {
+    for (int a = 0; a < 3; ++a) {
+      mn[a] = fminf(mn[a], __shfl_xor_sync(0xffffffffu, mn[a], o));
+      mx[a] = fmaxf(mx[a], __shfl_xor_sync(0xffffffffu, mx[a], o));
+    }
+    cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
+  }
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  if (lane == 0) {
+    for (int a = 0; a < 3; ++a) { s_mn[a][w] = mn[a]; s_mx[a][w] = mx[a]; }
+    s_cnt[w] = cnt;
+  }
+  __syncthreads();
+  if (threadIdx.x != 0) return;
+  GridParams g;
+  g.n_points = 0;
+  for (int k = 0; k < BB_THREADS / 32; ++k) {
+    for (int a = 0; a < 3; ++a) { mn[a] = fminf(mn[a], s_mn[a][k]); mx[a] = fmaxf(mx[a], s_mx[a][k]); }
+    g.n_points += s_cnt[k];
+  }
+  if (g.n_points <= 0) { mn[0] = mn[1] = mn[2] = 0.f; mx[0] = mx[1] = mx[2] = 0.f; }
+  float maxabs = 1.0f;
+  for (int a = 0; a < 3; ++a) {
+    maxabs = fmaxf(maxabs, fmaxf(fabsf(mn[a]), fabsf(mx[a])));
+    maxabs = fmaxf(maxabs, mx[a] - mn[a]);
+  }
+  g.ox = mn[0]; g.oy = mn[1]; g.oz = mn[2];
+  float h = cell;
+  for (;;) {
+    const float inv = 1.0f / h;
+    const double nx = floor((double)(mx[0] - mn[0]) * inv) + 1, ny = floor((double)(mx[1] - mn[1]) * inv) + 1,
+                 nz = floor((double)(mx[2] - mn[2]) * inv) + 1;
+    if (nx * ny * nz <= (double)max_cells) {
+      g.nx = (int)nx; g.ny = (int)ny; g.nz = (int)nz;
+      g.h = h; g.inv_h = inv;
+      break;
+    }
+    h *= 2.0f;
+  }
+  g.n_cells = (unsigned)g.nx * (unsigned)g.ny * (unsigned)g.nz;
+  g.slack = maxabs * 9.5367431640625e-07f;  // 2^-20, as grid_setup_kernel
+  g.gate_d2 = 1.0f;
+  g.gate1_d2 = 1.0f;
+  gp[p] = g;
+}
+
+__global__ void __launch_bounds__(256)
+icpb_key_kernel(const float4* __restrict__ tgt, int nt, const int* __restrict__ tp, int n, const GridParams* __restrict__ gp,
+                const unsigned* __restrict__ cell_base, unsigned total_cells, uint32_t* __restrict__ keys,
+                uint32_t* __restrict__ cell_count) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= nt) return;
+  const float4 q = tgt[i];
+  uint32_t key = total_cells;  // non-finite points sort last and are never referenced
+  if (isfinite(q.x) && isfinite(q.y) && isfinite(q.z)) {
+    const int p = find_seg(tp, n, i);
+    const GridParams g = gp[p];
+    const int cx = sor_cell(q.x, g.ox, g.inv_h, g.nx);
+    const int cy = sor_cell(q.y, g.oy, g.inv_h, g.ny);
+    const int cz = sor_cell(q.z, g.oz, g.inv_h, g.nz);
+    key = cell_base[p] + ((uint32_t)cz * (uint32_t)g.ny + (uint32_t)cy) * (uint32_t)g.nx + (uint32_t)cx;
+    atomicAdd(&cell_count[key], 1u);
+  }
+  keys[i] = key;
+}
+
+__global__ void __launch_bounds__(256)
+icpb_gather_kernel(const float4* __restrict__ tgt, const uint32_t* __restrict__ perm, int n_valid, const int* __restrict__ tp,
+                   int n, float4* __restrict__ sorted) {
+  const int j = blockIdx.x * blockDim.x + threadIdx.x;
+  if (j >= n_valid) return;
+  const int src = (int)perm[j];
+  const float4 q = tgt[src];
+  sorted[j] = make_float4(q.x, q.y, q.z, __int_as_float(src - tp[find_seg(tp, n, src)]));
+}
+
+// thread per source point of every live pair: shells 0..2 (icp_nn_kernel); the block's points that need more are then
+// taken warp per point for shells 3..5 (icp_left_kernel), starting from the nearest point the thread already found
+constexpr int NB_THREADS = 128;
+__global__ void __launch_bounds__(NB_THREADS)
+icpb_nn_kernel(const IcpbArgs A) {
+  __shared__ int s_n;
+  __shared__ int s_i[NB_THREADS], s_p[NB_THREADS];
+  __shared__ unsigned long long s_key[NB_THREADS];
+  __shared__ float4 s_pt[NB_THREADS];
+  if (threadIdx.x == 0) {
+    s_n = 0;
+    if (blockIdx.x == 0) A.cnt->n_brute[A.par ^ 1] = 0;  // the next launch's list (this launch's was cleared by the last)
+  }
+  __syncthreads();
+  const int i = blockIdx.x * NB_THREADS + threadIdx.x;
+  if (i < A.ns) {
+    const int p = find_seg(A.sp, A.n, i);
+    const IcpDevState* st = A.st + p;
+    if (A.fitness || !st->done) {
+      float4 q = A.fitness ? A.src[i] : A.cur[i];
+      if (A.fitness || st->iter > 0) {
+        q = se3(A.fitness ? st->finalT : st->T_inc, q);
+        A.cur[i] = q;
+      }
+      if (!(isfinite(q.x) && isfinite(q.y) && isfinite(q.z))) {
+        A.nn_idx[i] = -1;
+        A.nn_d2[i] = CUDART_INF_F;
+      } else {
+        const GridParams g = A.gp[p];
+        const uint32_t* cs = A.cs + A.cell_base[p];
+        const double max_d2 = A.fitness ? CUDART_INF : st->max_d2;
+        const HomeCell hc = home_cell(g, q);
+        Best1 best;
+        best.init();
+        int verdict = 0;
+        for (int R = 0; R < NN_THREAD_SHELLS && verdict == 0; ++R) {
+          const int z0 = max(hc.cz - R, 0), z1 = min(hc.cz + R, g.nz - 1);
+          const int y0 = max(hc.cy - R, 0), y1 = min(hc.cy + R, g.ny - 1);
+          for (int z = z0; z <= z1; ++z)
+            for (int y = y0; y <= y1; ++y) scan_shell_row(A.sorted, cs, g, hc, R, y, z, q, best);
+          verdict = nn_verdict(best, covered_d2(g, hc, R), max_d2);
+        }
+        if (verdict == 0) {
+          const int slot = atomicAdd(&s_n, 1);
+          s_i[slot] = i; s_p[slot] = p; s_key[slot] = best.key; s_pt[slot] = q;
+        } else {
+          A.nn_idx[i] = verdict == 1 ? best.idx() : -1;
+          A.nn_d2[i] = best.d2();
+        }
+      }
+    }
+  }
+  __syncthreads();
+  const int lane = threadIdx.x & 31;
+  for (int e = threadIdx.x >> 5; e < s_n; e += NB_THREADS / 32) {
+    const int i = s_i[e], p = s_p[e];
+    const float4 q = s_pt[e];
+    const GridParams g = A.gp[p];
+    const uint32_t* cs = A.cs + A.cell_base[p];
+    const double max_d2 = A.fitness ? CUDART_INF : A.st[p].max_d2;
+    const HomeCell hc = home_cell(g, q);
+    Best1 best;
+    best.init();
+    if (lane == 0) best.key = s_key[e];
+    Best1 all;
+    all.init();
+    int verdict = 0;
+    for (int R = NN_THREAD_SHELLS; R < NN_WARP_SHELLS && verdict == 0; ++R) {
+      const int side = 2 * R + 1, rows = side * side;
+      for (int r = lane; r < rows; r += 32) {
+        const int z = hc.cz + r / side - R, y = hc.cy + r % side - R;
+        if (z < 0 || z >= g.nz || y < 0 || y >= g.ny) continue;
+        scan_shell_row(A.sorted, cs, g, hc, R, y, z, q, best);
+      }
+      all.key = warp_min_u64(best.key);
+      verdict = nn_verdict(all, covered_d2(g, hc, R), max_d2);
+    }
+    if (lane == 0) {
+      if (verdict == 0) {
+        A.brute[atomicAdd(&A.cnt->n_brute[A.par], 1u)] = (uint32_t)i;
+      } else {
+        A.nn_idx[i] = verdict == 1 ? all.idx() : -1;
+        A.nn_d2[i] = all.d2();
+      }
+    }
+  }
+}
+
+// block per isolated point: one pass over its pair's finite targets (icp_brute_kernel)
+__global__ void __launch_bounds__(BRT)
+icpb_brute_kernel(const IcpbArgs A) {
+  __shared__ unsigned long long sh[BRT / 32];
+  const unsigned n_brute = A.cnt->n_brute[A.par];
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  for (unsigned e = blockIdx.x; e < n_brute; e += gridDim.x) {
+    const uint32_t i = A.brute[e];
+    const int p = find_seg(A.sp, A.n, (int)i);
+    const float4 pt = A.cur[i];
+    const float4* sorted = A.sorted + A.cs[A.cell_base[p]];
+    const int n_points = A.gp[p].n_points;
+    const double max_d2 = A.fitness ? CUDART_INF : A.st[p].max_d2;
+    Best1 best;
+    best.init();
+    for (int base = 0; base < n_points; base += BRT * 8) {
+      float4 q[8];
+#pragma unroll
+      for (int u = 0; u < 8; ++u) {
+        const int t = base + u * BRT + (int)threadIdx.x;
+        q[u] = t < n_points ? __ldg(sorted + t) : make_float4(CUDART_INF_F, 0.f, 0.f, __int_as_float(-1));
+      }
+#pragma unroll
+      for (int u = 0; u < 8; ++u) best.push(sor_d2(pt, q[u]), q[u].w);
+    }
+    const unsigned long long wm = warp_min_u64(best.key);
+    if (lane == 0) sh[w] = wm;
+    __syncthreads();
+    if (w == 0) {
+      unsigned long long v = lane < BRT / 32 ? sh[lane] : ~0ULL;
+      v = warp_min_u64(v);
+      if (lane == 0) {
+        Best1 b;
+        b.key = v;
+        const bool ok = (double)b.d2() <= max_d2;
+        A.nn_idx[i] = ok ? b.idx() : -1;
+        A.nn_d2[i] = b.d2();
+      }
+    }
+    __syncthreads();
+  }
+}
+
+// icp_reduce_kernel for every live pair: pair p owns blocks rp[p] .. rp[p+1] (min(ceil(ns / 256), 256) of them, as the
+// single call launches), the same grid-stride assignment, shuffle tree and fold; the pair's last block runs its tail
+__global__ void __launch_bounds__(RD_THREADS)
+icpb_reduce_kernel(const IcpbArgs A) {
+  __shared__ double sh[RD_THREADS / 32][ICP_SUMS];
+  __shared__ bool s_last;
+  const int p = find_seg(A.rp, A.n, (int)blockIdx.x);
+  IcpDevState* st = A.st + p;
+  if (!A.fitness && st->done) return;
+  const double max_d2 = A.fitness ? CUDART_INF : st->max_d2;
+  const int rb0 = A.rp[p], nblk = A.rp[p + 1] - rb0, lb = (int)blockIdx.x - rb0;
+  const int s0 = A.sp[p], ns = A.sp[p + 1] - s0, t0 = A.tp[p];
+  double acc[ICP_SUMS];
+#pragma unroll
+  for (int q = 0; q < ICP_SUMS; ++q) acc[q] = 0.0;
+  for (int i = lb * RD_THREADS + (int)threadIdx.x; i < ns; i += nblk * RD_THREADS) {
+    const int j = A.nn_idx[s0 + i];
+    const float d2 = A.nn_d2[s0 + i];
+    if (j < 0 || (double)d2 > max_d2) continue;
+    acc[15] += (double)d2;
+    acc[16] += 1.0;
+    if (!A.fitness) {
+      const float4 s = A.cur[s0 + i], t = A.tgt[t0 + j];
+      const double sv[3] = {s.x, s.y, s.z}, tv[3] = {t.x, t.y, t.z};
+#pragma unroll
+      for (int a = 0; a < 3; ++a) {
+        acc[a] += sv[a];
+        acc[3 + a] += tv[a];
+#pragma unroll
+        for (int b = 0; b < 3; ++b) acc[6 + 3 * a + b] += tv[a] * sv[b];
+      }
+    }
+  }
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+#pragma unroll
+  for (int q = 0; q < ICP_SUMS; ++q) {
+    double v = acc[q];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
+    if (lane == 0) sh[w][q] = v;
+  }
+  __syncthreads();
+  if (threadIdx.x < ICP_SUMS) {
+    double v = 0.0;
+    for (int k = 0; k < RD_THREADS / 32; ++k) v += sh[k][threadIdx.x];
+    A.partials[(size_t)blockIdx.x * ICP_SUMS + threadIdx.x] = v;
+  }
+  __threadfence();
+  __syncthreads();
+  if (threadIdx.x == 0) s_last = atomicAdd(&st->ticket, 1u) == (unsigned)nblk - 1;
+  __syncthreads();
+  if (!s_last) return;
+  __threadfence();
+  {
+    const int q = threadIdx.x & 31, slice = threadIdx.x >> 5;
+    double v = 0.0;
+    if (q < ICP_SUMS) {
+      for (int b = slice; b < nblk; b += RD_THREADS / 32) v += A.partials[(size_t)(rb0 + b) * ICP_SUMS + q];
+      sh[slice][q] = v;
+    }
+  }
+  __syncthreads();
+  if (threadIdx.x < ICP_SUMS) {
+    double v = 0.0;
+    for (int k = 0; k < RD_THREADS / 32; ++k) v += sh[k][threadIdx.x];
+    sh[0][threadIdx.x] = v;
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    if (A.fitness) {
+      st->fit_nr = (int)sh[0][16];
+      st->fitness = sh[0][16] > 0.0 ? sh[0][15] / sh[0][16] : DBL_MAX;
+    } else {
+      icp_finalize(st, sh[0]);
+      if (st->done) atomicSub(&A.cnt->live, 1);
+    }
+    st->ticket = 0;
+  }
+}
+
 }  // namespace
 
 // source / target: packed float4 on device.  The target's grid index is built into the outlier filter's buffers
@@ -475,6 +824,145 @@ int icp_align_dev(Ctx* c, const float4* src, int ns, const float4* tgt, int nt, 
   info->fitness_score = h->fitness;
   info->last_mse = h->last_mse;
   info->gpu_ms = c->last_ms;
+  return LIOGPU_OK;
+}
+
+
+int icp_batch_dev(Ctx* c, const float4* src, const int* so, const float4* tgt, const int* to, int n,
+                  const liogpu_icp_params* prm, float (*final_T)[16], liogpu_icp_info* info) {
+  if (n <= 0) return LIOGPU_OK;
+  const int ns = so[n], nt = to[n];
+  std::vector<int> rp(n + 1, 0);
+  for (int p = 0; p < n; ++p) {
+    const int blocks = div_up(so[p + 1] - so[p], RD_THREADS);
+    rp[p + 1] = rp[p] + (blocks < 256 ? blocks : 256);
+  }
+  // device tables: sp | tp | rp | cell_base | gp | st | counters | partials
+  auto up256 = [](size_t b) { return (b + 255) & ~(size_t)255; };
+  const size_t o_tp = up256((size_t)(n + 1) * sizeof(int)), o_rp = o_tp + o_tp, o_cb = o_rp + o_tp;
+  const size_t o_gp = o_cb + up256((size_t)n * sizeof(unsigned)), o_st = o_gp + up256((size_t)n * sizeof(GridParams));
+  const size_t o_cnt = o_st + up256((size_t)n * sizeof(IcpDevState)), o_part = o_cnt + 256;
+  LIOGPU_CUDA_OK(c, c->lc_tab.reserve(o_part + (size_t)rp[n] * ICP_SUMS * sizeof(double)));
+  char* d = (char*)c->lc_tab.p;
+  std::vector<char> h(o_part, 0);
+  memcpy(h.data(), so, (size_t)(n + 1) * sizeof(int));
+  memcpy(h.data() + o_tp, to, (size_t)(n + 1) * sizeof(int));
+  memcpy(h.data() + o_rp, rp.data(), (size_t)(n + 1) * sizeof(int));
+  IcpDevState* hs = reinterpret_cast<IcpDevState*>(h.data() + o_st);
+  for (int p = 0; p < n; ++p) {  // as icp_align_dev
+    IcpDevState& s = hs[p];
+    for (int q = 0; q < 16; ++q) s.T_inc[q] = s.finalT[q] = (q % 5 == 0) ? 1.f : 0.f;
+    s.prev_mse = DBL_MAX;
+    s.max_d2 = (double)prm->max_correspondence_distance * (double)prm->max_correspondence_distance;
+    s.rot_thr = 1.0 - prm->transformation_epsilon;
+    s.trans_thr = prm->transformation_epsilon;
+    s.rel_thr = prm->euclidean_fitness_epsilon;
+    s.abs_thr = 1e-12;
+    s.max_iter = prm->max_iterations;
+  }
+  reinterpret_cast<IcpbCounters*>(h.data() + o_cnt)->live = n;
+  LIOGPU_CUDA_OK(c, cudaMemcpyAsync(d, h.data(), o_part, cudaMemcpyHostToDevice, c->stream));
+  IcpbArgs A;
+  A.src = src; A.tgt = tgt; A.n = n; A.ns = ns;
+  A.sp = reinterpret_cast<const int*>(d); A.tp = reinterpret_cast<const int*>(d + o_tp);
+  A.rp = reinterpret_cast<const int*>(d + o_rp);
+  unsigned* d_cb = reinterpret_cast<unsigned*>(d + o_cb);
+  A.cell_base = d_cb;
+  GridParams* d_gp = reinterpret_cast<GridParams*>(d + o_gp);
+  A.gp = d_gp;
+  A.st = reinterpret_cast<IcpDevState*>(d + o_st);
+  A.cnt = reinterpret_cast<IcpbCounters*>(d + o_cnt);
+  A.partials = reinterpret_cast<double*>(d + o_part);
+
+  // one segmented grid index over all targets.  The cell count per pair is capped so that the concatenated cells stay
+  // within 2^28 (the grid's cell size never changes a result)
+  const float cell = prm->cell_size > 0.f ? prm->cell_size : 0.5f;
+  const unsigned max_cells = (unsigned)((1u << 28) / (unsigned)n) < (1u << 25) ? (unsigned)((1u << 28) / (unsigned)n) : (1u << 25);
+  icpb_grid_kernel<<<n, BB_THREADS, 0, c->stream>>>(tgt, A.tp, cell, max_cells, d_gp);
+  c->launches++;
+  LIOGPU_CUDA_OK(c, cudaGetLastError());
+  std::vector<GridParams> hg(n);
+  LIOGPU_CUDA_OK(c, cudaMemcpyAsync(hg.data(), d_gp, (size_t)n * sizeof(GridParams), cudaMemcpyDeviceToHost, c->stream));
+  LIOGPU_CUDA_OK(c, cudaStreamSynchronize(c->stream));
+  std::vector<unsigned> cb(n);
+  unsigned long long total_cells = 0;
+  int n_valid = 0;
+  for (int p = 0; p < n; ++p) {
+    cb[p] = (unsigned)total_cells;
+    total_cells += hg[p].n_cells;
+    n_valid += hg[p].n_points;
+  }
+  if (total_cells > (1ull << 30)) { c->err = "icp batch: grid too large"; return LIOGPU_E_INVALID; }
+  LIOGPU_CUDA_OK(c, cudaMemcpyAsync(d_cb, cb.data(), (size_t)n * sizeof(unsigned), cudaMemcpyHostToDevice, c->stream));
+  LIOGPU_CUDA_OK(c, c->keys0.reserve((size_t)nt * 4));
+  LIOGPU_CUDA_OK(c, c->keys1.reserve((size_t)nt * 4));
+  LIOGPU_CUDA_OK(c, c->vals0.reserve((size_t)nt * 4));
+  LIOGPU_CUDA_OK(c, c->vals1.reserve((size_t)nt * 4));
+  LIOGPU_CUDA_OK(c, c->sor_sorted.reserve((size_t)nt * sizeof(float4)));
+  LIOGPU_CUDA_OK(c, c->sor_cell_start.reserve((size_t)(total_cells + 2) * sizeof(uint32_t)));
+  uint32_t* cell_start = c->sor_cell_start.as<uint32_t>();
+  LIOGPU_CUDA_OK(c, cudaMemsetAsync(cell_start, 0, (size_t)(total_cells + 2) * sizeof(uint32_t), c->stream));
+  icpb_key_kernel<<<div_up(nt, 256), 256, 0, c->stream>>>(tgt, nt, A.tp, n, d_gp, d_cb, (unsigned)total_cells,
+                                                         c->keys0.as<uint32_t>(), cell_start);
+  c->launches++;
+  LIOGPU_CUDA_OK(c, exclusive_scan_u32(c, cell_start, cell_start, (int)total_cells + 1, nullptr));
+  int bits = 0;
+  while (bits < 32 && (total_cells >> bits) != 0ull) ++bits;
+  uint32_t *skeys = nullptr, *sperm = nullptr;
+  LIOGPU_CUDA_OK(c, radix_sort_pairs(c, nt, bits, nullptr, &skeys, &sperm));
+  if (n_valid > 0) {
+    icpb_gather_kernel<<<div_up(n_valid, 256), 256, 0, c->stream>>>(tgt, sperm, n_valid, A.tp, n, c->sor_sorted.as<float4>());
+    c->launches++;
+  }
+  A.sorted = c->sor_sorted.as<float4>();
+  A.cs = cell_start;
+
+  LIOGPU_CUDA_OK(c, c->lm_a.reserve((size_t)ns * sizeof(float4)));
+  LIOGPU_CUDA_OK(c, c->lm_flag.reserve((size_t)ns * sizeof(int)));
+  LIOGPU_CUDA_OK(c, c->lm_md.reserve((size_t)ns * sizeof(float)));
+  LIOGPU_CUDA_OK(c, c->lm_left.reserve((size_t)ns * sizeof(uint32_t)));
+  A.cur = c->lm_a.as<float4>();
+  A.nn_idx = c->lm_flag.as<int>(); A.nn_d2 = c->lm_md.as<float>();
+  A.brute = c->lm_left.as<uint32_t>();
+  A.fitness = 0;
+  A.par = 0;
+  LIOGPU_CUDA_OK(c, cudaMemcpyAsync(A.cur, src, (size_t)ns * sizeof(float4), cudaMemcpyDeviceToDevice, c->stream));
+  const int CHUNK = 10;  // as icp_align_dev: the same number of iterations is enqueued as for the slowest pair alone
+  int launched = 0;
+  int* h_live = reinterpret_cast<int*>((char*)c->h_pinned + 12800);
+  auto enqueue_iteration = [&](IcpbArgs& a) {
+    icpb_nn_kernel<<<div_up(ns, NB_THREADS), NB_THREADS, 0, c->stream>>>(a);
+    icpb_brute_kernel<<<c->sm_count, BRT, 0, c->stream>>>(a);
+    icpb_reduce_kernel<<<rp[n], RD_THREADS, 0, c->stream>>>(a);
+    c->launches += 3;
+    a.par ^= 1;
+  };
+  for (;;) {
+    const int todo = (prm->max_iterations - launched) < CHUNK ? (prm->max_iterations - launched) : CHUNK;
+    for (int it = 0; it < todo; ++it) enqueue_iteration(A);
+    launched += todo;
+    LIOGPU_CUDA_OK(c, cudaGetLastError());
+    LIOGPU_CUDA_OK(c, cudaMemcpyAsync(h_live, &A.cnt->live, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+    LIOGPU_CUDA_OK(c, cudaStreamSynchronize(c->stream));
+    if (*h_live == 0 || launched >= prm->max_iterations) break;
+  }
+  A.fitness = 1;  // getFitnessScore
+  enqueue_iteration(A);
+  LIOGPU_CUDA_OK(c, cudaGetLastError());
+  std::vector<IcpDevState> hst(n);
+  LIOGPU_CUDA_OK(c, cudaMemcpyAsync(hst.data(), A.st, (size_t)n * sizeof(IcpDevState), cudaMemcpyDeviceToHost, c->stream));
+  LIOGPU_CUDA_OK(c, cudaStreamSynchronize(c->stream));
+  for (int p = 0; p < n; ++p) {
+    const IcpDevState& s = hst[p];
+    for (int q = 0; q < 16; ++q) final_T[p][q] = s.finalT[q];
+    info[p].iterations = s.iter;
+    info[p].convergence_state = s.state;
+    info[p].converged = (s.state >= 1 && s.state <= 4) ? 1 : 0;
+    info[p].n_correspondences = s.n_corr;
+    info[p].fitness_score = s.fitness;
+    info[p].last_mse = s.last_mse;
+    info[p].gpu_ms = 0.f;
+  }
   return LIOGPU_OK;
 }
 

@@ -288,19 +288,44 @@ void mapOptimization::loopFindNearKeyframes(Cloud& nearKeyframes, int key, int s
   nearKeyframes.resize(st < 0 ? 0 : n);
 }
 
-bool mapOptimization::loopClosureICP(int loopKeyCur, int loopKeyPre, float correctionLidarFrame[16], float* noiseScore) {
-  Cloud cureKeyframeCloud, prevKeyframeCloud;
-  loopFindNearKeyframes(cureKeyframeCloud, loopKeyCur, 0);                          // :1102
-  loopFindNearKeyframes(prevKeyframeCloud, loopKeyPre, historyKeyframeSearchNum);   // :1103
-  if (cureKeyframeCloud.size() < 300 || prevKeyframeCloud.size() < 1000) return false;  // :1104
+int mapOptimization::loopClosureICPBatch(const std::vector<std::pair<int, int>>& pairs,
+                                         std::vector<LoopClosureOutcome>& results) {
+  results.assign(pairs.size(), LoopClosureOutcome{});
+  std::vector<int> cur(pairs.size()), pre(pairs.size());
+  for (size_t j = 0; j < pairs.size(); ++j) { cur[j] = pairs[j].first; pre[j] = pairs[j].second; }
+  std::vector<float> poses;
+  for (const PointTypePose& p : cloudKeyPoses6D) {
+    const float pose6[6] = {p.roll, p.pitch, p.yaw, p.x, p.y, p.z};
+    poses.insert(poses.end(), pose6, pose6 + 6);
+  }
+  std::vector<liogpu_loop_icp_result> raw(pairs.size());
   liogpu_icp_params ip;
   liogpu_default_icp_params(&ip, historyKeyframeSearchRadius);                     // :1112-1116
-  lastStatus = liogpu_icp_align(ctx_, cureKeyframeCloud.data(), (int)cureKeyframeCloud.size(), sizeof(PointType),
-                                prevKeyframeCloud.data(), (int)prevKeyframeCloud.size(), sizeof(PointType), &ip,
-                                correctionLidarFrame, &lastIcpInfo);
-  if (lastStatus < 0) return false;
-  if (!lastIcpInfo.converged || lastIcpInfo.fitness_score > historyKeyframeFitnessScore) return false;  // :1123
-  if (noiseScore) *noiseScore = (float)lastIcpInfo.fitness_score;                   // :1145
+  // loopFindNearKeyframes(cur, 0) / (pre, historyKeyframeSearchNum) with downSizeFilterICP (:1102-1103), icp.align
+  lastStatus = liogpu_loop_closure_icp_batch(ctx_, cur.data(), pre.data(), (int)pairs.size(), poses.data(),
+                                             (int)cloudKeyPoses6D.size(), historyKeyframeSearchNum,
+                                             loopClosureICPSurfLeafSize, &ip, raw.data());
+  if (lastStatus < 0) return lastStatus;
+  for (size_t j = 0; j < pairs.size(); ++j) {
+    LoopClosureOutcome& o = results[j];
+    o.result = raw[j];
+    std::memcpy(o.correctionLidarFrame, raw[j].final_transformation, sizeof(o.correctionLidarFrame));
+    o.noiseScore = (float)raw[j].icp.fitness_score;                                 // :1145
+    o.accepted = !raw[j].rejected_by_size && raw[j].icp.converged &&                 // :1104
+                 raw[j].icp.fitness_score <= historyKeyframeFitnessScore;            // :1123
+  }
+  return lastStatus;
+}
+
+bool mapOptimization::loopClosureICP(int loopKeyCur, int loopKeyPre, float correctionLidarFrame[16], float* noiseScore) {
+  std::vector<LoopClosureOutcome> out;
+  if (loopClosureICPBatch({{loopKeyCur, loopKeyPre}}, out) < 0) return false;
+  const LoopClosureOutcome& o = out[0];
+  if (o.result.rejected_by_size) return false;                                      // :1104
+  lastIcpInfo = o.result.icp;
+  std::memcpy(correctionLidarFrame, o.correctionLidarFrame, sizeof(o.correctionLidarFrame));
+  if (!o.accepted) return false;                                                    // :1123
+  if (noiseScore) *noiseScore = o.noiseScore;                                       // :1145
   return true;
 }
 

@@ -12,6 +12,7 @@
 #include <cstdint>
 #include <map>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include "../../include/liogpu.h"
@@ -123,7 +124,17 @@ class mapOptimization {
   void loopFindNearKeyframes(Cloud& nearKeyframes, int key, int searchNum);  // :1360-1383 -> liogpu_merge_keyframes
   // the cloud / ICP part of performRSLoopClosure (:1098-1125): false when a guard rejects the closure;
   // correctionLidarFrame = icp.getFinalTransformation() (row-major 4x4), noiseScore = icp.getFitnessScore()
+  // One pair through liogpu_loop_closure_icp_batch: the submaps stay on the device.
   bool loopClosureICP(int loopKeyCur, int loopKeyPre, float correctionLidarFrame[16], float* noiseScore);
+  // loopClosureICP for many (loopKeyCur, loopKeyPre) pairs in one library call (an offline job verifying the loops of a
+  // whole sequence).  results[j] holds pair j's verdict; loopIndexContainer is left to the caller, as above.
+  struct LoopClosureOutcome {
+    bool accepted = false;                 // passed the guards of MO:1104 and MO:1123
+    float correctionLidarFrame[16] = {0};  // icp.getFinalTransformation() (identity when the size guard rejected it)
+    float noiseScore = 0.f;                // icp.getFitnessScore()
+    liogpu_loop_icp_result result{};       // submap sizes, overflow flags and the ICP's own report
+  };
+  int loopClosureICPBatch(const std::vector<std::pair<int, int>>& pairs, std::vector<LoopClosureOutcome>& results);
   // ---- loop-closure detection (the loop context of INTEGRATION.md); descriptors are stored in this node's context ----
   // scManager.makeAndSaveScancontextAndKeys(*thisSurfKeyFrame) (:2151-2166) on the keyframe's cloud as
   // saveKeyFrameResident leaves it (the downsampled sweep, SCInputType::SINGLE_SCAN_FEAT) -> liogpu_make_scancontext +

@@ -72,6 +72,12 @@ class IcpInfo(C.Structure):
                 ("gpu_ms", C.c_float), ("reserved", C.c_int * 5)]
 
 
+class LoopIcpResult(C.Structure):
+    _fields_ = [("n_source", C.c_int), ("n_target", C.c_int), ("source_overflow", C.c_int), ("target_overflow", C.c_int),
+                ("rejected_by_size", C.c_int), ("final_transformation", C.c_float * 16), ("icp", IcpInfo),
+                ("reserved", C.c_int * 4)]
+
+
 class TileInfo(C.Structure):
     _fields_ = [("n_points", C.c_int), ("n_rows", C.c_int), ("n_bins", C.c_int), ("bin_lo", C.c_int), ("bin_hi", C.c_int),
                 ("n_tile_points", C.c_int), ("leaf_overflow", C.c_int), ("gpu_ms", C.c_float), ("plan_ms", C.c_float),
@@ -102,7 +108,7 @@ EXPORTS = ["liogpu_abi_version", "liogpu_default_params", "liogpu_create", "liog
            "liogpu_stream", "liogpu_resident_size", "liogpu_default_local_map_params", "liogpu_publish_local_map", "liogpu_merge_keyframes", "liogpu_default_icp_params", "liogpu_icp_align", "liogpu_make_scancontext", "liogpu_extract_nearby",
            "liogpu_scan2map_trace", "liogpu_voxel_tile", "liogpu_upload_scan_async", "liogpu_fetch_result",
            "liogpu_default_sc_params", "liogpu_sc_add", "liogpu_sc_clear", "liogpu_sc_detect_loop", "liogpu_sc_detect_loops",
-           "liogpu_detect_loop_distance"]
+           "liogpu_detect_loop_distance", "liogpu_loop_closure_icp_batch"]
 
 RESIDENT = "resident"   # LIOGPU_DEVICE_RESIDENT: the cloud the context kept in HBM (include/liogpu.h)
 UPLOADED = "uploaded"   # LIOGPU_UPLOADED_SCAN: the sweep liogpu_upload_scan_async put on its way
@@ -170,6 +176,8 @@ def load_library() -> C.CDLL:
     lib.liogpu_default_icp_params.restype = None
     lib.liogpu_icp_align.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int,
                                      C.POINTER(IcpParams), C.c_void_p, C.POINTER(IcpInfo)]
+    lib.liogpu_loop_closure_icp_batch.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int,
+                                                  C.c_float, C.POINTER(IcpParams), C.c_void_p]
     lib.liogpu_default_local_map_params.argtypes = [C.POINTER(LocalMapParams)]
     lib.liogpu_default_local_map_params.restype = None
     lib.liogpu_publish_local_map.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p,
@@ -428,6 +436,32 @@ class LioGpu:
         self._check(self.lib.liogpu_icp_align(self.h, sp, sn, ss, tp, tn, ts, C.byref(prm), T.ctypes.data, C.byref(info)))
         d = {k: getattr(info, k) for k, _ in IcpInfo._fields_ if k != "reserved"}
         return T.reshape(4, 4), d
+
+    def loop_closure_icp_batch(self, key_cur, key_pre, key_pose6s, search_num: int = 25, icp_leaf: float = 0.3,
+                               history_keyframe_search_radius: float = 10.0, **over):
+        """loopFindNearKeyframes for both ends of every pair + the ICP of mapOptmization.cpp:1104-1123, many pairs in one
+        call (liogpu_loop_closure_icp_batch) -> (T (n, 4, 4) float32, list of per-pair dicts: the submap sizes and
+        overflow flags, rejected_by_size and the icp_align info keys)."""
+        prm = IcpParams()
+        self.lib.liogpu_default_icp_params(C.byref(prm), C.c_float(history_keyframe_search_radius))
+        for k, v in over.items():
+            setattr(prm, k, v)
+        kc = np.ascontiguousarray(key_cur, np.int32).reshape(-1)
+        kp = np.ascontiguousarray(key_pre, np.int32).reshape(-1)
+        assert kc.shape == kp.shape
+        poses = np.ascontiguousarray(key_pose6s, np.float32).reshape(-1, 6)
+        n = kc.shape[0]
+        res = (LoopIcpResult * max(n, 1))()
+        self._check(self.lib.liogpu_loop_closure_icp_batch(self.h, kc.ctypes.data, kp.ctypes.data, n, poses.ctypes.data,
+                                                           poses.shape[0], int(search_num), C.c_float(icp_leaf),
+                                                           C.byref(prm), res))
+        T = np.array([np.ctypeslib.as_array(r.final_transformation) for r in res[:n]], np.float32).reshape(n, 4, 4)
+        out = []
+        for r in res[:n]:
+            d = {k: getattr(r, k) for k in ("n_source", "n_target", "source_overflow", "target_overflow", "rejected_by_size")}
+            d.update({k: getattr(r.icp, k) for k, _ in IcpInfo._fields_ if k != "reserved"})
+            out.append(d)
+        return T, out
 
     def make_scancontext(self, cloud, lidar_height: float = 2.0, max_radius: float = 80.0):
         """SCManager::makeScancontext + keys (Scancontext.cpp:151-225) -> (desc (20,60), ringkey, sectorkey), f64."""
