@@ -252,6 +252,20 @@ int liogpu_publish_local_map(liogpu_ctx* ctx, const int* ids, const float* pose6
 int liogpu_merge_keyframes(liogpu_ctx* ctx, const int* ids, const float* pose6s /* k*6 */, int k, float leaf,
                            void* xyzi_out, int out_stride, int cap_out, int* n_out);
 
+/* liogpu_merge_keyframes for n_windows windows in one call (offline loop verification, submap export).  Window w is
+ * ids[win_off[w] .. win_off[w+1]) with the poses pose6s[6*j] of the same entries (win_off: n_windows + 1 entries,
+ * non-decreasing from 0; ids may repeat, inside a window and across windows).  Its cloud is bit-equal to
+ * liogpu_merge_keyframes of that window with the same leaf, whatever windows surround it, and is written to xyzi_out
+ * records [out_off[w], out_off[w+1]).  overflow (may be NULL) receives each window's VoxelGrid guard flag (q4; that
+ * window's cloud is its transformed concatenation).  Returns LIOGPU_W_LEAF_OVERFLOW if any window's guard fired, and
+ * LIOGPU_E_CAPACITY when cap_out < out_off[n_windows], with out_off filled: liogpu_fetch_result then copies the whole
+ * concatenation without recomputing it.  Malformed arguments and window inputs of more than INT32_MAX points in all
+ * (LIOGPU_E_INVALID) and unknown ids (LIOGPU_E_NO_KEYFRAME) are refused before any work is done.  The registration's
+ * local map and index and the resident cloud are left untouched. */
+int liogpu_merge_keyframes_batch(liogpu_ctx* ctx, const int* ids, const float* pose6s, const int* win_off,
+                                 int n_windows, float leaf, void* xyzi_out, int out_stride, int cap_out,
+                                 int* out_off /* n_windows + 1 */, int* overflow /* n_windows or NULL */);
+
 /* ---- loop-closure registration (SURVEY §8 row f3): pcl::IterativeClosestPoint<PointXYZI,PointXYZI> as configured
  * at MO:1111-1121 (performRSLoopClosure) / MO:1203-1213 (performSCLoopClosure). */
 typedef struct liogpu_icp_params {
@@ -444,7 +458,7 @@ int liogpu_scan2map_trace(liogpu_ctx* ctx, const void* scan_ds, int n, int strid
 int liogpu_upload_scan_async(liogpu_ctx* ctx, const void* xyzi, int n, int stride);
 
 /* Copy out the cloud produced by the call RIGHT BEFORE this one (liogpu_build_local_map, liogpu_merge_keyframes,
- * liogpu_publish_local_map, liogpu_voxel_tile) without recomputing it: a caller that does not know the size passes
+ * liogpu_merge_keyframes_batch, liogpu_publish_local_map, liogpu_voxel_tile) without recomputing it: a caller that does not know the size passes
  * cap_out = 0 to the producing call, reads the size from its LIOGPU_E_CAPACITY return, sizes its buffer and fetches.
  * Returns the status the producing call would have returned (LIOGPU_OK or LIOGPU_W_LEAF_OVERFLOW). */
 int liogpu_fetch_result(liogpu_ctx* ctx, void* xyzi_out, int out_stride, int cap_out, int* n_out);

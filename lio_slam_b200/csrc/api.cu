@@ -3,6 +3,7 @@
 // without a usable CUDA device every entry point fails with LIOGPU_E_CUDA.
 #include "common.cuh"
 
+#include <algorithm>
 #include <cmath>
 #include <cstdlib>
 #include <cstring>
@@ -106,17 +107,12 @@ void clobber(Ctx* c, DevBuf* buf) {
   if (c->resident == buf) { c->resident = nullptr; c->resident_n = 0; }
 }
 
+}  // namespace
+
 // The k named keyframes as device tables for the multi-keyframe transform kernels: validates the ids, stages
 // poses [k*6 f32] | offsets [k+1 i32] | source pointers [k u64] in pinned memory (second half of h_pinned) and
 // uploads them in one copy.  Concatenation order = argument order (the reference's "+=" loops).
-struct KfTables {
-  const float4* const* srcs;
-  const int* offs;
-  const float* poses;
-  float* T12;
-  size_t total;
-};
-int stage_keyframes(Ctx* c, const char* who, const int* ids, const float* pose6s, int k, KfTables& t) {
+int liogpu::stage_keyframes(Ctx* c, const char* who, const int* ids, const float* pose6s, int k, KfTables& t) {
   t.total = 0;
   for (int f = 0; f < k; ++f) {
     auto it = c->keyframes.find(ids[f]);
@@ -160,6 +156,20 @@ int stage_keyframes(Ctx* c, const char* who, const int* ids, const float* pose6s
   t.T12 = reinterpret_cast<float*>(dp + tab_bytes);
   return LIOGPU_OK;
 }
+
+int liogpu::reserve_keep(Ctx* c, DevBuf& b, size_t need, size_t used) {
+  if (need <= b.cap) return LIOGPU_OK;
+  const size_t want = need + need / 2 + 4096;
+  void* np_ = nullptr;
+  LIOGPU_CUDA_OK(c, cudaMallocAsync(&np_, want, c->stream));
+  if (used) LIOGPU_CUDA_OK(c, cudaMemcpyAsync(np_, b.p, used, cudaMemcpyDeviceToDevice, c->stream));
+  if (b.p) LIOGPU_CUDA_OK(c, cudaFreeAsync(b.p, c->stream));
+  b.p = np_;
+  b.cap = want;
+  return LIOGPU_OK;
+}
+
+namespace {
 
 int enter(liogpu_ctx* ctx) {
   if (!ctx) return LIOGPU_E_INVALID;
@@ -238,7 +248,7 @@ int liogpu_create(liogpu_ctx** out, const liogpu_params* params) {
                       &c.tile_hist, &c.tile_pts, &c.tile_out, &c.dbg_idx, &c.dbg_d2, &c.dbg_coeff, &c.dbg_flag, &c.dbg_tie,
                       &c.imu_tab, &c.dsk_flags, &c.dsk_scan, &c.lm_flag, &c.lm_pos, &c.lm_a, &c.lm_b, &c.lm_md, &c.lm_left,
                       &c.lm_out, &c.lm_stats, &c.sor_setup, &c.sor_sorted, &c.sor_cell_start, &c.kf_tab,
-                      &c.sc_q, &c.sc_part, &c.sc_cand, &c.sc_out, &c.lc_src, &c.lc_tgt, &c.lc_tab};
+                      &c.sc_q, &c.sc_part, &c.sc_cand, &c.sc_out, &c.lc_src, &c.lc_tgt, &c.lc_tab, &c.mw_tab, &c.mw_seg};
     for (DevBuf* b : bufs) { b->stream = c.stream; b->async = true; }
   }
   // scratch hint of allocateMemory (mapOptmization.cpp:333-335)
@@ -266,7 +276,7 @@ void liogpu_destroy(liogpu_ctx* ctx) {
                     &c.fail_buf, &c.prev_nn, &c.hopeless, &c.fz_rows, &c.fz_left, &c.fz_lb, &c.fz_probe, &c.tile_plan, &c.tile_hist, &c.tile_pts, &c.tile_out, &c.dbg_idx, &c.dbg_d2, &c.dbg_coeff, &c.dbg_flag, &c.dbg_tie, &c.imu_tab, &c.dsk_flags, &c.dsk_scan,
                     &c.lm_flag, &c.lm_pos, &c.lm_a, &c.lm_b, &c.lm_md, &c.lm_left, &c.lm_out, &c.lm_stats, &c.sor_setup,
                     &c.sor_sorted, &c.sor_cell_start, &c.sc_q, &c.sc_part, &c.sc_cand, &c.sc_out, &c.lc_src, &c.lc_tgt,
-                    &c.lc_tab};
+                    &c.lc_tab, &c.mw_tab, &c.mw_seg};
   for (DevBuf* b : bufs) b->release();
   sc_release(&c);
   for (auto& kv : c.keyframes) kv.second.first.release();
@@ -672,6 +682,49 @@ int liogpu_merge_keyframes(liogpu_ctx* ctx, const int* ids, const float* pose6s,
   return overflow ? LIOGPU_W_LEAF_OVERFLOW : LIOGPU_OK;
 }
 
+int liogpu_merge_keyframes_batch(liogpu_ctx* ctx, const int* ids, const float* pose6s, const int* win_off, int n_windows,
+                                 float leaf, void* xyzi_out, int out_stride, int cap_out, int* out_off, int* overflow) {
+  NvtxRange nvtx_range_(__func__);
+  int rc = enter(ctx);
+  if (rc) return rc;
+  Ctx* c = &ctx->c;
+  bool ok = n_windows >= 0 && win_off && out_off && win_off[0] == 0 && (!xyzi_out || stride_ok(out_stride));
+  for (int w = 0; ok && w < n_windows; ++w) ok = win_off[w + 1] >= win_off[w];
+  if (ok && win_off[n_windows] > 0 && (!ids || !pose6s)) ok = false;
+  if (!ok) { c->err = "liogpu_merge_keyframes_batch: bad arguments"; return LIOGPU_E_INVALID; }
+  const int k = win_off[n_windows];
+  long long total = 0;
+  for (int j = 0; j < k; ++j) {
+    auto it = c->keyframes.find(ids[j]);
+    if (it == c->keyframes.end()) { c->err = "liogpu_merge_keyframes_batch: unknown keyframe id"; return LIOGPU_E_NO_KEYFRAME; }
+    total += it->second.second;
+  }
+  if (total > 0x7fffffffLL) { c->err = "liogpu_merge_keyframes_batch: windows too large"; return LIOGPU_E_INVALID; }
+  std::vector<int> ovf(n_windows);
+  LIOGPU_CUDA_OK(c, cudaEventRecord(c->ev0, c->stream));
+  // lm_b: neither the registration's local map / index nor a resident sweep lives there
+  rc = merge_windows_dev(c, ids, pose6s, win_off, n_windows, leaf, c->lm_b, out_off, ovf.data());
+  if (rc) return rc;
+  LIOGPU_CUDA_OK(c, cudaEventRecord(c->ev1, c->stream));
+  bool any = false;
+  for (int w = 0; w < n_windows; ++w) {
+    any = any || ovf[w];
+    if (overflow) overflow[w] = ovf[w];
+  }
+  const int m = out_off[n_windows];
+  if (m > 0) {
+    c->last_result = c->lm_b.as<float4>(); c->last_result_n = m; c->last_result_status = any ? LIOGPU_W_LEAF_OVERFLOW : LIOGPU_OK;
+  }
+  if (xyzi_out && m > 0) {
+    if (m > cap_out) { c->err = "liogpu_merge_keyframes_batch: output capacity too small"; return LIOGPU_E_CAPACITY; }
+    rc = store_cloud(c, c->lm_b.as<float4>(), m, xyzi_out, out_stride);
+    if (rc) return rc;
+  }
+  LIOGPU_CUDA_OK(c, cudaStreamSynchronize(c->stream));
+  cudaEventElapsedTime(&c->last_ms, c->ev0, c->ev1);
+  return any ? LIOGPU_W_LEAF_OVERFLOW : LIOGPU_OK;
+}
+
 void liogpu_default_icp_params(liogpu_icp_params* p, float history_keyframe_search_radius) {
   if (!p) return;
   std::memset(p, 0, sizeof(*p));
@@ -706,52 +759,6 @@ int liogpu_icp_align(liogpu_ctx* ctx, const void* source_xyzi, int n_source, int
 
 }  // extern "C"
 
-namespace {
-
-// grows `b` to `need` bytes keeping its first `used` bytes (stream-ordered, like DevBuf::reserve)
-int reserve_keep(Ctx* c, DevBuf& b, size_t need, size_t used) {
-  if (need <= b.cap) return LIOGPU_OK;
-  const size_t want = need + need / 2 + 4096;
-  void* np_ = nullptr;
-  LIOGPU_CUDA_OK(c, cudaMallocAsync(&np_, want, c->stream));
-  if (used) LIOGPU_CUDA_OK(c, cudaMemcpyAsync(np_, b.p, used, cudaMemcpyDeviceToDevice, c->stream));
-  if (b.p) LIOGPU_CUDA_OK(c, cudaFreeAsync(b.p, c->stream));
-  b.p = np_;
-  b.cap = want;
-  return LIOGPU_OK;
-}
-
-// loopFindNearKeyframes (MO:1360-1383) for the window [key - search_num, key + search_num] ∩ [0, n_key): the
-// liogpu_merge_keyframes pipeline (transform + concatenate + VoxelGrid), the result appended to `arena` at record `used`
-int loop_submap(Ctx* c, int key, int search_num, const float* key_pose6s, int n_key, float leaf, DevBuf& arena, int used,
-                int* m, bool* overflow) {
-  *m = 0;
-  *overflow = false;
-  std::vector<int> ids;
-  std::vector<float> poses;
-  const long long lo = (long long)key - search_num, hi = (long long)key + search_num;
-  for (long long k = lo < 0 ? 0 : lo; k <= hi && k < n_key; ++k) {
-    ids.push_back((int)k);
-    poses.insert(poses.end(), key_pose6s + 6 * k, key_pose6s + 6 * k + 6);
-  }
-  KfTables t;
-  int rc = stage_keyframes(c, "liogpu_loop_closure_icp_batch", ids.data(), poses.data(), (int)ids.size(), t);
-  if (rc || t.total == 0) return rc;
-  const int total = (int)t.total;
-  LIOGPU_CUDA_OK(c, c->lm_a.reserve(t.total * sizeof(float4)));
-  LIOGPU_CUDA_OK(c, launch_transform_multi(c, t.srcs, t.offs, (int)ids.size(), t.poses, t.T12, (long long)total, c->lm_a.as<float4>()));
-  rc = voxel_downsample_dev(c, c->lm_a.as<float4>(), total, leaf, c->lm_out, m, overflow);
-  if (rc) return rc;
-  if (*m == 0) return LIOGPU_OK;
-  rc = reserve_keep(c, arena, ((size_t)used + *m) * sizeof(float4), (size_t)used * sizeof(float4));
-  if (rc) return rc;
-  LIOGPU_CUDA_OK(c, cudaMemcpyAsync(arena.as<float4>() + used, c->lm_out.p, (size_t)*m * sizeof(float4),
-                                    cudaMemcpyDeviceToDevice, c->stream));
-  return LIOGPU_OK;
-}
-
-}  // namespace
-
 extern "C" {
 
 int liogpu_loop_closure_icp_batch(liogpu_ctx* ctx, const int* key_cur, const int* key_pre, int n_pairs,
@@ -780,26 +787,55 @@ int liogpu_loop_closure_icp_batch(liogpu_ctx* ctx, const int* key_cur, const int
     std::memset(&results[j], 0, sizeof(results[j]));
     for (int q = 0; q < 16; ++q) results[j].final_transformation[q] = (q % 5 == 0) ? 1.f : 0.f;
   }
-  // Pairs go to the device in groups that keep the submaps (and with them the index and per-point buffers) under a
-  // fixed size; every pair's result is independent of the group it lands in.  LIOGPU_LOOP_ICP_GROUP caps the pairs of
-  // a group (tests use it to split small batches).
-  constexpr long long GROUP_POINTS = 1ll << 25;
+  // Submaps: loopFindNearKeyframes (MO:1360-1383) of both ends of every pair, window [key - n, key + n] ∩ [0, n_key)
+  // (MO:1102-1103), built by merge_windows_dev for a batch of pairs at a time (the batch's inputs stay under 2^25
+  // points, so the submaps are bounded too).  The pairs that pass the size guard (MO:1104) are copied into the
+  // contiguous lc_src / lc_tgt layout and go to the ICP in groups that keep the submaps (and with them the index and
+  // per-point buffers) under a fixed size; every pair's result is independent of the batch and group it lands in.
+  // LIOGPU_LOOP_ICP_GROUP caps the pairs of a group (tests use it to split small batches).
+  constexpr long long GROUP_POINTS = 1ll << 25, BATCH_POINTS = 1ll << 25;
   int group_pairs = 1024;
   if (const char* e = getenv("LIOGPU_LOOP_ICP_GROUP")) {
     const int v = atoi(e);
     if (v > 0 && v < group_pairs) group_pairs = v;
   }
   LIOGPU_CUDA_OK(c, cudaEventRecord(c->ev0, c->stream));
-  std::vector<int> members, so{0}, to{0};
-  std::vector<float> T;
+  auto kf_points = [&](int key, int s) {
+    long long n = 0;
+    for (long long k = std::max(0ll, (long long)key - s); k <= (long long)key + s && k < n_key; ++k)
+      n += c->keyframes.at((int)k).second;
+    return n;
+  };
+  std::vector<int> members, so{0}, to{0}, ids, win_off, out_off, ovf;
+  std::vector<const float4*> src_seg, tgt_seg;  // submaps of the group's members not yet copied to lc_src / lc_tgt
+  std::vector<float> T, poses;
   std::vector<liogpu_icp_info> info;
+  int copied = 0;  // members already in lc_src / lc_tgt
+  auto gather = [&]() -> int {
+    const int n = (int)members.size();
+    if (n == copied) return LIOGPU_OK;
+    for (auto* v : {&so, &to}) {
+      std::vector<int> off(v->begin() + copied, v->end());
+      for (int& o : off) o -= (*v)[copied];
+      DevBuf& dst = v == &so ? c->lc_src : c->lc_tgt;
+      int r = reserve_keep(c, dst, (size_t)v->back() * sizeof(float4), (size_t)(*v)[copied] * sizeof(float4));
+      if (!r) r = gather_segments(c, v == &so ? src_seg : tgt_seg, off, dst.as<float4>() + (*v)[copied]);
+      if (r) return r;
+    }
+    src_seg.clear();
+    tgt_seg.clear();
+    copied = n;
+    return LIOGPU_OK;
+  };
   auto flush = [&]() -> int {
     const int n = (int)members.size();
     if (n == 0) return LIOGPU_OK;
+    int r = gather();
+    if (r) return r;
     T.resize((size_t)n * 16);
     info.assign(n, liogpu_icp_info{});
-    int r = icp_batch_dev(c, c->lc_src.as<float4>(), so.data(), c->lc_tgt.as<float4>(), to.data(), n, params,
-                          reinterpret_cast<float(*)[16]>(T.data()), info.data());
+    r = icp_batch_dev(c, c->lc_src.as<float4>(), so.data(), c->lc_tgt.as<float4>(), to.data(), n, params,
+                      reinterpret_cast<float(*)[16]>(T.data()), info.data());
     if (r) return r;
     for (int g = 0; g < n; ++g) {
       liogpu_loop_icp_result& res = results[members[g]];
@@ -809,31 +845,60 @@ int liogpu_loop_closure_icp_batch(liogpu_ctx* ctx, const int* key_cur, const int
     members.clear();
     so.assign(1, 0);
     to.assign(1, 0);
+    copied = 0;
     return LIOGPU_OK;
   };
-  for (int j = 0; j < n_pairs; ++j) {
-    liogpu_loop_icp_result& res = results[j];
-    int ms = 0, mt = 0;
-    bool os = false, ot = false;
-    rc = loop_submap(c, key_cur[j], 0, key_pose6s, n_key, icp_leaf, c->lc_src, so.back(), &ms, &os);       // MO:1102
-    if (rc) return rc;
-    rc = loop_submap(c, key_pre[j], search_num, key_pose6s, n_key, icp_leaf, c->lc_tgt, to.back(), &mt, &ot);  // MO:1103
-    if (rc) return rc;
-    res.n_source = ms;
-    res.n_target = mt;
-    res.source_overflow = os ? 1 : 0;
-    res.target_overflow = ot ? 1 : 0;
-    if (ms < 300 || mt < 1000) {  // MO:1104; the submaps just appended are overwritten by the next pair
-      res.rejected_by_size = 1;
-      continue;
+  for (int j0 = 0; j0 < n_pairs;) {
+    // a batch of pairs, windows in the order (source, target) of each pair
+    ids.clear();
+    poses.clear();
+    win_off.assign(1, 0);
+    long long pts = 0;
+    int j1 = j0;
+    for (; j1 < n_pairs; ++j1) {
+      const long long add = kf_points(key_cur[j1], 0) + kf_points(key_pre[j1], search_num);
+      if (j1 > j0 && pts + add > BATCH_POINTS) break;
+      pts += add;
+      for (int e = 0; e < 2; ++e) {
+        const int key = e ? key_pre[j1] : key_cur[j1], s = e ? search_num : 0;
+        for (long long k = std::max(0ll, (long long)key - s); k <= (long long)key + s && k < n_key; ++k) {
+          ids.push_back((int)k);
+          poses.insert(poses.end(), key_pose6s + 6 * k, key_pose6s + 6 * k + 6);
+        }
+        win_off.push_back((int)ids.size());
+      }
     }
-    members.push_back(j);
-    so.push_back(so.back() + ms);
-    to.push_back(to.back() + mt);
-    if ((int)members.size() >= group_pairs || (long long)so.back() + to.back() >= GROUP_POINTS) {
-      rc = flush();
-      if (rc) return rc;
+    const int nw = 2 * (j1 - j0);
+    out_off.assign(nw + 1, 0);
+    ovf.assign(nw, 0);
+    rc = merge_windows_dev(c, ids.data(), poses.data(), win_off.data(), nw, icp_leaf, c->lm_b, out_off.data(), ovf.data());
+    if (rc) return rc;
+    const float4* arena = c->lm_b.as<float4>();
+    for (int j = j0; j < j1; ++j) {
+      liogpu_loop_icp_result& res = results[j];
+      const int ws = 2 * (j - j0), wt = ws + 1;
+      const int ms = out_off[ws + 1] - out_off[ws], mt = out_off[wt + 1] - out_off[wt];
+      res.n_source = ms;
+      res.n_target = mt;
+      res.source_overflow = ovf[ws];
+      res.target_overflow = ovf[wt];
+      if (ms < 300 || mt < 1000) {  // MO:1104
+        res.rejected_by_size = 1;
+        continue;
+      }
+      members.push_back(j);
+      src_seg.push_back(arena + out_off[ws]);
+      tgt_seg.push_back(arena + out_off[wt]);
+      so.push_back(so.back() + ms);
+      to.push_back(to.back() + mt);
+      if ((int)members.size() >= group_pairs || (long long)so.back() + to.back() >= GROUP_POINTS) {
+        rc = flush();
+        if (rc) return rc;
+      }
     }
+    rc = gather();  // the next batch reuses the arena
+    if (rc) return rc;
+    j0 = j1;
   }
   rc = flush();
   if (rc) return rc;

@@ -195,6 +195,9 @@ struct Ctx {
   // batched loop-closure ICP: the group's source / target submaps (packed float4, one segment per pair) and its
   // device tables (per-pair offsets, grids, ICP states, reduce partials)
   DevBuf lc_src, lc_tgt, lc_tab;
+  // segmented VoxelGrid over many keyframe windows (voxel.cu merge_windows_dev): per-window tables of a pass, and the
+  // segment table of the copy that places the windows' clouds
+  DevBuf mw_tab, mw_seg;
 };
 
 #define LIOGPU_CUDA_OK(ctx, expr)                                                        \
@@ -218,9 +221,31 @@ cudaError_t launch_transform_multi(Ctx* c, const float4* const* d_srcs, const in
 cudaError_t radix_sort_pairs(Ctx* c, int n, int key_bits, const int* d_key_bits, uint32_t** keys_out,
                              uint32_t** vals_out);
 cudaError_t exclusive_scan_u32(Ctx* c, const uint32_t* in, uint32_t* out, int n, uint32_t* d_total);
+// --- api.cu
+// The k named keyframes as device tables for launch_transform_multi (ids must have been validated by the caller or
+// are refused here with LIOGPU_E_NO_KEYFRAME).  The tables are staged in pinned memory that the next call reuses, so
+// the stream must have passed the upload before stage_keyframes runs again.
+struct KfTables {
+  const float4* const* srcs;
+  const int* offs;
+  const float* poses;
+  float* T12;
+  size_t total;
+};
+int stage_keyframes(Ctx* c, const char* who, const int* ids, const float* pose6s, int k, KfTables& t);
+// grows `b` to `need` bytes keeping its first `used` bytes (stream-ordered, like DevBuf::reserve)
+int reserve_keep(Ctx* c, DevBuf& b, size_t need, size_t used);
 // --- voxel.cu
 cudaError_t launch_minmax(Ctx* c, const float4* pts, int n, unsigned* mm);
 int voxel_downsample_dev(Ctx* c, const float4* in, int n, float leaf, DevBuf& out, int* n_out, bool* overflow);
+// liogpu_merge_keyframes of n_windows windows (window w = ids / pose6s entries [win_off[w], win_off[w+1]), host
+// arrays, ids validated, input total <= INT32_MAX): the clouds go to `out` one after another in window order, window w
+// at records [out_off[w], out_off[w+1]); overflow[w] = its VoxelGrid guard fired.  Each window's cloud is bit-equal
+// to the single-window call whatever windows surround it.  `out` must not be lm_a, lm_out or mw_seg.
+int merge_windows_dev(Ctx* c, const int* ids, const float* pose6s, const int* win_off, int n_windows, float leaf,
+                      DevBuf& out, int* out_off, int* overflow);
+// dst[off[s] .. off[s+1]) = srcs[s][0 .. off[s+1] - off[s]) for every segment s, in one launch (off[0] = 0)
+int gather_segments(Ctx* c, const std::vector<const float4*>& srcs, const std::vector<int>& off, float4* dst);
 // --- tile.cu
 int voxel_tile_dev(Ctx* c, const float4* pts, int n, float leaf, int tile, int n_tiles, DevBuf& out, int* n_out,
                    bool* overflow, liogpu_tile_info* info);

@@ -13,6 +13,7 @@
 //   vox_segstart_kernel scatter segment starts
 //   vox_centroid_kernel one thread per voxel, members gathered through the sorted permutation
 #include "common.cuh"
+#include <stdlib.h>
 
 namespace liogpu {
 
@@ -453,6 +454,346 @@ int voxel_downsample_dev(Ctx* c, const float4* in, int n, float leaf, DevBuf& ou
     return LIOGPU_OK;
   }
   *n_out = (int)h_setup->n_vox;
+  return LIOGPU_OK;
+}
+
+// ---- segmented VoxelGrid: many keyframe windows per pass (liogpu_merge_keyframes_batch, the loop-closure submaps).
+// A pass holds the transformed concatenation of consecutive windows.  Each window gets the single-cloud setup of its
+// own points (same bounds, same vox_setup_compute); window w's keys are base_w + its single-cloud key, base_w = the
+// cells of the pass's earlier windows, and every point that the single-cloud pipeline drops (non-finite, or in a
+// window whose guard fired) gets the pass's sentinel key above every base.  The stable sort keeps each window's
+// points in their concatenation order, so the head / scan / centroid kernels above, run unchanged on the pass, sum
+// every voxel's members in the order the single-cloud pipeline does (DESIGN.md §7a).
+
+// the window of point i: the last w in [lo, hi) with off[w] <= i (empty windows are skipped)
+__device__ __forceinline__ int mw_window_of(const int* __restrict__ off, int lo, int hi, int i) {
+  while (hi - lo > 1) {
+    const int mid = (lo + hi) >> 1;
+    if (__ldg(off + mid) <= i) lo = mid; else hi = mid;
+  }
+  return lo;
+}
+
+// per-window bounds in vox_minmax_kernel's encoding: mn[3w+a] / mx[3w+a] ordered uint, cnt[w] finite points.  A block
+// covers MW_TILE consecutive points: one reduction when they lie in one window, else per-point atomics.
+constexpr int MW_ITEMS = 4;
+constexpr int MW_TILE = 256 * MW_ITEMS;
+__global__ void __launch_bounds__(256)
+mw_minmax_kernel(const float4* __restrict__ pts, int n, const int* __restrict__ off, int nw, unsigned* __restrict__ mn_o,
+                 unsigned* __restrict__ mx_o, unsigned* __restrict__ cnt_o) {
+  const int b0 = blockIdx.x * MW_TILE;
+  const int b1 = min(b0 + MW_TILE, n);
+  const int w0 = mw_window_of(off, 0, nw, b0), w1 = mw_window_of(off, 0, nw, b1 - 1);
+  if (w0 != w1) {
+    for (int i = b0 + threadIdx.x; i < b1; i += 256) {
+      const float4 p = pts[i];
+      if (!finite3(p)) continue;
+      const int w = mw_window_of(off, w0, w1 + 1, i);
+      atomicMin(&mn_o[3 * w], f2ord(p.x)); atomicMin(&mn_o[3 * w + 1], f2ord(p.y)); atomicMin(&mn_o[3 * w + 2], f2ord(p.z));
+      atomicMax(&mx_o[3 * w], f2ord(p.x)); atomicMax(&mx_o[3 * w + 1], f2ord(p.y)); atomicMax(&mx_o[3 * w + 2], f2ord(p.z));
+      atomicAdd(&cnt_o[w], 1u);
+    }
+    return;
+  }
+  float mn[3] = {FLT_MAX, FLT_MAX, FLT_MAX}, mx[3] = {-FLT_MAX, -FLT_MAX, -FLT_MAX};
+  unsigned cnt = 0;
+#pragma unroll
+  for (int k = 0; k < MW_ITEMS; ++k) {
+    const int i = b0 + k * 256 + threadIdx.x;
+    if (i < b1) {
+      const float4 p = pts[i];
+      if (finite3(p)) {
+        mn[0] = fminf(mn[0], p.x); mn[1] = fminf(mn[1], p.y); mn[2] = fminf(mn[2], p.z);
+        mx[0] = fmaxf(mx[0], p.x); mx[1] = fmaxf(mx[1], p.y); mx[2] = fmaxf(mx[2], p.z);
+        ++cnt;
+      }
+    }
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+#pragma unroll
+    for (int a = 0; a < 3; ++a) {
+      mn[a] = fminf(mn[a], __shfl_xor_sync(0xffffffffu, mn[a], o));
+      mx[a] = fmaxf(mx[a], __shfl_xor_sync(0xffffffffu, mx[a], o));
+    }
+    cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
+  }
+  __shared__ float smn[8][3], smx[8][3];
+  __shared__ unsigned scnt[8];
+  const int lane = threadIdx.x & 31, wp = threadIdx.x >> 5;
+  if (lane == 0) {
+#pragma unroll
+    for (int a = 0; a < 3; ++a) { smn[wp][a] = mn[a]; smx[wp][a] = mx[a]; }
+    scnt[wp] = cnt;
+  }
+  __syncthreads();
+  if (threadIdx.x < 3) {
+    const int a = threadIdx.x;
+    float lo = smn[0][a], hi = smx[0][a];
+    for (int k = 1; k < 8; ++k) { lo = fminf(lo, smn[k][a]); hi = fmaxf(hi, smx[k][a]); }
+    unsigned c = 0;
+    for (int k = 0; k < 8; ++k) c += scnt[k];
+    if (c) {  // a block of non-finite points leaves the window's bounds at their initial values
+      atomicMin(&mn_o[3 * w0 + a], f2ord(lo));
+      atomicMax(&mx_o[3 * w0 + a], f2ord(hi));
+    }
+  } else if (threadIdx.x == 3) {
+    unsigned c = 0;
+    for (int k = 0; k < 8; ++k) c += scnt[k];
+    atomicAdd(&cnt_o[w0], c);
+  }
+}
+
+// one thread per window: vox_setup_kernel on the window's bounds
+__global__ void mw_setup_kernel(const unsigned* __restrict__ mn_o, const unsigned* __restrict__ mx_o,
+                                const unsigned* __restrict__ cnt_o, int nw, float leaf, VoxelSetup* __restrict__ s) {
+  const int w = blockIdx.x * blockDim.x + threadIdx.x;
+  if (w >= nw) return;
+  VoxelSetup v;
+  float mn[3], mx[3];
+  for (int a = 0; a < 3; ++a) { mn[a] = ord2f(mn_o[3 * w + a]); mx[a] = ord2f(mx_o[3 * w + a]); }
+  vox_setup_compute(mn, mx, (int)cnt_o[w], leaf, v);
+  s[w] = v;
+}
+
+// keys of the pass's points [p0, p0 + n) (windows [wa, wb)); keys[i - p0]
+__global__ void __launch_bounds__(256)
+mw_key_kernel(const float4* __restrict__ pts, int p0, int n, const int* __restrict__ off, int wa, int wb,
+              const VoxelSetup* __restrict__ setups, const unsigned* __restrict__ base, unsigned sentinel,
+              uint32_t* __restrict__ keys) {
+  const int t = blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= n) return;
+  const int i = p0 + t;
+  const int w = mw_window_of(off, wa, wb, i);
+  const float4 p = pts[i];
+  const VoxelSetup& s = setups[w];
+  keys[t] = (s.overflow || !finite3(p)) ? sentinel : __ldg(base + w) + vox_key_of(p, s);
+}
+
+// voxels of each window of the pass: the scanned head flags at its first and past its last sorted position
+__global__ void mw_count_kernel(const uint32_t* __restrict__ rank, int n, const uint32_t* __restrict__ n_vox,
+                                const int2* __restrict__ vrange, int wa, int wb, uint32_t* __restrict__ vcount) {
+  const int w = wa + blockIdx.x * blockDim.x + threadIdx.x;
+  if (w >= wb) return;
+  const int2 r = vrange[w];
+  const uint32_t s = r.x < n ? rank[r.x] : *n_vox, e = r.y < n ? rank[r.y] : *n_vox;
+  vcount[w] = e - s;
+}
+
+__global__ void __launch_bounds__(256)
+mw_gather_kernel(const float4* const* __restrict__ srcs, const int* __restrict__ off, int nseg, int total,
+                 float4* __restrict__ dst) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= total) return;
+  const int s = mw_window_of(off, 0, nseg, i);
+  dst[i] = srcs[s][i - __ldg(off + s)];
+}
+
+int gather_segments(Ctx* c, const std::vector<const float4*>& srcs, const std::vector<int>& off, float4* dst) {
+  const int nseg = (int)srcs.size();
+  if (nseg == 0 || off[nseg] == 0) return LIOGPU_OK;
+  const size_t b_srcs = (size_t)nseg * sizeof(void*), b_off = ((size_t)nseg + 1) * sizeof(int);
+  LIOGPU_CUDA_OK(c, c->mw_seg.reserve(b_srcs + b_off));
+  char* d = (char*)c->mw_seg.p;
+  // pageable sources: cudaMemcpyAsync has copied them out when it returns
+  LIOGPU_CUDA_OK(c, cudaMemcpyAsync(d, srcs.data(), b_srcs, cudaMemcpyHostToDevice, c->stream));
+  LIOGPU_CUDA_OK(c, cudaMemcpyAsync(d + b_srcs, off.data(), b_off, cudaMemcpyHostToDevice, c->stream));
+  mw_gather_kernel<<<div_up(off[nseg], 256), 256, 0, c->stream>>>(reinterpret_cast<const float4* const*>(d),
+                                                                 reinterpret_cast<const int*>(d + b_srcs), nseg, off[nseg], dst);
+  c->launches++;
+  LIOGPU_CUDA_OK(c, cudaGetLastError());
+  return LIOGPU_OK;
+}
+
+// Input points of a pass (all its windows' transformed points).  A window larger than this runs alone.  The pass
+// scratch is about 56 bytes a point: the transformed points and the centroids (16 + 16), the sort's keys and values
+// (4 x 4) and the head flags and segment starts (2 x 4).  LIOGPU_MERGE_PASS_POINTS lowers it (tests use it to split
+// small batches).
+static long long merge_pass_points() {
+  long long cap = 1ll << 25;
+  if (const char* e = getenv("LIOGPU_MERGE_PASS_POINTS")) {
+    const long long v = atoll(e);
+    if (v > 0 && v < cap) cap = v;
+  }
+  return cap;
+}
+
+// One pass: windows [0, nw) of ids / poses (entries [win_off[0], win_off[nw]) of the caller's arrays, n_in[w] points
+// each), appended to `out` at record `out_base`; out_off / overflow are the pass's own nw + 1 / nw entries.
+static int merge_pass(Ctx* c, const int* ids, const float* pose6s, const int* win_off, const long long* n_in, int nw,
+                      float leaf, DevBuf& out, int* out_off, int* overflow) {
+  const int out_base = out_off[0];
+  for (int w = 0; w < nw; ++w) overflow[w] = 0;
+  const int k = win_off[nw] - win_off[0];
+  KfTables t;
+  int rc = stage_keyframes(c, "liogpu_merge_keyframes_batch", ids + win_off[0], pose6s + 6 * (size_t)win_off[0], k, t);
+  if (rc) return rc;
+  const int total = (int)t.total;
+  if (!(leaf > 0.f)) {  // no VoxelGrid: the transformed concatenation, which is already in window order
+    for (int w = 0; w < nw; ++w) out_off[w + 1] = out_off[w] + (int)n_in[w];
+    if (total == 0) return LIOGPU_OK;
+    rc = reserve_keep(c, out, ((size_t)out_base + total) * sizeof(float4), (size_t)out_base * sizeof(float4));
+    if (rc) return rc;
+    LIOGPU_CUDA_OK(c, launch_transform_multi(c, t.srcs, t.offs, k, t.poses, t.T12, (long long)total,
+                                             out.as<float4>() + out_base));
+    LIOGPU_CUDA_OK(c, cudaStreamSynchronize(c->stream));  // the next pass restages the keyframe tables
+    return LIOGPU_OK;
+  }
+  if (total == 0) {
+    for (int w = 0; w < nw; ++w) out_off[w + 1] = out_off[w];
+    return LIOGPU_OK;
+  }
+  std::vector<int> off(nw + 1, 0);
+  for (int w = 0; w < nw; ++w) off[w + 1] = off[w] + (int)n_in[w];
+  // device tables: off | mn | mx | cnt | vcount | setups | base | vrange | pass setups (<= nw)
+  auto up256 = [](size_t b) { return (b + 255) & ~(size_t)255; };
+  const size_t o_mn = up256(((size_t)nw + 1) * 4), o_mx = o_mn + up256((size_t)nw * 12), o_cnt = o_mx + up256((size_t)nw * 12);
+  const size_t o_vc = o_cnt + up256((size_t)nw * 4), o_set = o_vc + up256((size_t)nw * 4);
+  const size_t o_base = o_set + up256((size_t)nw * sizeof(VoxelSetup)), o_vr = o_base + up256((size_t)nw * 4);
+  const size_t o_ps = o_vr + up256((size_t)nw * 8), tab_bytes = o_ps + (size_t)nw * sizeof(VoxelSetup);
+  LIOGPU_CUDA_OK(c, c->mw_tab.reserve(tab_bytes));
+  char* d = (char*)c->mw_tab.p;
+  const int* d_off = reinterpret_cast<const int*>(d);
+  unsigned *d_mn = reinterpret_cast<unsigned*>(d + o_mn), *d_mx = reinterpret_cast<unsigned*>(d + o_mx);
+  unsigned *d_cnt = reinterpret_cast<unsigned*>(d + o_cnt), *d_vc = reinterpret_cast<unsigned*>(d + o_vc);
+  VoxelSetup* d_set = reinterpret_cast<VoxelSetup*>(d + o_set);
+  VoxelSetup* d_ps = reinterpret_cast<VoxelSetup*>(d + o_ps);
+  const unsigned* d_base = reinterpret_cast<const unsigned*>(d + o_base);
+  const int2* d_vr = reinterpret_cast<const int2*>(d + o_vr);
+  LIOGPU_CUDA_OK(c, c->lm_a.reserve((size_t)total * sizeof(float4)));
+  LIOGPU_CUDA_OK(c, c->lm_out.reserve((size_t)total * sizeof(float4)));
+  LIOGPU_CUDA_OK(c, c->keys0.reserve((size_t)total * 4));
+  LIOGPU_CUDA_OK(c, c->keys1.reserve((size_t)total * 4));
+  LIOGPU_CUDA_OK(c, c->vals0.reserve((size_t)total * 4));
+  LIOGPU_CUDA_OK(c, c->vals1.reserve((size_t)total * 4));
+  LIOGPU_CUDA_OK(c, c->seg_flag.reserve((size_t)total * 4 + 16));
+  LIOGPU_CUDA_OK(c, c->seg_start.reserve((size_t)total * 4 + 16));
+  LIOGPU_CUDA_OK(c, c->misc.reserve(256));
+  float4* pts = c->lm_a.as<float4>();
+  float4* cent = c->lm_out.as<float4>();
+  LIOGPU_CUDA_OK(c, launch_transform_multi(c, t.srcs, t.offs, k, t.poses, t.T12, (long long)total, pts));
+  // bounds and setups of every window, read back once
+  LIOGPU_CUDA_OK(c, cudaMemcpyAsync(d, off.data(), ((size_t)nw + 1) * 4, cudaMemcpyHostToDevice, c->stream));
+  LIOGPU_CUDA_OK(c, cudaMemsetAsync(d_mn, 0xff, (size_t)nw * 12, c->stream));
+  LIOGPU_CUDA_OK(c, cudaMemsetAsync(d_mx, 0, o_set - o_mx, c->stream));  // mx, cnt and vcount
+  mw_minmax_kernel<<<div_up(total, MW_TILE), 256, 0, c->stream>>>(pts, total, d_off, nw, d_mn, d_mx, d_cnt);
+  mw_setup_kernel<<<div_up(nw, 128), 128, 0, c->stream>>>(d_mn, d_mx, d_cnt, nw, leaf, d_set);
+  c->launches += 2;
+  LIOGPU_CUDA_OK(c, cudaGetLastError());
+  std::vector<VoxelSetup> set(nw);
+  LIOGPU_CUDA_OK(c, cudaMemcpyAsync(set.data(), d_set, (size_t)nw * sizeof(VoxelSetup), cudaMemcpyDeviceToHost, c->stream));
+  LIOGPU_CUDA_OK(c, cudaStreamSynchronize(c->stream));
+  // key space: windows share it while their cells fit 32 bits next to the sentinel; a window that needs all of it
+  // keys alone, with exactly the single-cloud keys and sentinel
+  std::vector<unsigned> base(nw);
+  std::vector<int2> vr(nw);
+  std::vector<VoxelSetup> ps;
+  std::vector<int> seg_w{0};  // key segments: windows [seg_w[s], seg_w[s+1])
+  unsigned long long cells_sum = 0;
+  int valid = 0;
+  bool alone = false;
+  auto close = [&]() {
+    VoxelSetup v{};
+    v.n_valid = valid;
+    v.n_cells = (unsigned)cells_sum;
+    int b = 0;
+    while (b < 32 && (v.n_cells >> b) != 0u) ++b;
+    v.key_bits = b;
+    ps.push_back(v);
+  };
+  for (int w = 0; w < nw; ++w) {
+    const VoxelSetup& s = set[w];
+    const bool used = !s.overflow && s.n_valid > 0;
+    const unsigned long long cells =
+        used ? (unsigned long long)s.div_b[0] * (unsigned long long)s.div_b[1] * (unsigned long long)s.div_b[2] : 0ull;
+    const bool big = cells > 0xffffffffull;
+    if (w > seg_w.back() && (alone || big || cells_sum + cells > 0xffffffffull)) {
+      close();
+      seg_w.push_back(w);
+      cells_sum = 0;
+      valid = 0;
+    }
+    alone = big;
+    base[w] = (unsigned)cells_sum;
+    const int nv = used ? s.n_valid : 0;
+    vr[w] = make_int2(valid, valid + nv);
+    cells_sum += cells;
+    valid += nv;
+    overflow[w] = s.overflow ? 1 : 0;
+  }
+  close();
+  seg_w.push_back(nw);
+  const int n_seg = (int)ps.size();
+  LIOGPU_CUDA_OK(c, cudaMemcpyAsync(d + o_base, base.data(), (size_t)nw * 4, cudaMemcpyHostToDevice, c->stream));
+  LIOGPU_CUDA_OK(c, cudaMemcpyAsync(d + o_vr, vr.data(), (size_t)nw * 8, cudaMemcpyHostToDevice, c->stream));
+  LIOGPU_CUDA_OK(c, cudaMemcpyAsync(d_ps, ps.data(), (size_t)n_seg * sizeof(VoxelSetup), cudaMemcpyHostToDevice, c->stream));
+  uint32_t* d_nvox = c->misc.as<uint32_t>();
+  uint32_t* d_long = c->misc.as<uint32_t>() + 2;  // [0] long count, [1] work counter
+  for (int sg = 0; sg < n_seg; ++sg) {
+    if (ps[sg].n_valid == 0) continue;  // nothing but dropped points: every window of it keeps vcount 0
+    const int wa = seg_w[sg], wb = seg_w[sg + 1];
+    const int p0 = off[wa], n = off[wb] - off[wa];
+    mw_key_kernel<<<div_up(n, 256), 256, 0, c->stream>>>(pts, p0, n, d_off, wa, wb, d_set, d_base, ps[sg].n_cells,
+                                                         c->keys0.as<uint32_t>());
+    c->launches++;
+    uint32_t *skeys = nullptr, *sperm = nullptr;
+    LIOGPU_CUDA_OK(c, radix_sort_pairs(c, n, ps[sg].key_bits, nullptr, &skeys, &sperm));
+    uint32_t* head = c->seg_flag.as<uint32_t>();
+    vox_head_kernel<<<div_up(n, 256), 256, 0, c->stream>>>(skeys, n, d_ps + sg, head);
+    c->launches++;
+    LIOGPU_CUDA_OK(c, exclusive_scan_u32(c, head, head, n, d_nvox));
+    vox_segstart_kernel<<<div_up(n, 256), 256, 0, c->stream>>>(skeys, head, n, d_ps + sg, c->seg_start.as<uint32_t>(), d_nvox);
+    uint32_t* long_list = (skeys == c->keys0.as<uint32_t>()) ? c->keys1.as<uint32_t>() : c->keys0.as<uint32_t>();
+    LIOGPU_CUDA_OK(c, cudaMemsetAsync(d_long, 0, 2 * sizeof(uint32_t), c->stream));
+    vox_centroid_kernel<<<div_up(n, 256), 256, 0, c->stream>>>(pts + p0, sperm, c->seg_start.as<uint32_t>(), d_nvox,
+                                                               cent + p0, long_list, d_long);
+    vox_centroid_long_kernel<<<c->sm_count * 8, 32 * VOX_LONG_WARPS, 0, c->stream>>>(
+        pts + p0, sperm, c->seg_start.as<uint32_t>(), long_list, d_long, d_long + 1, cent + p0);
+    mw_count_kernel<<<div_up(wb - wa, 128), 128, 0, c->stream>>>(head, n, d_nvox, d_vr, wa, wb, d_vc);
+    c->launches += 4;
+    LIOGPU_CUDA_OK(c, cudaGetLastError());
+  }
+  std::vector<unsigned> vc(nw);
+  LIOGPU_CUDA_OK(c, cudaMemcpyAsync(vc.data(), d_vc, (size_t)nw * 4, cudaMemcpyDeviceToHost, c->stream));
+  LIOGPU_CUDA_OK(c, cudaStreamSynchronize(c->stream));
+  // placement: window w's centroids start at its key segment's first point plus the voxels of the segment's earlier
+  // windows; a window whose guard fired is its transformed input (q4)
+  std::vector<const float4*> srcs(nw);
+  std::vector<int> dst(nw + 1, 0);
+  for (int sg = 0; sg < n_seg; ++sg) {
+    long long v = 0;
+    for (int w = seg_w[sg]; w < seg_w[sg + 1]; ++w) {
+      const int m = overflow[w] ? (int)n_in[w] : (int)vc[w];
+      srcs[w] = overflow[w] ? pts + off[w] : cent + off[seg_w[sg]] + v;
+      if (!overflow[w]) v += vc[w];
+      dst[w + 1] = dst[w] + m;
+      out_off[w + 1] = out_off[w] + m;
+    }
+  }
+  if (dst[nw] == 0) return LIOGPU_OK;
+  rc = reserve_keep(c, out, ((size_t)out_base + dst[nw]) * sizeof(float4), (size_t)out_base * sizeof(float4));
+  if (rc) return rc;
+  return gather_segments(c, srcs, dst, out.as<float4>() + out_base);
+}
+
+int merge_windows_dev(Ctx* c, const int* ids, const float* pose6s, const int* win_off, int n_windows, float leaf,
+                      DevBuf& out, int* out_off, int* overflow) {
+  out_off[0] = 0;
+  std::vector<long long> n_in(n_windows);
+  for (int w = 0; w < n_windows; ++w) {
+    long long n = 0;
+    for (int j = win_off[w]; j < win_off[w + 1]; ++j) n += c->keyframes.at(ids[j]).second;
+    n_in[w] = n;
+  }
+  const long long cap = merge_pass_points();
+  for (int w0 = 0; w0 < n_windows;) {
+    long long pts = n_in[w0];
+    int w1 = w0 + 1;
+    while (w1 < n_windows && pts + n_in[w1] <= cap) pts += n_in[w1++];
+    const int rc = merge_pass(c, ids, pose6s, win_off + w0, n_in.data() + w0, w1 - w0, leaf, out, out_off + w0, overflow + w0);
+    if (rc) return rc;
+    w0 = w1;
+  }
   return LIOGPU_OK;
 }
 

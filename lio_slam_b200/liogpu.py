@@ -108,7 +108,7 @@ EXPORTS = ["liogpu_abi_version", "liogpu_default_params", "liogpu_create", "liog
            "liogpu_stream", "liogpu_resident_size", "liogpu_default_local_map_params", "liogpu_publish_local_map", "liogpu_merge_keyframes", "liogpu_default_icp_params", "liogpu_icp_align", "liogpu_make_scancontext", "liogpu_extract_nearby",
            "liogpu_scan2map_trace", "liogpu_voxel_tile", "liogpu_upload_scan_async", "liogpu_fetch_result",
            "liogpu_default_sc_params", "liogpu_sc_add", "liogpu_sc_clear", "liogpu_sc_detect_loop", "liogpu_sc_detect_loops",
-           "liogpu_detect_loop_distance", "liogpu_loop_closure_icp_batch"]
+           "liogpu_detect_loop_distance", "liogpu_loop_closure_icp_batch", "liogpu_merge_keyframes_batch"]
 
 RESIDENT = "resident"   # LIOGPU_DEVICE_RESIDENT: the cloud the context kept in HBM (include/liogpu.h)
 UPLOADED = "uploaded"   # LIOGPU_UPLOADED_SCAN: the sweep liogpu_upload_scan_async put on its way
@@ -154,6 +154,8 @@ def load_library() -> C.CDLL:
     lib.liogpu_set_local_map.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int]
     lib.liogpu_merge_keyframes.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_float, C.c_void_p, C.c_int,
                                            C.c_int, C.POINTER(C.c_int)]
+    lib.liogpu_merge_keyframes_batch.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_float,
+                                                 C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p]
     lib.liogpu_upload_scan_async.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int]
     lib.liogpu_fetch_result.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_int)]
     lib.liogpu_voxel_tile.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_float, C.c_int, C.c_int, C.c_void_p,
@@ -422,6 +424,30 @@ class LioGpu:
             st = self.lib.liogpu_fetch_result(self.h, out.ctypes.data, 16, out.shape[0], C.byref(n_out))
         self._check(st)
         return out[: n_out.value].copy(), st
+
+    def merge_keyframes_batch(self, windows, leaf: float = 0.0):
+        """merge_keyframes of many windows in one call (liogpu_merge_keyframes_batch); windows = [(ids, poses), ...]
+        -> (list of clouds (n_w, 4), overflow flags (n_windows,) bool, status)."""
+        ids = [np.ascontiguousarray(i, np.int32).reshape(-1) for i, _ in windows]
+        poses = [np.ascontiguousarray(p, np.float32).reshape(-1, 6) for _, p in windows]
+        assert all(p.shape[0] == i.shape[0] for i, p in zip(ids, poses))
+        n = len(windows)
+        win_off = np.zeros(n + 1, np.int32)
+        win_off[1:] = np.cumsum([i.shape[0] for i in ids])
+        flat_ids = np.concatenate(ids + [np.zeros(1, np.int32)])
+        flat_poses = np.concatenate(poses + [np.zeros((1, 6), np.float32)])
+        out_off = np.zeros(n + 1, np.int32)
+        ovf = np.zeros(max(n, 1), np.int32)
+        n_out = C.c_int(0)
+        out = np.empty((1, 4), np.float32)
+        st = self.lib.liogpu_merge_keyframes_batch(self.h, flat_ids.ctypes.data, flat_poses.ctypes.data,
+                                                   win_off.ctypes.data, n, C.c_float(leaf), out.ctypes.data, 16,
+                                                   out.shape[0], out_off.ctypes.data, ovf.ctypes.data)
+        if st == E_CAPACITY:  # the clouds exist on the device: copy them out without recomputing
+            out = np.empty((int(out_off[n]), 4), np.float32)
+            st = self.lib.liogpu_fetch_result(self.h, out.ctypes.data, 16, out.shape[0], C.byref(n_out))
+        self._check(st)
+        return [out[out_off[w]:out_off[w + 1]].copy() for w in range(n)], ovf[:n].astype(bool), st
 
     def icp_align(self, source, target, history_keyframe_search_radius: float = 10.0, **over):
         """pcl::IterativeClosestPoint as configured at mapOptmization.cpp:1111-1123 -> (T (4,4), info dict)."""
