@@ -371,6 +371,19 @@ void liogpu_default_sc_params(liogpu_sc_params* p);
  * The keys are derived on the device with the same code as liogpu_make_scancontext, so they are bit-equal to the ones it
  * returns. */
 int liogpu_sc_add(liogpu_ctx* ctx, const double* descs, int n);
+/* makeAndSaveScancontextAndKeys (Scancontext.cpp:228-243) for n resident keyframes, in the given order: the
+ * descriptor of each keyframe's lidar-frame cloud (as liogpu_keyframe_put stored it) is appended to the store and
+ * its keys derived, exactly as liogpu_make_scancontext on that cloud followed by liogpu_sc_add would.  ids may
+ * repeat.  descs_out (n x 1200 f64, host or device, may be NULL) receives the descriptors.
+ * Entry j and descs_out[j] are bit-equal to liogpu_make_scancontext of keyframe ids[j] with the same lidar_height and
+ * max_radius, whatever the batch around it; a keyframe of 0 points gives an all-zero descriptor.  The call appends after
+ * whatever is stored (it interleaves freely with liogpu_sc_add) and does not advance liogpu_sc_detect_loop's tree
+ * counter.  The clouds are read in place and the descriptors never leave the device unless descs_out asks for them:
+ * three launches and one sync whatever n, per 2^31 - 1 points of the keyframes (two launches and one sync per further
+ * such pass).  Refused before any work, with the store unchanged: LIOGPU_E_INVALID for n <= 0, ids == NULL,
+ * !(max_radius > 0) or a store count past INT32_MAX; LIOGPU_E_NO_KEYFRAME for an id that was never put. */
+int liogpu_sc_add_keyframes(liogpu_ctx* ctx, const int* ids, int n, double lidar_height, double max_radius,
+                            double* descs_out);
 /* drop every stored descriptor and reset the tree counter (a fresh SCManager); liogpu_keyframe_clear does not touch the
  * store */
 int liogpu_sc_clear(liogpu_ctx* ctx);

@@ -111,7 +111,8 @@ void clobber(Ctx* c, DevBuf* buf) {
 
 // The k named keyframes as device tables for the multi-keyframe transform kernels: validates the ids, stages
 // poses [k*6 f32] | offsets [k+1 i32] | source pointers [k u64] in pinned memory (second half of h_pinned) and
-// uploads them in one copy.  Concatenation order = argument order (the reference's "+=" loops).
+// uploads them in one copy.  Concatenation order = argument order (the reference's "+=" loops).  pose6s may be NULL
+// for a caller that reads the clouds in the lidar frame (the pose table is then left unset).
 int liogpu::stage_keyframes(Ctx* c, const char* who, const int* ids, const float* pose6s, int k, KfTables& t) {
   t.total = 0;
   for (int f = 0; f < k; ++f) {
@@ -138,7 +139,7 @@ int liogpu::stage_keyframes(Ctx* c, const char* who, const int* ids, const float
   float* hposes = reinterpret_cast<float*>(hp);
   int* hoffs = reinterpret_cast<int*>(hp + off_offs);
   const float4** hsrcs = reinterpret_cast<const float4**>(hp + off_srcs);
-  std::memcpy(hposes, pose6s, (size_t)k * 6 * sizeof(float));
+  if (pose6s) std::memcpy(hposes, pose6s, (size_t)k * 6 * sizeof(float));
   size_t off = 0;
   for (int f = 0; f < k; ++f) {
     auto& kf = c->keyframes[ids[f]];
@@ -974,6 +975,25 @@ int liogpu_sc_add(liogpu_ctx* ctx, const double* descs, int n) {
   Ctx* c = &ctx->c;
   if (!descs || n <= 0 || (long long)c->sc.count + n > 0x7fffffffLL) { c->err = "liogpu_sc_add: bad arguments"; return LIOGPU_E_INVALID; }
   return sc_add_dev(c, descs, n);
+}
+
+int liogpu_sc_add_keyframes(liogpu_ctx* ctx, const int* ids, int n, double lidar_height, double max_radius,
+                            double* descs_out) {
+  NvtxRange nvtx_range_(__func__);
+  int rc = enter(ctx);
+  if (rc) return rc;
+  Ctx* c = &ctx->c;
+  if (!ids || n <= 0 || !(max_radius > 0.0) || (long long)c->sc.count + n > 0x7fffffffLL) {
+    c->err = "liogpu_sc_add_keyframes: bad arguments";
+    return LIOGPU_E_INVALID;
+  }
+  std::vector<int> n_pts((size_t)n);
+  for (int f = 0; f < n; ++f) {
+    auto it = c->keyframes.find(ids[f]);
+    if (it == c->keyframes.end()) { c->err = "liogpu_sc_add_keyframes: unknown keyframe id"; return LIOGPU_E_NO_KEYFRAME; }
+    n_pts[f] = it->second.second;
+  }
+  return sc_add_keyframes_dev(c, ids, n_pts, lidar_height, max_radius, descs_out);
 }
 
 int liogpu_sc_clear(liogpu_ctx* ctx) {

@@ -264,6 +264,10 @@ int extract_nearby_dev(Ctx* c, const float4* key3d, int n, const double* h_times
 int scancontext_dev(Ctx* c, const float4* pts, int n, double lidar_height, double max_radius, double* h_out);
 // --- loopdetect.cu
 int sc_add_dev(Ctx* c, const double* descs, int n);
+// liogpu_sc_add_keyframes after its argument checks (ids validated, count + n_pts.size() <= INT32_MAX): appends the
+// descriptors of the keyframes ids[f], n_pts[f] points each
+int sc_add_keyframes_dev(Ctx* c, const int* ids, const std::vector<int>& n_pts, double lidar_height, double max_radius,
+                         double* descs_out);
 void sc_release(Ctx* c);
 int sc_detect_dev(Ctx* c, const std::vector<int2>& qm, int k, int R, double thres, ScQueryOut* h_out, liogpu_sc_info* info);
 int detect_loop_distance_dev(Ctx* c, const float4* key3d, int n, const double* h_times, double time_cur, float radius,

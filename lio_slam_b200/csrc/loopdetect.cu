@@ -9,7 +9,9 @@
 //
 //   sc_store_kernel      block per added descriptor: ring key (-> f32, eig2stdvec), sector key (scancontext.cuh, the
 //                        code of liogpu_make_scancontext) and the 60 column norms (shift-invariant: circshift moves
-//                        whole columns) in the oracle's Eigen order
+//                        whole columns) in the oracle's Eigen order.  For liogpu_sc_add_keyframes it first turns the
+//                        u32 image that the binning left in the first half of the slot into the f64 descriptor
+//                        (scancontext.cu's header)
 //   sc_knn_chunk_kernel  block per (query, 1024 prefix keys): nanoflann L2_Adaptor<float> distances as 64-bit
 //                        (d2 bits << 32 | index) keys, bitonic sort in shared memory, the k+1 smallest out
 //   sc_knn_merge_kernel  block per query: merges its chunks' lists -> k candidates in (d2, index) order, ties counted
@@ -75,12 +77,19 @@ __device__ __forceinline__ void bitonic_sort(u64* s, int n) {
   __syncthreads();
 }
 
+template <bool FROM_IMAGE>
 __global__ void __launch_bounds__(256)
-sc_store_kernel(const double* __restrict__ desc, float* __restrict__ rkey, double* __restrict__ vkey,
-                double* __restrict__ cnorm) {
+sc_store_kernel(double* __restrict__ desc, float* __restrict__ rkey, double* __restrict__ vkey, double* __restrict__ cnorm) {
   __shared__ double d[SC_BINS];
   const size_t e = blockIdx.x;
-  for (int k = threadIdx.x; k < SC_BINS; k += blockDim.x) d[k] = desc[e * SC_BINS + k];
+  if (FROM_IMAGE) {
+    const unsigned* img = reinterpret_cast<const unsigned*>(desc + e * SC_BINS);
+    for (int k = threadIdx.x; k < SC_BINS; k += blockDim.x) d[k] = sc_bin_value(img[k]);
+    __syncthreads();  // the doubles overwrite the image
+    for (int k = threadIdx.x; k < SC_BINS; k += blockDim.x) desc[e * SC_BINS + k] = d[k];
+  } else {
+    for (int k = threadIdx.x; k < SC_BINS; k += blockDim.x) d[k] = desc[e * SC_BINS + k];
+  }
   __syncthreads();
   const int k = threadIdx.x;
   if (k < SC_RING) {
@@ -303,34 +312,108 @@ cudaError_t sc_grow_array(Ctx* c, void** p, size_t old_bytes, size_t new_bytes) 
   return e;
 }
 
+// Room for `need` entries: geometric growth, contents carried over on the stream (stream-ordered: no device-wide sync).
+int sc_reserve(Ctx* c, int need) {
+  ScStore& st = c->sc;
+  if (need <= st.cap) return LIOGPU_OK;
+  int cap = st.cap > 0 ? st.cap : 1024;
+  while (cap < need) cap = cap > (1 << 29) ? need : cap * 2;
+  const size_t o = (size_t)st.count, nw = (size_t)cap;
+  LIOGPU_CUDA_OK(c, sc_grow_array(c, (void**)&st.desc, o * SC_BINS * 8, nw * SC_BINS * 8));
+  LIOGPU_CUDA_OK(c, sc_grow_array(c, (void**)&st.rkey, o * SC_RING * 4, nw * SC_RING * 4));
+  LIOGPU_CUDA_OK(c, sc_grow_array(c, (void**)&st.vkey, o * SC_SECTOR * 8, nw * SC_SECTOR * 8));
+  LIOGPU_CUDA_OK(c, sc_grow_array(c, (void**)&st.cnorm, o * SC_SECTOR * 8, nw * SC_SECTOR * 8));
+  st.cap = cap;
+  return LIOGPU_OK;
+}
+
 }  // namespace
 
 // Appends n descriptors (host or device memory, row-major [ring][sector] f64) to the store and derives their keys.
 int sc_add_dev(Ctx* c, const double* descs, int n) {
   ScStore& st = c->sc;
   const int need = st.count + n;
-  if (need > st.cap) {  // geometric growth, contents carried over on the stream (stream-ordered: no device-wide sync)
-    int cap = st.cap > 0 ? st.cap : 1024;
-    while (cap < need) cap = cap > (1 << 29) ? need : cap * 2;
-    const size_t o = (size_t)st.count, nw = (size_t)cap;
-    LIOGPU_CUDA_OK(c, sc_grow_array(c, (void**)&st.desc, o * SC_BINS * 8, nw * SC_BINS * 8));
-    LIOGPU_CUDA_OK(c, sc_grow_array(c, (void**)&st.rkey, o * SC_RING * 4, nw * SC_RING * 4));
-    LIOGPU_CUDA_OK(c, sc_grow_array(c, (void**)&st.vkey, o * SC_SECTOR * 8, nw * SC_SECTOR * 8));
-    LIOGPU_CUDA_OK(c, sc_grow_array(c, (void**)&st.cnorm, o * SC_SECTOR * 8, nw * SC_SECTOR * 8));
-    st.cap = cap;
-  }
+  int rc = sc_reserve(c, need);
+  if (rc) return rc;
   const size_t e0 = (size_t)st.count;
   LIOGPU_CUDA_OK(c, cudaMemcpyAsync(st.desc + e0 * SC_BINS, descs, (size_t)n * SC_BINS * sizeof(double), cudaMemcpyDefault,
                                     c->stream));
   LIOGPU_CUDA_OK(c, cudaEventRecord(c->ev0, c->stream));
-  sc_store_kernel<<<n, 256, 0, c->stream>>>(st.desc + e0 * SC_BINS, st.rkey + e0 * SC_RING, st.vkey + e0 * SC_SECTOR,
-                                            st.cnorm + e0 * SC_SECTOR);
+  sc_store_kernel<false><<<n, 256, 0, c->stream>>>(st.desc + e0 * SC_BINS, st.rkey + e0 * SC_RING, st.vkey + e0 * SC_SECTOR,
+                                                   st.cnorm + e0 * SC_SECTOR);
   c->launches++;
   LIOGPU_CUDA_OK(c, cudaGetLastError());
   LIOGPU_CUDA_OK(c, cudaEventRecord(c->ev1, c->stream));
   LIOGPU_CUDA_OK(c, cudaStreamSynchronize(c->stream));
   cudaEventElapsedTime(&c->last_ms, c->ev0, c->ev1);
   st.count = need;
+  return LIOGPU_OK;
+}
+
+// Points of a pass: the stage_keyframes tables address a pass's clouds with 32-bit offsets.  LIOGPU_SC_PASS_POINTS
+// lowers the cap (tests use it to split small batches).
+static long long sc_pass_points() {
+  long long cap = 0x7fffffffLL;
+  if (const char* e = getenv("LIOGPU_SC_PASS_POINTS")) {
+    const long long v = atoll(e);
+    if (v > 0 && v < cap) cap = v;
+  }
+  return cap;
+}
+
+// The new entries' slots hold the binning's u32 images until sc_store_kernel<true> replaces them with the doubles, so
+// the batch needs no table memory of its own.  A pass takes consecutive keyframes up to sc_pass_points() points (a
+// larger keyframe runs alone) and costs two launches (slot init, binning) and, before the next pass restages the
+// tables, one sync; one store launch for all entries follows.  Up to 2^31 - 1 points in all: one pass.
+int sc_add_keyframes_dev(Ctx* c, const int* ids, const std::vector<int>& n_pts, double lidar_height, double max_radius,
+                         double* descs_out) {
+  ScStore& st = c->sc;
+  const int k = (int)n_pts.size();
+  const long long cap = sc_pass_points();
+  // pass p = keyframes [pass[p], pass[p + 1]); its block-offset table (relative to its first block, one entry past
+  // its last keyframe) at tab[pass[p] + p ...]
+  std::vector<int> pass{0}, tab;
+  tab.reserve((size_t)k + 8);
+  long long acc = 0, nb = 0;
+  for (int f = 0; f < k; ++f) {
+    if (f > pass.back() && acc + n_pts[f] > cap) {
+      tab.push_back((int)nb);
+      pass.push_back(f);
+      acc = nb = 0;
+    }
+    acc += n_pts[f];
+    tab.push_back((int)nb);
+    nb += (n_pts[f] + (long long)SC_CHUNK - 1) / SC_CHUNK;  // < cap / SC_CHUNK + k per pass
+  }
+  tab.push_back((int)nb);
+  pass.push_back(k);
+  const int need = st.count + k;
+  int rc = sc_reserve(c, need);
+  if (rc) return rc;
+  LIOGPU_CUDA_OK(c, c->sc_q.reserve(tab.size() * sizeof(int)));
+  LIOGPU_CUDA_OK(c, cudaMemcpyAsync(c->sc_q.p, tab.data(), tab.size() * sizeof(int), cudaMemcpyHostToDevice, c->stream));
+  const size_t e0 = (size_t)st.count;
+  double* slots = st.desc + e0 * SC_BINS;
+  LIOGPU_CUDA_OK(c, cudaEventRecord(c->ev0, c->stream));
+  for (int p = 0; p + 1 < (int)pass.size(); ++p) {
+    const int f0 = pass[p], kp = pass[p + 1] - f0;
+    if (p > 0) LIOGPU_CUDA_OK(c, cudaStreamSynchronize(c->stream));  // the previous pass's tables were uploaded
+    KfTables t{};
+    rc = stage_keyframes(c, "liogpu_sc_add_keyframes", ids + f0, nullptr, kp, t);
+    if (rc) return rc;
+    LIOGPU_CUDA_OK(c, launch_sc_bin_keyframes(c, t.srcs, t.offs, c->sc_q.as<int>() + f0 + p, kp, tab[f0 + p + kp],
+                                              lidar_height, max_radius, slots + (size_t)f0 * SC_BINS));
+  }
+  sc_store_kernel<true><<<k, 256, 0, c->stream>>>(slots, st.rkey + e0 * SC_RING, st.vkey + e0 * SC_SECTOR,
+                                                  st.cnorm + e0 * SC_SECTOR);
+  c->launches++;
+  LIOGPU_CUDA_OK(c, cudaGetLastError());
+  LIOGPU_CUDA_OK(c, cudaEventRecord(c->ev1, c->stream));
+  st.count = need;
+  if (descs_out)
+    LIOGPU_CUDA_OK(c, cudaMemcpyAsync(descs_out, slots, (size_t)k * SC_BINS * sizeof(double), cudaMemcpyDefault, c->stream));
+  LIOGPU_CUDA_OK(c, cudaStreamSynchronize(c->stream));
+  cudaEventElapsedTime(&c->last_ms, c->ev0, c->ev1);
   return LIOGPU_OK;
 }
 

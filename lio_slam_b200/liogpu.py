@@ -108,7 +108,8 @@ EXPORTS = ["liogpu_abi_version", "liogpu_default_params", "liogpu_create", "liog
            "liogpu_stream", "liogpu_resident_size", "liogpu_default_local_map_params", "liogpu_publish_local_map", "liogpu_merge_keyframes", "liogpu_default_icp_params", "liogpu_icp_align", "liogpu_make_scancontext", "liogpu_extract_nearby",
            "liogpu_scan2map_trace", "liogpu_voxel_tile", "liogpu_upload_scan_async", "liogpu_fetch_result",
            "liogpu_default_sc_params", "liogpu_sc_add", "liogpu_sc_clear", "liogpu_sc_detect_loop", "liogpu_sc_detect_loops",
-           "liogpu_detect_loop_distance", "liogpu_loop_closure_icp_batch", "liogpu_merge_keyframes_batch"]
+           "liogpu_detect_loop_distance", "liogpu_loop_closure_icp_batch", "liogpu_merge_keyframes_batch",
+           "liogpu_sc_add_keyframes"]
 
 RESIDENT = "resident"   # LIOGPU_DEVICE_RESIDENT: the cloud the context kept in HBM (include/liogpu.h)
 UPLOADED = "uploaded"   # LIOGPU_UPLOADED_SCAN: the sweep liogpu_upload_scan_async put on its way
@@ -167,6 +168,7 @@ def load_library() -> C.CDLL:
     lib.liogpu_default_sc_params.argtypes = [C.POINTER(ScParams)]
     lib.liogpu_default_sc_params.restype = None
     lib.liogpu_sc_add.argtypes = [C.c_void_p, C.c_void_p, C.c_int]
+    lib.liogpu_sc_add_keyframes.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_double, C.c_double, C.c_void_p]
     lib.liogpu_sc_clear.argtypes = [C.c_void_p]
     lib.liogpu_sc_detect_loop.argtypes = [C.c_void_p, C.POINTER(ScParams), C.POINTER(C.c_int), C.POINTER(C.c_float),
                                           C.POINTER(ScInfo)]
@@ -515,6 +517,16 @@ class LioGpu:
         """makeAndSaveScancontextAndKeys for descriptors as make_scancontext returns them: (20, 60) or (n, 20, 60) f64."""
         d = np.ascontiguousarray(descs, np.float64).reshape(-1, 1200)
         self._check(self.lib.liogpu_sc_add(self.h, d.ctypes.data, d.shape[0]))
+
+    def sc_add_keyframes(self, ids, lidar_height: float = 2.0, max_radius: float = 80.0, return_descs: bool = False):
+        """make_scancontext + sc_add of resident keyframes in one call (liogpu_sc_add_keyframes): the descriptors of
+        the keyframes' clouds are appended to the store in the order of `ids` -> (n, 20, 60) f64 when return_descs,
+        else None."""
+        i = np.ascontiguousarray(ids, np.int32).reshape(-1)
+        out = np.empty((i.shape[0], 20, 60), np.float64) if return_descs else None
+        self._check(self.lib.liogpu_sc_add_keyframes(self.h, i.ctypes.data, i.shape[0], lidar_height, max_radius,
+                                                     None if out is None else out.ctypes.data))
+        return out
 
     def sc_clear(self) -> None:
         self._check(self.lib.liogpu_sc_clear(self.h))
