@@ -69,6 +69,58 @@ struct GridParams {
   float gate1_d2;     // squared radius of the cheap first search phase (>= gate_d2 disables it)
 };
 
+// Order-preserving integer image of a float: atomicMin / atomicMax on images are the min / max of the floats.
+__device__ __forceinline__ unsigned f2ord(float f) {
+  const unsigned u = __float_as_uint(f);
+  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+__device__ __forceinline__ float ord2f(unsigned o) {
+  const unsigned u = (o & 0x80000000u) ? (o & 0x7fffffffu) : ~o;
+  return __uint_as_float(u);
+}
+
+// cell of coordinate p along one axis of a grid (origin o, n cells), clamped into the grid
+__device__ __forceinline__ int cell_coord(float p, float o, float inv_h, int n) {
+  int c = (int)((p - o) * inv_h);
+  c = c < 0 ? 0 : c;
+  return c >= n ? n - 1 : c;
+}
+
+// The grid over a bounding box [mn, mx] of n_points finite points: origin at the minimum, cell edge `cell` doubled
+// until at most max_cells cells cover the box.  A cloud with no finite point gets the one-cell grid at the origin.
+__device__ __forceinline__ GridParams grid_setup_compute(const float mn[3], const float mx[3], int n_points, float cell,
+                                                         unsigned max_cells, float gate_d2, float gate1_d2) {
+  GridParams g;
+  g.n_points = n_points;
+  float lo[3] = {mn[0], mn[1], mn[2]}, hi[3] = {mx[0], mx[1], mx[2]};
+  if (n_points <= 0) { lo[0] = lo[1] = lo[2] = 0.f; hi[0] = hi[1] = hi[2] = 0.f; }
+  float maxabs = 1.0f;
+  for (int a = 0; a < 3; ++a) {
+    maxabs = fmaxf(maxabs, fmaxf(fabsf(lo[a]), fabsf(hi[a])));
+    maxabs = fmaxf(maxabs, hi[a] - lo[a]);
+  }
+  g.ox = lo[0]; g.oy = lo[1]; g.oz = lo[2];
+  float h = cell;
+  for (;;) {
+    const float inv = 1.0f / h;
+    const double nx = floor((double)(hi[0] - lo[0]) * inv) + 1, ny = floor((double)(hi[1] - lo[1]) * inv) + 1,
+                 nz = floor((double)(hi[2] - lo[2]) * inv) + 1;
+    if (nx * ny * nz <= (double)max_cells) {
+      g.nx = (int)nx; g.ny = (int)ny; g.nz = (int)nz;
+      g.h = h; g.inv_h = inv;
+      break;
+    }
+    h *= 2.0f;
+  }
+  g.n_cells = (unsigned)g.nx * (unsigned)g.ny * (unsigned)g.nz;
+  // positional slack: covers f32 rounding of (p - origin) * inv_h and of the cell bounds (4+ ulps of
+  // the largest coordinate), so a pruned cell can never hold a point that ties or beats the worst.
+  g.slack = maxabs * 9.5367431640625e-07f;  // 2^-20
+  g.gate_d2 = gate_d2;
+  g.gate1_d2 = gate1_d2;
+  return g;
+}
+
 #define LIOGPU_FZ_K 8  // members of a point's candidate set (s2m_fused.cuh)
 
 // ---- state of the LM loop kept on device between iterations (MO:171,176,177) ----

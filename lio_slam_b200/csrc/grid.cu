@@ -13,52 +13,13 @@
 
 namespace liogpu {
 
-__device__ __forceinline__ float ord2f_g(unsigned o) {
-  const unsigned u = (o & 0x80000000u) ? (o & 0x7fffffffu) : ~o;
-  return __uint_as_float(u);
-}
-
 // mm = output of vox_minmax_kernel (ordered-uint min[3], max[3], finite count)
 __global__ void grid_setup_kernel(const unsigned* __restrict__ mm, float cell, float gate_d2, float gate1_d2,
                                   unsigned max_cells, GridParams* __restrict__ gp) {
   if (threadIdx.x != 0 || blockIdx.x != 0) return;
-  GridParams g;
-  g.n_points = (int)mm[6];
   float mn[3], mx[3];
-  float maxabs = 1.0f;
-  for (int a = 0; a < 3; ++a) {
-    mn[a] = ord2f_g(mm[a]);
-    mx[a] = ord2f_g(mm[3 + a]);
-    maxabs = fmaxf(maxabs, fmaxf(fabsf(mn[a]), fabsf(mx[a])));
-    maxabs = fmaxf(maxabs, mx[a] - mn[a]);
-  }
-  if (g.n_points <= 0) { mn[0] = mn[1] = mn[2] = 0.f; mx[0] = mx[1] = mx[2] = 0.f; }
-  g.ox = mn[0]; g.oy = mn[1]; g.oz = mn[2];
-  float h = cell;
-  for (;;) {
-    const float inv = 1.0f / h;
-    const double nx = floor((double)(mx[0] - mn[0]) * inv) + 1, ny = floor((double)(mx[1] - mn[1]) * inv) + 1,
-                 nz = floor((double)(mx[2] - mn[2]) * inv) + 1;
-    if (nx * ny * nz <= (double)max_cells) {
-      g.nx = (int)nx; g.ny = (int)ny; g.nz = (int)nz;
-      g.h = h; g.inv_h = inv;
-      break;
-    }
-    h *= 2.0f;
-  }
-  g.n_cells = (unsigned)g.nx * (unsigned)g.ny * (unsigned)g.nz;
-  // positional slack: covers f32 rounding of (p - origin) * inv_h and of the cell bounds (4+ ulps of
-  // the largest coordinate), so a pruned cell can never hold a point that ties or beats the worst.
-  g.slack = maxabs * 9.5367431640625e-07f;  // 2^-20
-  g.gate_d2 = gate_d2;
-  g.gate1_d2 = gate1_d2;
-  *gp = g;
-}
-
-__device__ __forceinline__ int cell_coord(float p, float o, float inv_h, int n) {
-  int c = (int)((p - o) * inv_h);
-  c = c < 0 ? 0 : c;
-  return c >= n ? n - 1 : c;
+  for (int a = 0; a < 3; ++a) { mn[a] = ord2f(mm[a]); mx[a] = ord2f(mm[3 + a]); }
+  *gp = grid_setup_compute(mn, mx, (int)mm[6], cell, max_cells, gate_d2, gate1_d2);
 }
 
 __global__ void __launch_bounds__(256)

@@ -13,6 +13,11 @@
 // The search stops growing once every uninspected cell is farther than the correspondence distance (such a point
 // has no correspondence).  getFitnessScore: the same search with no distance limit on the source moved by the final
 // transformation, f64 mean of the squared distances.
+//
+// liogpu_loop_closure_icp_batch runs many pairs with three launches per iteration (icpb_*).  Both launch structures
+// are built from the same device functions: nn_thread_walk (shells 0..2 by one thread), nn_warp_walk (the next shells
+// by one warp), nn_brute_block (one pass over the target) and icp_reduce_block (a pair's sums and fold), so a pair's
+// result is bit-equal whichever call computed it.
 #include "common.cuh"
 
 #include <stdlib.h>
@@ -84,6 +89,55 @@ constexpr int NN_THREADS = 128;
 constexpr int NN_THREAD_SHELLS = 3;  // shells 0..2 per thread
 constexpr int NN_WARP_SHELLS = 6;    // shells 0..5 per warp
 
+__device__ __forceinline__ unsigned long long warp_min_u64(unsigned long long v) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    const unsigned long long u = __shfl_xor_sync(0xffffffffu, v, o);
+    v = u < v ? u : v;
+  }
+  return v;
+}
+
+// One thread searches shells 0..NN_THREAD_SHELLS-1 around the home cell of p (finite) and returns the verdict of the
+// last shell it inspected; `best` is the nearest point found in them.  max_d2 is a reference so that icp_nn_kernel
+// reads it from shared memory at each verdict rather than holding it in two more registers.
+__device__ __forceinline__ int nn_thread_walk(const float4* sorted, const uint32_t* cs, const GridParams& g,
+                                              const float4 p, const double& max_d2, Best1& best) {
+  const HomeCell hc = home_cell(g, p);
+  best.init();
+  int verdict = 0;
+  for (int R = 0; R < NN_THREAD_SHELLS && verdict == 0; ++R) {
+    const int z0 = max(hc.cz - R, 0), z1 = min(hc.cz + R, g.nz - 1);
+    const int y0 = max(hc.cy - R, 0), y1 = min(hc.cy + R, g.ny - 1);
+    for (int z = z0; z <= z1; ++z)
+      for (int y = y0; y <= y1; ++y) scan_shell_row(sorted, cs, g, hc, R, y, z, p, best);
+    verdict = nn_verdict(best, covered_d2(g, hc, R), max_d2);
+  }
+  return verdict;
+}
+
+// The whole warp searches shells R0..NN_WARP_SHELLS-1 around the home cell of p (finite, the same on every lane), each
+// lane's rows starting from `best` (what shells 0..R0-1 found, or empty).  Returns the verdict of the last shell
+// inspected; `all` is the warp's nearest point.
+__device__ __forceinline__ int nn_warp_walk(const float4* sorted, const uint32_t* cs, const GridParams& g,
+                                            const float4 p, double max_d2, int R0, Best1 best, Best1& all) {
+  const HomeCell hc = home_cell(g, p);
+  const int lane = threadIdx.x & 31;
+  all.init();
+  int verdict = 0;
+  for (int R = R0; R < NN_WARP_SHELLS && verdict == 0; ++R) {
+    const int side = 2 * R + 1, rows = side * side;
+    for (int r = lane; r < rows; r += 32) {
+      const int z = hc.cz + r / side - R, y = hc.cy + r % side - R;
+      if (z < 0 || z >= g.nz || y < 0 || y >= g.ny) continue;
+      scan_shell_row(sorted, cs, g, hc, R, y, z, p, best);
+    }
+    all.key = warp_min_u64(best.key);
+    verdict = nn_verdict(all, covered_d2(g, hc, R), max_d2);
+  }
+  return verdict;
+}
+
 __global__ void __launch_bounds__(NN_THREADS)
 icp_nn_kernel(const IcpArgs A) {
   __shared__ GridParams g;
@@ -107,32 +161,14 @@ icp_nn_kernel(const IcpArgs A) {
     A.cur[i] = p;
   }
   if (!(isfinite(p.x) && isfinite(p.y) && isfinite(p.z))) { A.nn_idx[i] = -1; A.nn_d2[i] = CUDART_INF_F; return; }
-  const HomeCell hc = home_cell(g, p);
   Best1 best;
-  best.init();
-  int verdict = 0;
-  for (int R = 0; R < NN_THREAD_SHELLS && verdict == 0; ++R) {
-    const int z0 = max(hc.cz - R, 0), z1 = min(hc.cz + R, g.nz - 1);
-    const int y0 = max(hc.cy - R, 0), y1 = min(hc.cy + R, g.ny - 1);
-    for (int z = z0; z <= z1; ++z)
-      for (int y = y0; y <= y1; ++y) scan_shell_row(A.sorted, A.cs, g, hc, R, y, z, p, best);
-    verdict = nn_verdict(best, covered_d2(g, hc, R), s_max_d2);
-  }
+  const int verdict = nn_thread_walk(A.sorted, A.cs, g, p, s_max_d2, best);
   if (verdict == 0) {
     A.left_list[atomicAdd(&A.st->n_left, 1u)] = (uint32_t)i;
   } else {
     A.nn_idx[i] = verdict == 1 ? best.idx() : -1;
     A.nn_d2[i] = best.d2();
   }
-}
-
-__device__ __forceinline__ unsigned long long warp_min_u64(unsigned long long v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) {
-    const unsigned long long u = __shfl_xor_sync(0xffffffffu, v, o);
-    v = u < v ? u : v;
-  }
-  return v;
 }
 
 __global__ void __launch_bounds__(256)
@@ -159,22 +195,9 @@ icp_left_kernel(const IcpArgs A) {
       if (lane == 0) { A.nn_idx[i] = -1; A.nn_d2[i] = CUDART_INF_F; }
       continue;
     }
-    const HomeCell hc = home_cell(g, p);
-    Best1 best;
-    best.init();
-    int verdict = 0;
-    Best1 all;
-    all.init();
-    for (int R = 0; R < NN_WARP_SHELLS && verdict == 0; ++R) {
-      const int side = 2 * R + 1, rows = side * side;
-      for (int r = lane; r < rows; r += 32) {
-        const int z = hc.cz + r / side - R, y = hc.cy + r % side - R;
-        if (z < 0 || z >= g.nz || y < 0 || y >= g.ny) continue;
-        scan_shell_row(A.sorted, A.cs, g, hc, R, y, z, p, best);
-      }
-      all.key = warp_min_u64(best.key);
-      verdict = nn_verdict(all, covered_d2(g, hc, R), max_d2);
-    }
+    Best1 seed, all;
+    seed.init();
+    const int verdict = nn_warp_walk(A.sorted, A.cs, g, p, max_d2, 0, seed, all);
     if (lane == 0) {
       if (verdict == 0) {
         A.left_list[A.ns + atomicAdd(&A.st->n_brute, 1u)] = i;
@@ -186,45 +209,51 @@ icp_left_kernel(const IcpArgs A) {
   }
 }
 
+// The whole block finds the nearest of the n_points sorted targets to point i at p in one pass (eight loads in flight
+// per thread), then the block minimum, and writes nn_idx[i] / nn_d2[i]
 constexpr int BRT = 512;
+__device__ __forceinline__ void nn_brute_block(const float4* sorted, int n_points, const float4 p, double max_d2,
+                                               uint32_t i, int* nn_idx, float* nn_d2) {
+  __shared__ unsigned long long sh[BRT / 32];
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  Best1 best;
+  best.init();
+  for (int base = 0; base < n_points; base += BRT * 8) {
+    float4 q[8];
+#pragma unroll
+    for (int u = 0; u < 8; ++u) {
+      const int t = base + u * BRT + (int)threadIdx.x;
+      q[u] = t < n_points ? __ldg(sorted + t) : make_float4(CUDART_INF_F, 0.f, 0.f, __int_as_float(-1));
+    }
+#pragma unroll
+    for (int u = 0; u < 8; ++u) best.push(sor_d2(p, q[u]), q[u].w);
+  }
+  const unsigned long long wm = warp_min_u64(best.key);
+  if (lane == 0) sh[w] = wm;
+  __syncthreads();
+  if (w == 0) {
+    unsigned long long v = lane < BRT / 32 ? sh[lane] : ~0ULL;
+    v = warp_min_u64(v);
+    if (lane == 0) {
+      Best1 b;
+      b.key = v;
+      const bool ok = (double)b.d2() <= max_d2;  // exhaustive: always the true nearest point
+      nn_idx[i] = ok ? b.idx() : -1;
+      nn_d2[i] = b.d2();
+    }
+  }
+  __syncthreads();
+}
+
 __global__ void __launch_bounds__(BRT)
 icp_brute_kernel(const IcpArgs A) {
-  __shared__ unsigned long long sh[BRT / 32];
   if (!A.fitness && A.st->done) return;
   const double max_d2 = A.fitness ? CUDART_INF : A.st->max_d2;
   const int n_points = A.gp->n_points;
   const unsigned n_brute = A.st->n_brute;
-  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
   for (unsigned e = blockIdx.x; e < n_brute; e += gridDim.x) {
     const uint32_t i = A.left_list[A.ns + e];
-    const float4 p = A.cur[i];
-    Best1 best;
-    best.init();
-    for (int base = 0; base < n_points; base += BRT * 8) {
-      float4 q[8];
-#pragma unroll
-      for (int u = 0; u < 8; ++u) {
-        const int t = base + u * BRT + (int)threadIdx.x;
-        q[u] = t < n_points ? __ldg(A.sorted + t) : make_float4(CUDART_INF_F, 0.f, 0.f, __int_as_float(-1));
-      }
-#pragma unroll
-      for (int u = 0; u < 8; ++u) best.push(sor_d2(p, q[u]), q[u].w);
-    }
-    const unsigned long long wm = warp_min_u64(best.key);
-    if (lane == 0) sh[w] = wm;
-    __syncthreads();
-    if (w == 0) {
-      unsigned long long v = lane < BRT / 32 ? sh[lane] : ~0ULL;
-      v = warp_min_u64(v);
-      if (lane == 0) {
-        Best1 b;
-        b.key = v;
-        const bool ok = (double)b.d2() <= max_d2;  // exhaustive: always the true nearest point
-        A.nn_idx[i] = ok ? b.idx() : -1;
-        A.nn_d2[i] = b.d2();
-      }
-    }
-    __syncthreads();
+    nn_brute_block(A.sorted, n_points, A.cur[i], max_d2, i, A.nn_idx, A.nn_d2);
   }
 }
 
@@ -324,25 +353,29 @@ __device__ void icp_finalize(IcpDevState* st, const double* S) {
   if (state != 0) st->done = 1;
 }
 
+// One block's part of the reduction of a pair of ns source points over nblk blocks (lb = this block's index among
+// them): the f64 sums of its grid-stride share of the correspondences (d^2 <= max^2; only the squared distances and
+// the count for the fitness score), a shuffle tree, the block's row of `partials`; then the block that takes the last
+// ticket folds the pair's rows in a fixed order.  Returns the pair's ICP_SUMS sums (shared memory) in that block,
+// nullptr in the others.
 constexpr int RD_THREADS = 256;
-__global__ void __launch_bounds__(RD_THREADS)
-icp_reduce_kernel(const IcpArgs A) {
+__device__ __forceinline__ const double* icp_reduce_block(const int* nn_idx, const float* nn_d2, const float4* cur,
+                                                          const float4* tgt, int ns, int lb, int nblk, double* partials,
+                                                          IcpDevState* st, int fitness) {
   __shared__ double sh[RD_THREADS / 32][ICP_SUMS];
   __shared__ bool s_last;
-  IcpDevState* st = A.st;
-  if (!A.fitness && st->done) return;
-  const double max_d2 = A.fitness ? CUDART_INF : st->max_d2;
+  const double max_d2 = fitness ? CUDART_INF : st->max_d2;
   double acc[ICP_SUMS];
 #pragma unroll
   for (int q = 0; q < ICP_SUMS; ++q) acc[q] = 0.0;
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < A.ns; i += gridDim.x * blockDim.x) {
-    const int j = A.nn_idx[i];
-    const float d2 = A.nn_d2[i];
+  for (int i = lb * blockDim.x + threadIdx.x; i < ns; i += nblk * blockDim.x) {
+    const int j = nn_idx[i];
+    const float d2 = nn_d2[i];
     if (j < 0 || (double)d2 > max_d2) continue;
     acc[15] += (double)d2;
     acc[16] += 1.0;
-    if (!A.fitness) {
-      const float4 s = A.cur[i], t = A.tgt[j];
+    if (!fitness) {
+      const float4 s = cur[i], t = tgt[j];
       const double sv[3] = {s.x, s.y, s.z}, tv[3] = {t.x, t.y, t.z};
 #pragma unroll
       for (int a = 0; a < 3; ++a) {
@@ -365,19 +398,19 @@ icp_reduce_kernel(const IcpArgs A) {
   if (threadIdx.x < ICP_SUMS) {
     double v = 0.0;
     for (int k = 0; k < RD_THREADS / 32; ++k) v += sh[k][threadIdx.x];
-    A.partials[(size_t)blockIdx.x * ICP_SUMS + threadIdx.x] = v;
+    partials[(size_t)lb * ICP_SUMS + threadIdx.x] = v;
   }
   __threadfence();
   __syncthreads();
-  if (threadIdx.x == 0) s_last = atomicAdd(&st->ticket, 1u) == gridDim.x - 1;
+  if (threadIdx.x == 0) s_last = atomicAdd(&st->ticket, 1u) == (unsigned)nblk - 1;
   __syncthreads();
-  if (!s_last) return;
+  if (!s_last) return nullptr;
   __threadfence();
   {  // fixed order: eight interleaved slices of the blocks (their loads in flight together), then the slices
     const int q = threadIdx.x & 31, slice = threadIdx.x >> 5;
     double v = 0.0;
     if (q < ICP_SUMS) {
-      for (unsigned b = slice; b < gridDim.x; b += RD_THREADS / 32) v += A.partials[(size_t)b * ICP_SUMS + q];
+      for (int b = slice; b < nblk; b += RD_THREADS / 32) v += partials[(size_t)b * ICP_SUMS + q];
       sh[slice][q] = v;
     }
   }
@@ -388,12 +421,21 @@ icp_reduce_kernel(const IcpArgs A) {
     sh[0][threadIdx.x] = v;
   }
   __syncthreads();
-  if (threadIdx.x == 0) {
+  return sh[0];
+}
+
+__global__ void __launch_bounds__(RD_THREADS)
+icp_reduce_kernel(const IcpArgs A) {
+  IcpDevState* st = A.st;
+  if (!A.fitness && st->done) return;
+  const double* S = icp_reduce_block(A.nn_idx, A.nn_d2, A.cur, A.tgt, A.ns, (int)blockIdx.x, (int)gridDim.x, A.partials,
+                                     st, A.fitness);
+  if (S && threadIdx.x == 0) {
     if (A.fitness) {
-      st->fit_nr = (int)sh[0][16];
-      st->fitness = sh[0][16] > 0.0 ? sh[0][15] / sh[0][16] : DBL_MAX;
+      st->fit_nr = (int)S[16];
+      st->fitness = S[16] > 0.0 ? S[15] / S[16] : DBL_MAX;
     } else {
-      icp_finalize(st, sh[0]);
+      icp_finalize(st, S);
     }
     st->ticket = 0;
     st->n_left = 0;
@@ -402,9 +444,9 @@ icp_reduce_kernel(const IcpArgs A) {
 }
 
 // ---- many pairs at once (liogpu_loop_closure_icp_batch) ----
-// Every pair keeps its own IcpDevState and its own grid; the search gives each point the same nearest target point as
-// the single-pair kernels (the search is exact, ties go to the lower target index, whatever the grid), and the reduction
-// sums each pair in the exact order of icp_reduce_kernel, so every pair's result is bit-equal to icp_align_dev.
+// Every pair keeps its own IcpDevState and its own grid; the search is exact (ties go to the lower target index,
+// whatever the grid) and each pair is reduced over as many blocks as icp_align_dev launches for it, so every pair's
+// result is bit-equal to icp_align_dev.
 // The targets of all pairs share one sorted array: key = cell_base[pair] + the cell inside the pair's grid, so a pair's
 // points form one contiguous run and cell_start + cell_base[pair] is that pair's cell_start.
 
@@ -446,7 +488,7 @@ __device__ __forceinline__ int find_seg(const int* __restrict__ off, int n, int 
   return lo;
 }
 
-// block per pair: bounding box and finite count of its target, then grid_setup_kernel's choice of grid
+// block per pair: bounding box and finite count of its target, then its grid
 constexpr int BB_THREADS = 256;
 __global__ void __launch_bounds__(BB_THREADS)
 icpb_grid_kernel(const float4* __restrict__ tgt, const int* __restrict__ tp, float cell, unsigned max_cells,
@@ -477,36 +519,12 @@ icpb_grid_kernel(const float4* __restrict__ tgt, const int* __restrict__ tp, flo
   }
   __syncthreads();
   if (threadIdx.x != 0) return;
-  GridParams g;
-  g.n_points = 0;
+  int n_points = 0;
   for (int k = 0; k < BB_THREADS / 32; ++k) {
     for (int a = 0; a < 3; ++a) { mn[a] = fminf(mn[a], s_mn[a][k]); mx[a] = fmaxf(mx[a], s_mx[a][k]); }
-    g.n_points += s_cnt[k];
+    n_points += s_cnt[k];
   }
-  if (g.n_points <= 0) { mn[0] = mn[1] = mn[2] = 0.f; mx[0] = mx[1] = mx[2] = 0.f; }
-  float maxabs = 1.0f;
-  for (int a = 0; a < 3; ++a) {
-    maxabs = fmaxf(maxabs, fmaxf(fabsf(mn[a]), fabsf(mx[a])));
-    maxabs = fmaxf(maxabs, mx[a] - mn[a]);
-  }
-  g.ox = mn[0]; g.oy = mn[1]; g.oz = mn[2];
-  float h = cell;
-  for (;;) {
-    const float inv = 1.0f / h;
-    const double nx = floor((double)(mx[0] - mn[0]) * inv) + 1, ny = floor((double)(mx[1] - mn[1]) * inv) + 1,
-                 nz = floor((double)(mx[2] - mn[2]) * inv) + 1;
-    if (nx * ny * nz <= (double)max_cells) {
-      g.nx = (int)nx; g.ny = (int)ny; g.nz = (int)nz;
-      g.h = h; g.inv_h = inv;
-      break;
-    }
-    h *= 2.0f;
-  }
-  g.n_cells = (unsigned)g.nx * (unsigned)g.ny * (unsigned)g.nz;
-  g.slack = maxabs * 9.5367431640625e-07f;  // 2^-20, as grid_setup_kernel
-  g.gate_d2 = 1.0f;
-  g.gate1_d2 = 1.0f;
-  gp[p] = g;
+  gp[p] = grid_setup_compute(mn, mx, n_points, cell, max_cells, 1.0f, 1.0f);
 }
 
 __global__ void __launch_bounds__(256)
@@ -520,9 +538,9 @@ icpb_key_kernel(const float4* __restrict__ tgt, int nt, const int* __restrict__ 
   if (isfinite(q.x) && isfinite(q.y) && isfinite(q.z)) {
     const int p = find_seg(tp, n, i);
     const GridParams g = gp[p];
-    const int cx = sor_cell(q.x, g.ox, g.inv_h, g.nx);
-    const int cy = sor_cell(q.y, g.oy, g.inv_h, g.ny);
-    const int cz = sor_cell(q.z, g.oz, g.inv_h, g.nz);
+    const int cx = cell_coord(q.x, g.ox, g.inv_h, g.nx);
+    const int cy = cell_coord(q.y, g.oy, g.inv_h, g.ny);
+    const int cz = cell_coord(q.z, g.oz, g.inv_h, g.nz);
     key = cell_base[p] + ((uint32_t)cz * (uint32_t)g.ny + (uint32_t)cy) * (uint32_t)g.nx + (uint32_t)cx;
     atomicAdd(&cell_count[key], 1u);
   }
@@ -539,8 +557,8 @@ icpb_gather_kernel(const float4* __restrict__ tgt, const uint32_t* __restrict__ 
   sorted[j] = make_float4(q.x, q.y, q.z, __int_as_float(src - tp[find_seg(tp, n, src)]));
 }
 
-// thread per source point of every live pair: shells 0..2 (icp_nn_kernel); the block's points that need more are then
-// taken warp per point for shells 3..5 (icp_left_kernel), starting from the nearest point the thread already found
+// thread per source point of every live pair: shells 0..NN_THREAD_SHELLS-1; the block's points that need more are
+// then taken warp per point for the remaining shells, starting from the nearest point the thread already found
 constexpr int NB_THREADS = 128;
 __global__ void __launch_bounds__(NB_THREADS)
 icpb_nn_kernel(const IcpbArgs A) {
@@ -568,19 +586,9 @@ icpb_nn_kernel(const IcpbArgs A) {
         A.nn_d2[i] = CUDART_INF_F;
       } else {
         const GridParams g = A.gp[p];
-        const uint32_t* cs = A.cs + A.cell_base[p];
         const double max_d2 = A.fitness ? CUDART_INF : st->max_d2;
-        const HomeCell hc = home_cell(g, q);
         Best1 best;
-        best.init();
-        int verdict = 0;
-        for (int R = 0; R < NN_THREAD_SHELLS && verdict == 0; ++R) {
-          const int z0 = max(hc.cz - R, 0), z1 = min(hc.cz + R, g.nz - 1);
-          const int y0 = max(hc.cy - R, 0), y1 = min(hc.cy + R, g.ny - 1);
-          for (int z = z0; z <= z1; ++z)
-            for (int y = y0; y <= y1; ++y) scan_shell_row(A.sorted, cs, g, hc, R, y, z, q, best);
-          verdict = nn_verdict(best, covered_d2(g, hc, R), max_d2);
-        }
+        const int verdict = nn_thread_walk(A.sorted, A.cs + A.cell_base[p], g, q, max_d2, best);
         if (verdict == 0) {
           const int slot = atomicAdd(&s_n, 1);
           s_i[slot] = i; s_p[slot] = p; s_key[slot] = best.key; s_pt[slot] = q;
@@ -597,25 +605,11 @@ icpb_nn_kernel(const IcpbArgs A) {
     const int i = s_i[e], p = s_p[e];
     const float4 q = s_pt[e];
     const GridParams g = A.gp[p];
-    const uint32_t* cs = A.cs + A.cell_base[p];
     const double max_d2 = A.fitness ? CUDART_INF : A.st[p].max_d2;
-    const HomeCell hc = home_cell(g, q);
-    Best1 best;
-    best.init();
-    if (lane == 0) best.key = s_key[e];
-    Best1 all;
-    all.init();
-    int verdict = 0;
-    for (int R = NN_THREAD_SHELLS; R < NN_WARP_SHELLS && verdict == 0; ++R) {
-      const int side = 2 * R + 1, rows = side * side;
-      for (int r = lane; r < rows; r += 32) {
-        const int z = hc.cz + r / side - R, y = hc.cy + r % side - R;
-        if (z < 0 || z >= g.nz || y < 0 || y >= g.ny) continue;
-        scan_shell_row(A.sorted, cs, g, hc, R, y, z, q, best);
-      }
-      all.key = warp_min_u64(best.key);
-      verdict = nn_verdict(all, covered_d2(g, hc, R), max_d2);
-    }
+    Best1 seed, all;
+    seed.init();
+    if (lane == 0) seed.key = s_key[e];
+    const int verdict = nn_warp_walk(A.sorted, A.cs + A.cell_base[p], g, q, max_d2, NN_THREAD_SHELLS, seed, all);
     if (lane == 0) {
       if (verdict == 0) {
         A.brute[atomicAdd(&A.cnt->n_brute[A.par], 1u)] = (uint32_t)i;
@@ -627,127 +621,73 @@ icpb_nn_kernel(const IcpbArgs A) {
   }
 }
 
-// block per isolated point: one pass over its pair's finite targets (icp_brute_kernel)
+// block per isolated point: one pass over its pair's finite targets
 __global__ void __launch_bounds__(BRT)
 icpb_brute_kernel(const IcpbArgs A) {
-  __shared__ unsigned long long sh[BRT / 32];
   const unsigned n_brute = A.cnt->n_brute[A.par];
-  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
   for (unsigned e = blockIdx.x; e < n_brute; e += gridDim.x) {
     const uint32_t i = A.brute[e];
     const int p = find_seg(A.sp, A.n, (int)i);
-    const float4 pt = A.cur[i];
-    const float4* sorted = A.sorted + A.cs[A.cell_base[p]];
-    const int n_points = A.gp[p].n_points;
     const double max_d2 = A.fitness ? CUDART_INF : A.st[p].max_d2;
-    Best1 best;
-    best.init();
-    for (int base = 0; base < n_points; base += BRT * 8) {
-      float4 q[8];
-#pragma unroll
-      for (int u = 0; u < 8; ++u) {
-        const int t = base + u * BRT + (int)threadIdx.x;
-        q[u] = t < n_points ? __ldg(sorted + t) : make_float4(CUDART_INF_F, 0.f, 0.f, __int_as_float(-1));
-      }
-#pragma unroll
-      for (int u = 0; u < 8; ++u) best.push(sor_d2(pt, q[u]), q[u].w);
-    }
-    const unsigned long long wm = warp_min_u64(best.key);
-    if (lane == 0) sh[w] = wm;
-    __syncthreads();
-    if (w == 0) {
-      unsigned long long v = lane < BRT / 32 ? sh[lane] : ~0ULL;
-      v = warp_min_u64(v);
-      if (lane == 0) {
-        Best1 b;
-        b.key = v;
-        const bool ok = (double)b.d2() <= max_d2;
-        A.nn_idx[i] = ok ? b.idx() : -1;
-        A.nn_d2[i] = b.d2();
-      }
-    }
-    __syncthreads();
+    nn_brute_block(A.sorted + A.cs[A.cell_base[p]], A.gp[p].n_points, A.cur[i], max_d2, i, A.nn_idx, A.nn_d2);
   }
 }
 
-// icp_reduce_kernel for every live pair: pair p owns blocks rp[p] .. rp[p+1] (min(ceil(ns / 256), 256) of them, as the
-// single call launches), the same grid-stride assignment, shuffle tree and fold; the pair's last block runs its tail
+// every live pair's reduction: pair p owns blocks rp[p] .. rp[p+1], icp_reduce_blocks of them as for the pair alone
 __global__ void __launch_bounds__(RD_THREADS)
 icpb_reduce_kernel(const IcpbArgs A) {
-  __shared__ double sh[RD_THREADS / 32][ICP_SUMS];
-  __shared__ bool s_last;
   const int p = find_seg(A.rp, A.n, (int)blockIdx.x);
   IcpDevState* st = A.st + p;
   if (!A.fitness && st->done) return;
-  const double max_d2 = A.fitness ? CUDART_INF : st->max_d2;
-  const int rb0 = A.rp[p], nblk = A.rp[p + 1] - rb0, lb = (int)blockIdx.x - rb0;
-  const int s0 = A.sp[p], ns = A.sp[p + 1] - s0, t0 = A.tp[p];
-  double acc[ICP_SUMS];
-#pragma unroll
-  for (int q = 0; q < ICP_SUMS; ++q) acc[q] = 0.0;
-  for (int i = lb * RD_THREADS + (int)threadIdx.x; i < ns; i += nblk * RD_THREADS) {
-    const int j = A.nn_idx[s0 + i];
-    const float d2 = A.nn_d2[s0 + i];
-    if (j < 0 || (double)d2 > max_d2) continue;
-    acc[15] += (double)d2;
-    acc[16] += 1.0;
-    if (!A.fitness) {
-      const float4 s = A.cur[s0 + i], t = A.tgt[t0 + j];
-      const double sv[3] = {s.x, s.y, s.z}, tv[3] = {t.x, t.y, t.z};
-#pragma unroll
-      for (int a = 0; a < 3; ++a) {
-        acc[a] += sv[a];
-        acc[3 + a] += tv[a];
-#pragma unroll
-        for (int b = 0; b < 3; ++b) acc[6 + 3 * a + b] += tv[a] * sv[b];
-      }
-    }
-  }
-  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-#pragma unroll
-  for (int q = 0; q < ICP_SUMS; ++q) {
-    double v = acc[q];
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
-    if (lane == 0) sh[w][q] = v;
-  }
-  __syncthreads();
-  if (threadIdx.x < ICP_SUMS) {
-    double v = 0.0;
-    for (int k = 0; k < RD_THREADS / 32; ++k) v += sh[k][threadIdx.x];
-    A.partials[(size_t)blockIdx.x * ICP_SUMS + threadIdx.x] = v;
-  }
-  __threadfence();
-  __syncthreads();
-  if (threadIdx.x == 0) s_last = atomicAdd(&st->ticket, 1u) == (unsigned)nblk - 1;
-  __syncthreads();
-  if (!s_last) return;
-  __threadfence();
-  {
-    const int q = threadIdx.x & 31, slice = threadIdx.x >> 5;
-    double v = 0.0;
-    if (q < ICP_SUMS) {
-      for (int b = slice; b < nblk; b += RD_THREADS / 32) v += A.partials[(size_t)(rb0 + b) * ICP_SUMS + q];
-      sh[slice][q] = v;
-    }
-  }
-  __syncthreads();
-  if (threadIdx.x < ICP_SUMS) {
-    double v = 0.0;
-    for (int k = 0; k < RD_THREADS / 32; ++k) v += sh[k][threadIdx.x];
-    sh[0][threadIdx.x] = v;
-  }
-  __syncthreads();
-  if (threadIdx.x == 0) {
+  const int rb0 = A.rp[p], s0 = A.sp[p], t0 = A.tp[p];
+  const double* S = icp_reduce_block(A.nn_idx + s0, A.nn_d2 + s0, A.cur + s0, A.tgt + t0, A.sp[p + 1] - s0,
+                                     (int)blockIdx.x - rb0, A.rp[p + 1] - rb0, A.partials + (size_t)rb0 * ICP_SUMS, st,
+                                     A.fitness);
+  if (S && threadIdx.x == 0) {
     if (A.fitness) {
-      st->fit_nr = (int)sh[0][16];
-      st->fitness = sh[0][16] > 0.0 ? sh[0][15] / sh[0][16] : DBL_MAX;
+      st->fit_nr = (int)S[16];
+      st->fitness = S[16] > 0.0 ? S[15] / S[16] : DBL_MAX;
     } else {
-      icp_finalize(st, sh[0]);
+      icp_finalize(st, S);
       if (st->done) atomicSub(&A.cnt->live, 1);
     }
     st->ticket = 0;
   }
+}
+
+// Iterations enqueued between two host checks of convergence.  Both drivers enqueue the same number of iterations, so
+// a batch does no more iterations for a pair than icp_align_dev would for it alone.
+constexpr int ICP_CHUNK = 10;
+
+// grid cell edge; tuning only (the search is exact).  Measured: 0.5 m 1.33 ms, 1 m 1.58 ms, 1.5 m 1.96 ms
+float icp_cell_size(const liogpu_icp_params* prm) { return prm->cell_size > 0.f ? prm->cell_size : 0.5f; }
+
+// reduce blocks of a pair of ns source points
+int icp_reduce_blocks(int ns) { return div_up(ns, RD_THREADS) < 256 ? div_up(ns, RD_THREADS) : 256; }
+
+// IcpDevState before the first iteration
+void icp_state_init(IcpDevState& s, const liogpu_icp_params* prm) {
+  memset(&s, 0, sizeof(IcpDevState));
+  for (int q = 0; q < 16; ++q) s.T_inc[q] = s.finalT[q] = (q % 5 == 0) ? 1.f : 0.f;
+  s.prev_mse = DBL_MAX;
+  s.max_d2 = (double)prm->max_correspondence_distance * (double)prm->max_correspondence_distance;
+  s.rot_thr = 1.0 - prm->transformation_epsilon;   // transformation_rotation_epsilon_ unset (icp.hpp)
+  s.trans_thr = prm->transformation_epsilon;
+  s.rel_thr = prm->euclidean_fitness_epsilon;
+  s.abs_thr = 1e-12;
+  s.max_iter = prm->max_iterations;
+}
+
+// the caller's result from the final IcpDevState
+void icp_result(const IcpDevState& s, float gpu_ms, float final_T[16], liogpu_icp_info* info) {
+  for (int q = 0; q < 16; ++q) final_T[q] = s.finalT[q];
+  info->iterations = s.iter;
+  info->convergence_state = s.state;
+  info->converged = (s.state >= 1 && s.state <= 4) ? 1 : 0;
+  info->n_correspondences = s.n_corr;
+  info->fitness_score = s.fitness;
+  info->last_mse = s.last_mse;
+  info->gpu_ms = gpu_ms;
 }
 
 }  // namespace
@@ -757,10 +697,8 @@ icpb_reduce_kernel(const IcpbArgs A) {
 int icp_align_dev(Ctx* c, const float4* src, int ns, const float4* tgt, int nt, const liogpu_icp_params* prm,
                   float final_T[16], liogpu_icp_info* info) {
   GridParams g;
-  const float cell = prm->cell_size > 0.f ? prm->cell_size : 0.5f;  // measured: 0.5 m 1.33 ms, 1 m 1.58 ms, 1.5 m 1.96 ms
-  int rc = grid_build_core(c, tgt, nt, cell, 1.0f, 1.0f, c->sor_setup, c->sor_sorted, c->sor_cell_start, g);
+  int rc = grid_build_core(c, tgt, nt, icp_cell_size(prm), 1.0f, 1.0f, c->sor_setup, c->sor_sorted, c->sor_cell_start, g);
   if (rc) return rc;
-  const int rblocks = div_up(ns, RD_THREADS) < 256 ? div_up(ns, RD_THREADS) : 256;
   LIOGPU_CUDA_OK(c, c->lm_a.reserve((size_t)ns * sizeof(float4)));
   LIOGPU_CUDA_OK(c, c->lm_flag.reserve((size_t)ns * sizeof(int)));
   LIOGPU_CUDA_OK(c, c->lm_md.reserve((size_t)ns * sizeof(float)));
@@ -777,29 +715,20 @@ int icp_align_dev(Ctx* c, const float4* src, int ns, const float4* tgt, int nt, 
   A.fitness = 0;
   A.all_warp = (ns <= 65536 && !getenv("LIOGPU_ICP_THREAD_PASS")) ? 1 : 0;
   IcpDevState* h = reinterpret_cast<IcpDevState*>((char*)c->h_pinned + 12288);
-  memset(h, 0, sizeof(IcpDevState));
-  for (int q = 0; q < 16; ++q) h->T_inc[q] = h->finalT[q] = (q % 5 == 0) ? 1.f : 0.f;
-  h->prev_mse = DBL_MAX;
-  h->max_d2 = (double)prm->max_correspondence_distance * (double)prm->max_correspondence_distance;
-  h->rot_thr = 1.0 - prm->transformation_epsilon;   // transformation_rotation_epsilon_ unset (icp.hpp)
-  h->trans_thr = prm->transformation_epsilon;
-  h->rel_thr = prm->euclidean_fitness_epsilon;
-  h->abs_thr = 1e-12;
-  h->max_iter = prm->max_iterations;
+  icp_state_init(*h, prm);
   LIOGPU_CUDA_OK(c, cudaMemcpyAsync(A.st, h, sizeof(IcpDevState), cudaMemcpyHostToDevice, c->stream));
   LIOGPU_CUDA_OK(c, cudaMemcpyAsync(A.cur, src, (size_t)ns * sizeof(float4), cudaMemcpyDeviceToDevice, c->stream));
   LIOGPU_CUDA_OK(c, cudaEventRecord(c->ev0, c->stream));
-  const int CHUNK = 10;
   int launched = 0;
   auto enqueue_iteration = [&](const IcpArgs& a) {
     if (!a.all_warp) icp_nn_kernel<<<div_up(ns, NN_THREADS), NN_THREADS, 0, c->stream>>>(a);
     icp_left_kernel<<<a.all_warp ? c->sm_count * 8 : c->sm_count * 2, 256, 0, c->stream>>>(a);
     icp_brute_kernel<<<c->sm_count, BRT, 0, c->stream>>>(a);
-    icp_reduce_kernel<<<rblocks, RD_THREADS, 0, c->stream>>>(a);
+    icp_reduce_kernel<<<icp_reduce_blocks(ns), RD_THREADS, 0, c->stream>>>(a);
     c->launches += a.all_warp ? 3 : 4;
   };
   for (;;) {
-    const int todo = (prm->max_iterations - launched) < CHUNK ? (prm->max_iterations - launched) : CHUNK;
+    const int todo = (prm->max_iterations - launched) < ICP_CHUNK ? (prm->max_iterations - launched) : ICP_CHUNK;
     for (int it = 0; it < todo; ++it) enqueue_iteration(A);
     launched += todo;
     LIOGPU_CUDA_OK(c, cudaGetLastError());
@@ -816,27 +745,16 @@ int icp_align_dev(Ctx* c, const float4* src, int ns, const float4* tgt, int nt, 
   LIOGPU_CUDA_OK(c, cudaMemcpyAsync(h, A.st, sizeof(IcpDevState), cudaMemcpyDeviceToHost, c->stream));
   LIOGPU_CUDA_OK(c, cudaStreamSynchronize(c->stream));
   cudaEventElapsedTime(&c->last_ms, c->ev0, c->ev1);
-  for (int q = 0; q < 16; ++q) final_T[q] = h->finalT[q];
-  info->iterations = h->iter;
-  info->convergence_state = h->state;
-  info->converged = (h->state >= 1 && h->state <= 4) ? 1 : 0;
-  info->n_correspondences = h->n_corr;
-  info->fitness_score = h->fitness;
-  info->last_mse = h->last_mse;
-  info->gpu_ms = c->last_ms;
+  icp_result(*h, c->last_ms, final_T, info);
   return LIOGPU_OK;
 }
-
 
 int icp_batch_dev(Ctx* c, const float4* src, const int* so, const float4* tgt, const int* to, int n,
                   const liogpu_icp_params* prm, float (*final_T)[16], liogpu_icp_info* info) {
   if (n <= 0) return LIOGPU_OK;
   const int ns = so[n], nt = to[n];
   std::vector<int> rp(n + 1, 0);
-  for (int p = 0; p < n; ++p) {
-    const int blocks = div_up(so[p + 1] - so[p], RD_THREADS);
-    rp[p + 1] = rp[p] + (blocks < 256 ? blocks : 256);
-  }
+  for (int p = 0; p < n; ++p) rp[p + 1] = rp[p] + icp_reduce_blocks(so[p + 1] - so[p]);
   // device tables: sp | tp | rp | cell_base | gp | st | counters | partials
   auto up256 = [](size_t b) { return (b + 255) & ~(size_t)255; };
   const size_t o_tp = up256((size_t)(n + 1) * sizeof(int)), o_rp = o_tp + o_tp, o_cb = o_rp + o_tp;
@@ -849,17 +767,7 @@ int icp_batch_dev(Ctx* c, const float4* src, const int* so, const float4* tgt, c
   memcpy(h.data() + o_tp, to, (size_t)(n + 1) * sizeof(int));
   memcpy(h.data() + o_rp, rp.data(), (size_t)(n + 1) * sizeof(int));
   IcpDevState* hs = reinterpret_cast<IcpDevState*>(h.data() + o_st);
-  for (int p = 0; p < n; ++p) {  // as icp_align_dev
-    IcpDevState& s = hs[p];
-    for (int q = 0; q < 16; ++q) s.T_inc[q] = s.finalT[q] = (q % 5 == 0) ? 1.f : 0.f;
-    s.prev_mse = DBL_MAX;
-    s.max_d2 = (double)prm->max_correspondence_distance * (double)prm->max_correspondence_distance;
-    s.rot_thr = 1.0 - prm->transformation_epsilon;
-    s.trans_thr = prm->transformation_epsilon;
-    s.rel_thr = prm->euclidean_fitness_epsilon;
-    s.abs_thr = 1e-12;
-    s.max_iter = prm->max_iterations;
-  }
+  for (int p = 0; p < n; ++p) icp_state_init(hs[p], prm);
   reinterpret_cast<IcpbCounters*>(h.data() + o_cnt)->live = n;
   LIOGPU_CUDA_OK(c, cudaMemcpyAsync(d, h.data(), o_part, cudaMemcpyHostToDevice, c->stream));
   IcpbArgs A;
@@ -876,9 +784,8 @@ int icp_batch_dev(Ctx* c, const float4* src, const int* so, const float4* tgt, c
 
   // one segmented grid index over all targets.  The cell count per pair is capped so that the concatenated cells stay
   // within 2^28 (the grid's cell size never changes a result)
-  const float cell = prm->cell_size > 0.f ? prm->cell_size : 0.5f;
   const unsigned max_cells = (unsigned)((1u << 28) / (unsigned)n) < (1u << 25) ? (unsigned)((1u << 28) / (unsigned)n) : (1u << 25);
-  icpb_grid_kernel<<<n, BB_THREADS, 0, c->stream>>>(tgt, A.tp, cell, max_cells, d_gp);
+  icpb_grid_kernel<<<n, BB_THREADS, 0, c->stream>>>(tgt, A.tp, icp_cell_size(prm), max_cells, d_gp);
   c->launches++;
   LIOGPU_CUDA_OK(c, cudaGetLastError());
   std::vector<GridParams> hg(n);
@@ -927,7 +834,6 @@ int icp_batch_dev(Ctx* c, const float4* src, const int* so, const float4* tgt, c
   A.fitness = 0;
   A.par = 0;
   LIOGPU_CUDA_OK(c, cudaMemcpyAsync(A.cur, src, (size_t)ns * sizeof(float4), cudaMemcpyDeviceToDevice, c->stream));
-  const int CHUNK = 10;  // as icp_align_dev: the same number of iterations is enqueued as for the slowest pair alone
   int launched = 0;
   int* h_live = reinterpret_cast<int*>((char*)c->h_pinned + 12800);
   auto enqueue_iteration = [&](IcpbArgs& a) {
@@ -938,7 +844,7 @@ int icp_batch_dev(Ctx* c, const float4* src, const int* so, const float4* tgt, c
     a.par ^= 1;
   };
   for (;;) {
-    const int todo = (prm->max_iterations - launched) < CHUNK ? (prm->max_iterations - launched) : CHUNK;
+    const int todo = (prm->max_iterations - launched) < ICP_CHUNK ? (prm->max_iterations - launched) : ICP_CHUNK;
     for (int it = 0; it < todo; ++it) enqueue_iteration(A);
     launched += todo;
     LIOGPU_CUDA_OK(c, cudaGetLastError());
@@ -952,17 +858,7 @@ int icp_batch_dev(Ctx* c, const float4* src, const int* so, const float4* tgt, c
   std::vector<IcpDevState> hst(n);
   LIOGPU_CUDA_OK(c, cudaMemcpyAsync(hst.data(), A.st, (size_t)n * sizeof(IcpDevState), cudaMemcpyDeviceToHost, c->stream));
   LIOGPU_CUDA_OK(c, cudaStreamSynchronize(c->stream));
-  for (int p = 0; p < n; ++p) {
-    const IcpDevState& s = hst[p];
-    for (int q = 0; q < 16; ++q) final_T[p][q] = s.finalT[q];
-    info[p].iterations = s.iter;
-    info[p].convergence_state = s.state;
-    info[p].converged = (s.state >= 1 && s.state <= 4) ? 1 : 0;
-    info[p].n_correspondences = s.n_corr;
-    info[p].fitness_score = s.fitness;
-    info[p].last_mse = s.last_mse;
-    info[p].gpu_ms = 0.f;
-  }
+  for (int p = 0; p < n; ++p) icp_result(hst[p], 0.f, final_T[p], info + p);
   return LIOGPU_OK;
 }
 

@@ -55,7 +55,7 @@ __device__ __forceinline__ void sc_bin_block(const float4* __restrict__ pts, lon
     const double sc = ceil(((double)azim_angle / 360.0) * SC_SECTOR);    // :178
     int sector = isnan(sc) ? 0 : (int)sc;
     sector = max(min(SC_SECTOR, sector), 1);
-    atomicMax(&sh[(ring - 1) * SC_SECTOR + (sector - 1)], sc_f2ord(z));  // :181-182
+    atomicMax(&sh[(ring - 1) * SC_SECTOR + (sector - 1)], f2ord(z));  // :181-182
   }
   __syncthreads();
   for (int k = threadIdx.x; k < SC_BINS; k += blockDim.x)

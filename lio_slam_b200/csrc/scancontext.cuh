@@ -14,19 +14,11 @@ constexpr int SC_CHUNK = 4096;  // points per block when many keyframes are binn
 cudaError_t launch_sc_bin_keyframes(Ctx* c, const float4* const* srcs, const int* offs, const int* blk_off, int n,
                                     int n_blocks, double lidar_height, double max_radius, double* slots);
 
-// Order-preserving integer image of a float: atomicMax on the image is the max of the floats.
-__device__ __forceinline__ unsigned sc_f2ord(float f) {
-  const unsigned u = __float_as_uint(f);
-  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
-__device__ __forceinline__ float sc_ord2f(unsigned o) {
-  return __uint_as_float((o & 0x80000000u) ? (o & 0x7fffffffu) : ~o);
-}
 // image of NO_POINT (Scancontext.cpp:158), the initial value of every bin
-__device__ __forceinline__ unsigned sc_none() { return sc_f2ord(-1000.0f); }
+__device__ __forceinline__ unsigned sc_none() { return f2ord(-1000.0f); }
 // the descriptor entry of a bin's image: empty bins (still NO_POINT) -> 0 (:186-189)
 __device__ __forceinline__ double sc_bin_value(unsigned o) {
-  const float v = sc_ord2f(o);
+  const float v = ord2f(o);
   return v == -1000.0f ? 0.0 : (double)v;
 }
 

@@ -19,21 +19,15 @@ __device__ __forceinline__ float sor_d2(const float4& a, const float4& b) {
   return r;
 }
 
-__device__ __forceinline__ int sor_cell(float p, float o, float inv_h, int n) {  // == grid.cu cell_coord
-  int c = (int)((p - o) * inv_h);
-  c = c < 0 ? 0 : c;
-  return c >= n ? n - 1 : c;
-}
-
 struct HomeCell {
   int cx, cy, cz;
   float fx, fy, fz;  // position of the point inside its cell: distance to the cell's lower faces
 };
 __device__ __forceinline__ HomeCell home_cell(const GridParams& g, const float4& p) {
   HomeCell hc;
-  hc.cx = sor_cell(p.x, g.ox, g.inv_h, g.nx);
-  hc.cy = sor_cell(p.y, g.oy, g.inv_h, g.ny);
-  hc.cz = sor_cell(p.z, g.oz, g.inv_h, g.nz);
+  hc.cx = cell_coord(p.x, g.ox, g.inv_h, g.nx);
+  hc.cy = cell_coord(p.y, g.oy, g.inv_h, g.ny);
+  hc.cz = cell_coord(p.z, g.oz, g.inv_h, g.nz);
   hc.fx = (p.x - g.ox) - (float)hc.cx * g.h;
   hc.fy = (p.y - g.oy) - (float)hc.cy * g.h;
   hc.fz = (p.z - g.oz) - (float)hc.cz * g.h;

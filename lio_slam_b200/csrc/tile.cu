@@ -34,17 +34,12 @@ struct TilePlan {
   unsigned n_tile;    // finite points of this tile
 };
 
-__device__ __forceinline__ float tile_ord2f(unsigned o) {
-  const unsigned u = (o & 0x80000000u) ? (o & 0x7fffffffu) : ~o;
-  return __uint_as_float(u);
-}
-
 __global__ void tile_setup_kernel(const unsigned* __restrict__ mm, float leaf, TilePlan* __restrict__ plan) {
   if (threadIdx.x != 0 || blockIdx.x != 0) return;
   TilePlan p;
   p.n_valid = (int)mm[6];
   float mn[3], mx[3];
-  for (int a = 0; a < 3; ++a) { mn[a] = tile_ord2f(mm[a]); mx[a] = tile_ord2f(mm[3 + a]); }
+  for (int a = 0; a < 3; ++a) { mn[a] = ord2f(mm[a]); mx[a] = ord2f(mm[3 + a]); }
   const float inv = 1.0f / leaf;
   p.inv_leaf = inv;
   long long d[3];

@@ -17,14 +17,6 @@
 
 namespace liogpu {
 
-__device__ __forceinline__ unsigned f2ord(float f) {
-  const unsigned u = __float_as_uint(f);
-  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
-__device__ __forceinline__ float ord2f(unsigned o) {
-  const unsigned u = (o & 0x80000000u) ? (o & 0x7fffffffu) : ~o;
-  return __uint_as_float(u);
-}
 __device__ __forceinline__ bool finite3(const float4 p) { return isfinite(p.x) && isfinite(p.y) && isfinite(p.z); }
 
 // mm[0..2] = min (ordered uint), mm[3..5] = max, mm[6] = finite count
