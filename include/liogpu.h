@@ -408,6 +408,16 @@ int liogpu_detect_loop_distance(liogpu_ctx* ctx, const void* key_poses3d, int n_
                                 const void* key_times, int time_stride, double time_laser_info_cur,
                                 float search_radius, float time_diff, int* loop_key_pre);
 
+/* detectLoopClosureDistance for n_calls calls of the loop thread over one set of key poses: call j sees the first
+ * n_key_at[j] key poses (1..n_key, any order, repeats allowed) and time_laser_info_cur = time_cur[j].  loop_key_pre[j]
+ * is bit-equal to liogpu_detect_loop_distance on that prefix with that time.  Same pose / time layouts and argument
+ * rules as liogpu_detect_loop_distance; malformed arguments are refused (LIOGPU_E_INVALID) before any launch.  The
+ * registration's local map and index and the resident cloud are left untouched; liogpu_last_gpu_ms covers the call.
+ * One sorted-grid index over all key poses answers every call: the number of launches does not depend on n_calls. */
+int liogpu_detect_loops_distance(liogpu_ctx* ctx, const void* key_poses3d, int n_key, int stride3d,
+                                 const void* key_times, int time_stride, const int* n_key_at, const double* time_cur,
+                                 int n_calls, float search_radius, float time_diff, int* loop_key_pre);
+
 /* ---- key-pose selection (SURVEY §8 row f4): extractNearby (MO:1519-1554) + the guard of extractCloud (MO:1562).
  * key_poses3d = cloudKeyPoses3D->points (x, y, z, intensity = keyframe index; n_key records of stride3d bytes),
  * key_times = the `time` field of cloudKeyPoses6D->points (n_key doubles, time_stride bytes apart: 8 for a plain

@@ -249,7 +249,7 @@ int liogpu_create(liogpu_ctx** out, const liogpu_params* params) {
                       &c.tile_hist, &c.tile_pts, &c.tile_out, &c.dbg_idx, &c.dbg_d2, &c.dbg_coeff, &c.dbg_flag, &c.dbg_tie,
                       &c.imu_tab, &c.dsk_flags, &c.dsk_scan, &c.lm_flag, &c.lm_pos, &c.lm_a, &c.lm_b, &c.lm_md, &c.lm_left,
                       &c.lm_out, &c.lm_stats, &c.sor_setup, &c.sor_sorted, &c.sor_cell_start, &c.kf_tab,
-                      &c.sc_q, &c.sc_part, &c.sc_cand, &c.sc_out, &c.lc_src, &c.lc_tgt, &c.lc_tab, &c.mw_tab, &c.mw_seg};
+                      &c.sc_q, &c.sc_part, &c.sc_cand, &c.sc_out, &c.lc_src, &c.lc_tgt, &c.lc_tab, &c.mw_tab, &c.mw_seg, &c.ld_tab};
     for (DevBuf* b : bufs) { b->stream = c.stream; b->async = true; }
   }
   // scratch hint of allocateMemory (mapOptmization.cpp:333-335)
@@ -277,7 +277,7 @@ void liogpu_destroy(liogpu_ctx* ctx) {
                     &c.fail_buf, &c.prev_nn, &c.hopeless, &c.fz_rows, &c.fz_left, &c.fz_lb, &c.fz_probe, &c.tile_plan, &c.tile_hist, &c.tile_pts, &c.tile_out, &c.dbg_idx, &c.dbg_d2, &c.dbg_coeff, &c.dbg_flag, &c.dbg_tie, &c.imu_tab, &c.dsk_flags, &c.dsk_scan,
                     &c.lm_flag, &c.lm_pos, &c.lm_a, &c.lm_b, &c.lm_md, &c.lm_left, &c.lm_out, &c.lm_stats, &c.sor_setup,
                     &c.sor_sorted, &c.sor_cell_start, &c.sc_q, &c.sc_part, &c.sc_cand, &c.sc_out, &c.lc_src, &c.lc_tgt,
-                    &c.lc_tab, &c.mw_tab, &c.mw_seg};
+                    &c.lc_tab, &c.mw_tab, &c.mw_seg, &c.ld_tab};
   for (DevBuf* b : bufs) b->release();
   sc_release(&c);
   for (auto& kv : c.keyframes) kv.second.first.release();
@@ -1115,6 +1115,30 @@ int liogpu_detect_loop_distance(liogpu_ctx* ctx, const void* key_poses3d, int n_
   for (int i = 0; i < n_key; ++i) std::memcpy(&times[i], (const char*)key_times + (size_t)i * time_stride, sizeof(double));
   return detect_loop_distance_dev(c, c->lm_a.as<float4>(), n_key, times.data(), time_laser_info_cur, search_radius, time_diff,
                                   loop_key_pre);
+}
+
+int liogpu_detect_loops_distance(liogpu_ctx* ctx, const void* key_poses3d, int n_key, int stride3d, const void* key_times,
+                                 int time_stride, const int* n_key_at, const double* time_cur, int n_calls,
+                                 float search_radius, float time_diff, int* loop_key_pre) {
+  NvtxRange nvtx_range_(__func__);
+  int rc = enter(ctx);
+  if (rc) return rc;
+  Ctx* c = &ctx->c;
+  bool ok = loop_key_pre && n_key > 0 && key_poses3d && key_times && time_stride >= 8 && search_radius > 0.f &&
+            !std::isnan(time_diff) && key_poses3d != LIOGPU_DEVICE_RESIDENT && key_poses3d != LIOGPU_UPLOADED_SCAN &&
+            stride_ok(stride3d) && n_key_at && time_cur && n_calls > 0;
+  for (int j = 0; ok && j < n_calls; ++j) ok = n_key_at[j] >= 1 && n_key_at[j] <= n_key;
+  if (!ok) {
+    c->err = "liogpu_detect_loops_distance: bad arguments";
+    return LIOGPU_E_INVALID;
+  }
+  LIOGPU_CUDA_OK(c, cudaEventRecord(c->ev0, c->stream));
+  rc = load_cloud(c, key_poses3d, n_key, stride3d, c->lm_a);  // the key-pose upload of liogpu_detect_loop_distance
+  if (rc) return rc;
+  std::vector<double> times((size_t)n_key);
+  for (int i = 0; i < n_key; ++i) std::memcpy(&times[i], (const char*)key_times + (size_t)i * time_stride, sizeof(double));
+  return detect_loops_distance_dev(c, c->lm_a.as<float4>(), n_key, times.data(), n_key_at, time_cur, n_calls, search_radius,
+                                   time_diff, loop_key_pre);
 }
 
 int liogpu_set_local_map(liogpu_ctx* ctx, const void* xyzi, int n, int stride) {

@@ -250,6 +250,9 @@ struct Ctx {
   // segmented VoxelGrid over many keyframe windows (voxel.cu merge_windows_dev): per-window tables of a pass, and the
   // segment table of the copy that places the windows' clouds
   DevBuf mw_tab, mw_seg;
+  // batched radius loop detection (loopdetect.cu detect_loops_distance_dev): the calls' prefix lengths, times and
+  // answers, and the key times in the order of the key-pose index (which lives in sor_setup / sor_sorted / sor_cell_start)
+  DevBuf ld_tab;
 };
 
 #define LIOGPU_CUDA_OK(ctx, expr)                                                        \
@@ -324,6 +327,10 @@ void sc_release(Ctx* c);
 int sc_detect_dev(Ctx* c, const std::vector<int2>& qm, int k, int R, double thres, ScQueryOut* h_out, liogpu_sc_info* info);
 int detect_loop_distance_dev(Ctx* c, const float4* key3d, int n, const double* h_times, double time_cur, float radius,
                              float time_diff, int* loop_key_pre);
+// detect_loop_distance_dev for n_calls calls at once: call j on the prefix of n_key_at[j] poses (1..n, host array) at
+// time_cur[j] (host); answers to the host array loop_key_pre.  The caller records ev0 (the call's start).
+int detect_loops_distance_dev(Ctx* c, const float4* key3d, int n, const double* h_times, const int* n_key_at,
+                              const double* time_cur, int n_calls, float radius, float time_diff, int* loop_key_pre);
 // --- icp.cu
 int icp_align_dev(Ctx* c, const float4* src, int ns, const float4* tgt, int nt, const liogpu_icp_params* prm,
                   float final_T[16], liogpu_icp_info* info);

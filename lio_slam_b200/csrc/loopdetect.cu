@@ -20,6 +20,9 @@
 //                        then distDirectSC for the search window's shifts (lanes over columns, ordered column sum)
 //   sc_final_kernel      thread per query: best candidate in kNN order, threshold, yaw
 // The online call (liogpu_sc_detect_loop) is a batch of one query.
+//
+// The radius detector: loop_distance_kernel answers one call (thread per key pose, atomicMin of a (d2, index) key);
+// loop_distance_batch_kernel answers many calls against one sorted-grid index of all key poses (warp per call).
 #include "scancontext.cuh"
 
 #include <algorithm>
@@ -287,17 +290,99 @@ sc_final_kernel(const int* __restrict__ cand, const double* __restrict__ cdist, 
   out[q].yaw = (float)((double)deg * 3.14159265358979323846 / 180.0);
 }
 
+// FLANN L2_Simple between the query key pose a and key pose b (nearby.cu: nb_d2).  Both radius detectors take their
+// d2 from here, so the per-call and the batched answers cannot drift apart.
+__device__ __forceinline__ float key_pose_d2(const float4 a, const float4 b) {
+  float d2 = 0.f;
+  float d = a.x - b.x; d2 += d * d;
+  d = a.y - b.y;       d2 += d * d;
+  d = a.z - b.z;       d2 += d * d;
+  return d2;
+}
+
 __global__ void __launch_bounds__(256)
 loop_distance_kernel(const float4* __restrict__ key3d, const double* __restrict__ key_time, int n, double time_cur, float r2,
                      double time_diff, u64* __restrict__ best) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
-  const float4 a = key3d[n - 1], b = key3d[i];
-  float d2 = 0.f;  // FLANN L2_Simple (nearby.cu: nb_d2)
-  float d = a.x - b.x; d2 += d * d;
-  d = a.y - b.y;       d2 += d * d;
-  d = a.z - b.z;       d2 += d * d;
+  const float d2 = key_pose_d2(key3d[n - 1], key3d[i]);
   if (d2 < r2 && fabs(key_time[i] - time_cur) > time_diff) atomicMin(best, ((u64)__float_as_uint(d2) << 32) | (unsigned)i);
+}
+
+// key times in the order of the sorted index (the .w of a sorted entry is the key-pose index)
+__global__ void __launch_bounds__(256)
+loop_time_gather_kernel(const float4* __restrict__ sorted, const double* __restrict__ key_time, int n_valid,
+                        double* __restrict__ time_sorted) {
+  const int j = blockIdx.x * blockDim.x + threadIdx.x;
+  if (j < n_valid) time_sorted[j] = key_time[__float_as_int(sorted[j].w)];
+}
+
+constexpr int LD_WARPS = 8;  // calls per block of the batched radius detector
+
+// Warp per call j: the minimum (bits(d2) << 32 | i) over the key poses i < m = n_key_at[j] within the radius and old
+// enough, i.e. loop_distance_kernel's answer on that prefix.  The minimum does not depend on the order in which the
+// candidates are offered, so any cell walk and lane split give the same answer.  The cell range per axis comes from
+// q +- (r + slack) as in grid_knn5 (s2m.cu), clamped in float before the conversion so that a huge or infinite radius
+// scans the whole grid without overflow.  The stable sort keeps a cell's members in ascending key-pose index, so the
+// walk of a cell stops at its first member >= m.
+__global__ void __launch_bounds__(LD_WARPS * 32)
+loop_distance_batch_kernel(const float4* __restrict__ key3d, const float4* __restrict__ sorted,
+                           const double* __restrict__ time_sorted, const uint32_t* __restrict__ cell_start, const GridParams g,
+                           const int* __restrict__ n_key_at, const double* __restrict__ time_cur, int n_calls, float radius,
+                           float r2, double time_diff, int* __restrict__ out) {
+  const int lane = threadIdx.x & 31;
+  const int j = blockIdx.x * LD_WARPS + (threadIdx.x >> 5);
+  if (j >= n_calls) return;  // warp-uniform
+  const int m = n_key_at[j];
+  const float4 q = key3d[m - 1];
+  const double tc = time_cur[j];
+  u64 best = ~0ULL;
+  // a non-finite query has d2 NaN or inf to every pose, never < r2: no candidate (and it is not in the grid)
+  if (isfinite(q.x) && isfinite(q.y) && isfinite(q.z)) {
+    const float reach = radius * 1.000001f + 2.0f * g.slack;
+    const float qc[3] = {q.x, q.y, q.z}, o[3] = {g.ox, g.oy, g.oz};
+    const int nc[3] = {g.nx, g.ny, g.nz};
+    int lo[3], hi[3];
+#pragma unroll
+    for (int a = 0; a < 3; ++a) {
+      const float top = (float)(nc[a] - 1);
+      lo[a] = (int)fminf(fmaxf(floorf((qc[a] - reach - o[a]) * g.inv_h), 0.f), top);
+      hi[a] = (int)fminf(fmaxf(floorf((qc[a] + reach - o[a]) * g.inv_h), 0.f), top);
+    }
+    for (int z = lo[2]; z <= hi[2]; ++z)
+      for (int y = lo[1]; y <= hi[1]; ++y) {
+        const uint32_t row = ((uint32_t)z * (uint32_t)g.ny + (uint32_t)y) * (uint32_t)g.nx;
+        for (int x = lo[0]; x <= hi[0]; ++x) {
+          const uint32_t s = __ldg(cell_start + row + x), e = __ldg(cell_start + row + x + 1);
+          for (uint32_t b = s; b < e; b += 32) {
+            const uint32_t k = b + lane;
+            bool past = false;
+            if (k < e) {
+              const float4 p = __ldg(sorted + k);
+              const int i = __float_as_int(p.w);
+              past = i >= m;
+              if (!past) {
+                const float d2 = key_pose_d2(q, p);
+                if (d2 < r2 && fabs(__ldg(time_sorted + k) - tc) > time_diff) {
+                  const u64 key = ((u64)__float_as_uint(d2) << 32) | (unsigned)i;
+                  best = key < best ? key : best;
+                }
+              }
+            }
+            if (__any_sync(0xffffffffu, past)) break;  // the rest of the cell lies past the prefix
+          }
+        }
+      }
+  }
+#pragma unroll
+  for (int off = 16; off > 0; off >>= 1) {
+    const u64 ob = __shfl_xor_sync(0xffffffffu, best, off);
+    best = ob < best ? ob : best;
+  }
+  if (lane == 0) {
+    const int w = best == ~0ULL ? -1 : (int)(unsigned)(best & 0xffffffffULL);
+    out[j] = w == m - 1 ? -1 : w;
+  }
 }
 
 cudaError_t sc_grow_array(Ctx* c, void** p, size_t old_bytes, size_t new_bytes) {
@@ -503,6 +588,50 @@ int detect_loop_distance_dev(Ctx* c, const float4* key3d, int n, const double* h
   cudaEventElapsedTime(&c->last_ms, c->ev0, c->ev1);
   const int best = *h == ~0ULL ? -1 : (int)(unsigned)(*h & 0xffffffffULL);
   *loop_key_pre = best == n - 1 ? -1 : best;
+  return LIOGPU_OK;
+}
+
+// One sorted-grid index over all n key poses (cell edge = radius, doubled by grid_setup_compute while the grid is over
+// its cap), then every call answered against it by loop_distance_batch_kernel.  The index goes to sor_setup /
+// sor_sorted / sor_cell_start, the per-call scratch of the secondary grids: the registration's local map and index are
+// not touched.  Launches do not depend on n_calls; one sync inside grid_build_core, one for the answers.  The caller
+// records ev0 before it uploads the key poses, so that liogpu_last_gpu_ms covers the whole call.
+int detect_loops_distance_dev(Ctx* c, const float4* key3d, int n, const double* h_times, const int* n_key_at,
+                              const double* time_cur, int n_calls, float radius, float time_diff, int* loop_key_pre) {
+  // ld_tab: time_cur [n_calls] f64 | key times [n] f64 | key times in index order [n] f64 | n_key_at [n_calls] i32 |
+  // answers [n_calls] i32
+  const size_t nc = (size_t)n_calls, nk = (size_t)n;
+  LIOGPU_CUDA_OK(c, c->ld_tab.reserve((nc + 2 * nk) * sizeof(double) + 2 * nc * sizeof(int)));
+  double* d_tcur = c->ld_tab.as<double>();
+  double* d_time = d_tcur + nc;
+  double* d_time_sorted = d_time + nk;
+  int* d_m = reinterpret_cast<int*>(d_time_sorted + nk);
+  int* d_out = d_m + nc;
+  LIOGPU_CUDA_OK(c, cudaMemcpyAsync(d_tcur, time_cur, nc * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+  LIOGPU_CUDA_OK(c, cudaMemcpyAsync(d_time, h_times, nk * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+  LIOGPU_CUDA_OK(c, cudaMemcpyAsync(d_m, n_key_at, nc * sizeof(int), cudaMemcpyHostToDevice, c->stream));
+  GridParams g{};
+  int rc = grid_build_core(c, key3d, n, radius, 1.0f, 1.0f, c->sor_setup, c->sor_sorted, c->sor_cell_start, g);
+  if (rc) return rc;
+  if (g.n_points <= 0) {  // no finite key pose: no call has a candidate
+    std::fill(loop_key_pre, loop_key_pre + n_calls, -1);
+    LIOGPU_CUDA_OK(c, cudaEventRecord(c->ev1, c->stream));
+    LIOGPU_CUDA_OK(c, cudaStreamSynchronize(c->stream));
+    cudaEventElapsedTime(&c->last_ms, c->ev0, c->ev1);
+    return LIOGPU_OK;
+  }
+  const float4* sorted = c->sor_sorted.as<float4>();
+  loop_time_gather_kernel<<<div_up(g.n_points, 256), 256, 0, c->stream>>>(sorted, d_time, g.n_points, d_time_sorted);
+  const float r2 = (float)((double)radius * (double)radius);  // as detect_loop_distance_dev
+  loop_distance_batch_kernel<<<div_up(n_calls, LD_WARPS), LD_WARPS * 32, 0, c->stream>>>(
+      key3d, sorted, d_time_sorted, c->sor_cell_start.as<uint32_t>(), g, d_m, d_tcur, n_calls, radius, r2,
+      (double)time_diff, d_out);
+  c->launches += 2;
+  LIOGPU_CUDA_OK(c, cudaGetLastError());
+  LIOGPU_CUDA_OK(c, cudaEventRecord(c->ev1, c->stream));
+  LIOGPU_CUDA_OK(c, cudaMemcpyAsync(loop_key_pre, d_out, nc * sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+  LIOGPU_CUDA_OK(c, cudaStreamSynchronize(c->stream));
+  cudaEventElapsedTime(&c->last_ms, c->ev0, c->ev1);
   return LIOGPU_OK;
 }
 

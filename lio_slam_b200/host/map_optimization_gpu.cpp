@@ -290,11 +290,17 @@ void mapOptimization::loopFindNearKeyframes(Cloud& nearKeyframes, int key, int s
 
 int mapOptimization::loopClosureICPBatch(const std::vector<std::pair<int, int>>& pairs,
                                          std::vector<LoopClosureOutcome>& results) {
+  return loopClosureICPBatchAt((int)cloudKeyPoses6D.size(), pairs, results);
+}
+
+int mapOptimization::loopClosureICPBatchAt(int nKey, const std::vector<std::pair<int, int>>& pairs,
+                                           std::vector<LoopClosureOutcome>& results) {
   results.assign(pairs.size(), LoopClosureOutcome{});
   std::vector<int> cur(pairs.size()), pre(pairs.size());
   for (size_t j = 0; j < pairs.size(); ++j) { cur[j] = pairs[j].first; pre[j] = pairs[j].second; }
   std::vector<float> poses;
-  for (const PointTypePose& p : cloudKeyPoses6D) {
+  for (int k = 0; k < nKey; ++k) {
+    const PointTypePose& p = cloudKeyPoses6D[k];
     const float pose6[6] = {p.roll, p.pitch, p.yaw, p.x, p.y, p.z};
     poses.insert(poses.end(), pose6, pose6 + 6);
   }
@@ -303,7 +309,7 @@ int mapOptimization::loopClosureICPBatch(const std::vector<std::pair<int, int>>&
   liogpu_default_icp_params(&ip, historyKeyframeSearchRadius);                     // :1112-1116
   // loopFindNearKeyframes(cur, 0) / (pre, historyKeyframeSearchNum) with downSizeFilterICP (:1102-1103), icp.align
   lastStatus = liogpu_loop_closure_icp_batch(ctx_, cur.data(), pre.data(), (int)pairs.size(), poses.data(),
-                                             (int)cloudKeyPoses6D.size(), historyKeyframeSearchNum,
+                                             nKey, historyKeyframeSearchNum,
                                              loopClosureICPSurfLeafSize, &ip, raw.data());
   if (lastStatus < 0) return lastStatus;
   for (size_t j = 0; j < pairs.size(); ++j) {
@@ -335,6 +341,7 @@ void mapOptimization::makeAndSaveScancontextAndKeys() {
   lastStatus = liogpu_make_scancontext(ctx_, LIOGPU_DEVICE_RESIDENT, 0, 16, 2.0, 80.0, desc, ringkey, sectorkey);
   if (lastStatus < 0) return;
   lastStatus = liogpu_sc_add(ctx_, desc, 1);
+  if (lastStatus >= 0) ++scStored_;
 }
 
 std::pair<int, float> mapOptimization::detectLoopClosureID() {
@@ -392,6 +399,89 @@ bool mapOptimization::performRSLoopClosure(int* loopKeyCur, int* loopKeyPre, flo
   if (!loopClosureICP(*loopKeyCur, *loopKeyPre, correctionLidarFrame, noiseScore)) return false;
   loopIndexContainer[*loopKeyCur] = *loopKeyPre;
   return true;
+}
+
+int mapOptimization::performLoopClosuresOffline(const std::vector<LoopTick>& ticks, std::vector<LoopTickOutcome>& outcomes,
+                                                int* icpPairs) {
+  outcomes.assign(ticks.size(), LoopTickOutcome{});
+  if (icpPairs) *icpPairs = 0;
+  const int held = (int)std::min(cloudKeyPoses3D.size(), cloudKeyPoses6D.size());
+  int nAll = 0;
+  for (const LoopTick& t : ticks) {
+    if (t.n_key < nAll || t.n_key > held) return lastStatus = LIOGPU_E_INVALID;
+    nAll = t.n_key;
+  }
+  // the ticks that have a key pose; the others return at once in both halves (:1089, :1190)
+  std::vector<int> nAt, slot(ticks.size(), -1);
+  std::vector<double> timeAt;
+  for (size_t j = 0; j < ticks.size(); ++j) {
+    if (ticks[j].n_key == 0) continue;
+    slot[j] = (int)nAt.size();
+    nAt.push_back(ticks[j].n_key);
+    timeAt.push_back(ticks[j].timeLaserInfoCur);
+  }
+  if (nAt.empty()) return lastStatus = LIOGPU_OK;
+  const int nCalls = (int)nAt.size();
+  // detectLoopClosureDistance of every tick, without the loopIndexContainer check (replayed below)
+  std::vector<int> rsPre(nCalls), scPre(nCalls);
+  lastStatus = liogpu_detect_loops_distance(ctx_, cloudKeyPoses3D.data(), nAll, sizeof(PointType), &cloudKeyPoses6D[0].time,
+                                            sizeof(PointTypePose), nAt.data(), timeAt.data(), nCalls,
+                                            historyKeyframeSearchRadius, historyKeyframeSearchTimeDiff, rsPre.data());
+  if (lastStatus < 0) return lastStatus;
+  // makeAndSaveScancontextAndKeys of the keyframes whose descriptors are not stored yet (LIDAR_HEIGHT, PC_MAX_RADIUS)
+  if (scStored_ < nAll) {
+    std::vector<int> ids;
+    for (int k = scStored_; k < nAll; ++k) ids.push_back(k);
+    lastStatus = liogpu_sc_add_keyframes(ctx_, ids.data(), (int)ids.size(), 2.0, 80.0, nullptr);
+    if (lastStatus < 0) return lastStatus;
+    scStored_ = nAll;
+  }
+  // detectLoopClosureID of every tick: the store held the tick's n_key descriptors
+  lastStatus = liogpu_sc_detect_loops(ctx_, &scParams, nAt.data(), nCalls, scPre.data(), nullptr, nullptr);
+  if (lastStatus < 0) return lastStatus;
+  // loopClosureICP of every distinct detected pair.  At tick t the window of pre is clamped to [0, n_key_t): a pair with
+  // pre + historyKeyframeSearchNum >= n_key_t needs a call at that n_key; every other pair gives the same result at the
+  // full size.  Key: (n_key of the call, cur, pre).
+  std::map<int, std::vector<std::pair<int, int>>> groups;
+  std::map<std::pair<int, std::pair<int, int>>, size_t> where;  // -> index in its group
+  auto callSize = [&](int pre, int nKey) { return (long long)pre + historyKeyframeSearchNum >= nKey ? nKey : nAll; };
+  for (int k = 0; k < nCalls; ++k)
+    for (int pre : {rsPre[k], scPre[k]}) {
+      if (pre < 0) continue;
+      const int n = callSize(pre, nAt[k]);
+      const std::pair<int, std::pair<int, int>> key(n, std::make_pair(nAt[k] - 1, pre));
+      if (where.count(key)) continue;
+      where[key] = groups[n].size();
+      groups[n].push_back(key.second);
+    }
+  std::map<int, std::vector<LoopClosureOutcome>> verdicts;
+  for (const auto& gr : groups) {
+    const int st = loopClosureICPBatchAt(gr.first, gr.second, verdicts[gr.first]);
+    if (st < 0) return st;
+    if (icpPairs) *icpPairs += (int)gr.second.size();
+  }
+  // the loop thread's bookkeeping, tick by tick: RS skips a cur that already closed a loop (:1277-1279); an accepted
+  // closure of either half is recorded (:1183, :1266)
+  auto settle = [&](LoopHalfOutcome& o, int cur, int pre, int nKey) {
+    o.loopKeyCur = cur;
+    o.loopKeyPre = pre;
+    const int n = callSize(pre, nKey);
+    const LoopClosureOutcome& v = verdicts[n][where[std::make_pair(n, std::make_pair(cur, pre))]];
+    if (!v.result.rejected_by_size) std::memcpy(o.correctionLidarFrame, v.correctionLidarFrame, sizeof(o.correctionLidarFrame));
+    o.accepted = v.accepted;
+    if (v.accepted) {
+      o.noiseScore = v.noiseScore;
+      loopIndexContainer[cur] = pre;
+    }
+  };
+  for (size_t j = 0; j < ticks.size(); ++j) {
+    const int k = slot[j];
+    if (k < 0) continue;
+    const int cur = nAt[k] - 1;
+    if (rsPre[k] >= 0 && loopIndexContainer.find(cur) == loopIndexContainer.end()) settle(outcomes[j].rs, cur, rsPre[k], nAt[k]);
+    if (scPre[k] >= 0) settle(outcomes[j].sc, cur, scPre[k], nAt[k]);
+  }
+  return lastStatus = LIOGPU_OK;
 }
 
 void mapOptimization::publishLocalMap() {  // :2442-2541; the reference calls it after every registration (:504)

@@ -150,6 +150,37 @@ class mapOptimization {
   // closure passed every guard (it is then recorded in loopIndexContainer).
   bool performSCLoopClosure(int* loopKeyCur, int* loopKeyPre, float correctionLidarFrame[16], float* noiseScore);
   bool performRSLoopClosure(int* loopKeyCur, int* loopKeyPre, float correctionLidarFrame[16], float* noiseScore);
+  // ---- offline loop closure: the loop thread's work for every tick of a recorded sequence ----
+  // A tick is one wake-up of loopClosureThread (:1050-1084) after the first n_key key poses were saved, at
+  // timeLaserInfoCur.  Its outcome is what performRSLoopClosure and then performSCLoopClosure return at that tick on a
+  // node whose cloudKeyPoses3D / 6D hold the first n_key entries: each half's pair (written only when a candidate was
+  // detected, -1 otherwise), whether the closure was accepted, the correction (written once the ICP passed the size
+  // guard, zero otherwise) and the noise score (written when accepted, zero otherwise).  A tick with n_key == 0 gives the
+  // empty outcome.  loopIndexContainer is updated in tick order exactly as the online calls would update it.
+  struct LoopTick {
+    int n_key = 0;
+    double timeLaserInfoCur = 0;
+  };
+  struct LoopHalfOutcome {
+    int loopKeyCur = -1, loopKeyPre = -1;
+    bool accepted = false;
+    float correctionLidarFrame[16] = {0};
+    float noiseScore = 0.f;
+  };
+  struct LoopTickOutcome {
+    LoopHalfOutcome rs, sc;
+  };
+  // The ticks' n_key must not decrease and may not exceed the key poses held here.  The SC half assumes a fresh Scan
+  // Context manager that holds one descriptor per keyframe, in keyframe order, and serves no other detection calls
+  // (the contract of liogpu_sc_detect_loops): descriptors this node has not stored yet (makeAndSaveScancontextAndKeys
+  // or an earlier pass) are added from the resident keyframes.  Library calls: one liogpu_detect_loops_distance, at
+  // most one liogpu_sc_add_keyframes, one liogpu_sc_detect_loops and one liogpu_loop_closure_icp_batch per distinct
+  // n_key at which a detected pair's window [pre - historyKeyframeSearchNum, pre + historyKeyframeSearchNum] is
+  // clamped (every other pair shares one call at the full size).  The ICP runs once per distinct detected pair,
+  // including pairs whose tick ends up skipping the RS half; icpPairs (may be NULL) receives that count.
+  // Returns LIOGPU_OK or the failing call's status (LIOGPU_E_INVALID for malformed ticks).
+  int performLoopClosuresOffline(const std::vector<LoopTick>& ticks, std::vector<LoopTickOutcome>& outcomes,
+                                 int* icpPairs = nullptr);
   void publishLocalMap();                                // :2442-2541 -> liogpu_publish_local_map (fills localMapCloud)
   const char* lastError() const;
   liogpu_ctx* context() { return ctx_; }
@@ -159,6 +190,10 @@ class mapOptimization {
   bool owns_ctx_ = true;
   liogpu_params params_;
   std::vector<int> mapKeyIds_;  // keyframe set the device-resident local map was built from
+  int scStored_ = 0;            // descriptors this node added to the context's Scan Context store
+  // loopClosureICPBatch on a node that held only the first nKey key poses (windows clamped to [0, nKey))
+  int loopClosureICPBatchAt(int nKey, const std::vector<std::pair<int, int>>& pairs,
+                            std::vector<LoopClosureOutcome>& results);
   std::vector<float> mapKeyPoses_;
 };
 

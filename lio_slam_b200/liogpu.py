@@ -109,7 +109,7 @@ EXPORTS = ["liogpu_abi_version", "liogpu_default_params", "liogpu_create", "liog
            "liogpu_scan2map_trace", "liogpu_voxel_tile", "liogpu_upload_scan_async", "liogpu_fetch_result",
            "liogpu_default_sc_params", "liogpu_sc_add", "liogpu_sc_clear", "liogpu_sc_detect_loop", "liogpu_sc_detect_loops",
            "liogpu_detect_loop_distance", "liogpu_loop_closure_icp_batch", "liogpu_merge_keyframes_batch",
-           "liogpu_sc_add_keyframes"]
+           "liogpu_sc_add_keyframes", "liogpu_detect_loops_distance"]
 
 RESIDENT = "resident"   # LIOGPU_DEVICE_RESIDENT: the cloud the context kept in HBM (include/liogpu.h)
 UPLOADED = "uploaded"   # LIOGPU_UPLOADED_SCAN: the sweep liogpu_upload_scan_async put on its way
@@ -176,6 +176,8 @@ def load_library() -> C.CDLL:
                                            C.c_void_p]
     lib.liogpu_detect_loop_distance.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_double,
                                                 C.c_float, C.c_float, C.POINTER(C.c_int)]
+    lib.liogpu_detect_loops_distance.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p,
+                                                 C.c_void_p, C.c_int, C.c_float, C.c_float, C.c_void_p]
     lib.liogpu_default_icp_params.argtypes = [C.POINTER(IcpParams), C.c_float]
     lib.liogpu_default_icp_params.restype = None
     lib.liogpu_icp_align.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int,
@@ -568,6 +570,22 @@ class LioGpu:
         self._check(self.lib.liogpu_detect_loop_distance(self.h, ptr, n, stride, key_time.ctypes.data, 8, C.c_double(time_cur),
                                                          C.c_float(radius), C.c_float(time_diff), C.byref(out)))
         return out.value
+
+    def detect_loops_distance(self, key3d, key_time, n_key_at, time_cur, radius: float = 10.0,
+                              time_diff: float = 30.0) -> np.ndarray:
+        """detect_loop_distance for many calls in one (liogpu_detect_loops_distance): call j on the first n_key_at[j]
+        key poses at time time_cur[j] -> loop_key_pre per call (np.int32, -1 where there is none)."""
+        ptr, n, stride, keep = _cloud_args(key3d)
+        key_time = np.ascontiguousarray(key_time, np.float64)
+        assert key_time.shape[0] == n
+        m = np.ascontiguousarray(n_key_at, np.int32).reshape(-1)
+        tc = np.ascontiguousarray(time_cur, np.float64).reshape(-1)
+        assert tc.shape == m.shape
+        out = np.full(max(m.shape[0], 1), -1, np.int32)
+        self._check(self.lib.liogpu_detect_loops_distance(self.h, ptr, n, stride, key_time.ctypes.data, 8, m.ctypes.data,
+                                                          tc.ctypes.data, m.shape[0], C.c_float(radius), C.c_float(time_diff),
+                                                          out.ctypes.data))
+        return out[: m.shape[0]].copy()
 
     def upload_scan_async(self, cloud) -> None:
         """liogpu_upload_scan_async: the buffer must stay alive until the call that consumes UPLOADED returns."""
