@@ -19,6 +19,7 @@
 // by one warp), nn_brute_block (one pass over the target) and icp_reduce_block (a pair's sums and fold), so a pair's
 // result is bit-equal whichever call computed it.
 #include "common.cuh"
+#include "pose_math.cuh"
 
 #include <stdlib.h>
 #include "shell_search.cuh"
@@ -255,56 +256,6 @@ icp_brute_kernel(const IcpArgs A) {
     const uint32_t i = A.left_list[A.ns + e];
     nn_brute_block(A.sorted, n_points, A.cur[i], max_d2, i, A.nn_idx, A.nn_d2);
   }
-}
-
-// ---- Eigen::umeyama (no scaling) from the f64 sums; same operation order as the oracle's restatement ----
-__device__ void umeyama_rotation_dev(const float sigma[9], float R[9]) {
-  double A[3][3], V[3][3] = {{1, 0, 0}, {0, 1, 0}, {0, 0, 1}};
-  for (int i = 0; i < 3; ++i)
-    for (int j = 0; j < 3; ++j) A[i][j] = (double)sigma[3 * i + j];
-  for (int sweep = 0; sweep < 60; ++sweep) {
-    bool rotated = false;
-    for (int p = 0; p < 2; ++p)
-      for (int q = p + 1; q < 3; ++q) {
-        double alpha = 0, beta = 0, gamma = 0;
-        for (int i = 0; i < 3; ++i) { alpha += A[i][p] * A[i][p]; beta += A[i][q] * A[i][q]; gamma += A[i][p] * A[i][q]; }
-        if (gamma == 0.0 || fabs(gamma) <= 1e-17 * sqrt(alpha * beta)) continue;
-        rotated = true;
-        const double zeta = (beta - alpha) / (2.0 * gamma);
-        const double t = (zeta >= 0.0 ? 1.0 : -1.0) / (fabs(zeta) + sqrt(1.0 + zeta * zeta));
-        const double c = 1.0 / sqrt(1.0 + t * t), sn = c * t;
-        for (int i = 0; i < 3; ++i) {
-          const double ap = A[i][p], aq = A[i][q];
-          A[i][p] = c * ap - sn * aq; A[i][q] = sn * ap + c * aq;
-          const double vp = V[i][p], vq = V[i][q];
-          V[i][p] = c * vp - sn * vq; V[i][q] = sn * vp + c * vq;
-        }
-      }
-    if (!rotated) break;
-  }
-  double sv[3], U[3][3];
-  for (int j = 0; j < 3; ++j) sv[j] = sqrt(A[0][j] * A[0][j] + A[1][j] * A[1][j] + A[2][j] * A[2][j]);
-  int lo = 0;
-  if (sv[1] < sv[lo]) lo = 1;
-  if (sv[2] < sv[lo]) lo = 2;
-  const int a = (lo + 1) % 3, b = (lo + 2) % 3;
-  for (int j = 0; j < 3; ++j)
-    for (int i = 0; i < 3; ++i) U[i][j] = sv[j] > 0.0 ? A[i][j] / sv[j] : 0.0;
-  if (!(sv[lo] > 1e-12 * (sv[a] > sv[b] ? sv[a] : sv[b]))) {  // rank-deficient: complete U right-handed
-    U[0][lo] = U[1][a] * U[2][b] - U[2][a] * U[1][b];
-    U[1][lo] = U[2][a] * U[0][b] - U[0][a] * U[2][b];
-    U[2][lo] = U[0][a] * U[1][b] - U[1][a] * U[0][b];
-  }
-  const double detU = U[0][0] * (U[1][1] * U[2][2] - U[1][2] * U[2][1]) - U[0][1] * (U[1][0] * U[2][2] - U[1][2] * U[2][0]) +
-                      U[0][2] * (U[1][0] * U[2][1] - U[1][1] * U[2][0]);
-  const double detV = V[0][0] * (V[1][1] * V[2][2] - V[1][2] * V[2][1]) - V[0][1] * (V[1][0] * V[2][2] - V[1][2] * V[2][0]) +
-                      V[0][2] * (V[1][0] * V[2][1] - V[1][1] * V[2][0]);
-  const double d = detU * detV < 0.0 ? -1.0 : 1.0;
-  for (int i = 0; i < 3; ++i)
-    for (int j = 0; j < 3; ++j) {
-      const double r = U[i][a] * V[j][a] + U[i][b] * V[j][b] + d * (U[i][lo] * V[j][lo]);
-      R[3 * i + j] = (float)r;
-    }
 }
 
 __device__ void icp_finalize(IcpDevState* st, const double* S) {

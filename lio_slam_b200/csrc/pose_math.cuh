@@ -209,12 +209,64 @@ __device__ __forceinline__ void jacobian_row(const LmTrig g, const float4 o, con
   rhs = -c.w;
 }
 
-// ---- OpenCV 4.x 6x6 pieces (SURVEY A.4): the solve / eigen / inverse routines live in s2m.cu ----
+// ---- OpenCV 4.x 6x6 pieces (SURVEY A.4): the solve / eigen / inverse routines live in lm_tail.cuh ----
 __device__ __forceinline__ float cv_hypotf(float a, float b) {
   a = fabsf(a); b = fabsf(b);
   if (a > b) { b /= a; return a * sqrtf(1 + b * b); }
   if (b > 0) { a /= b; return b * sqrtf(1 + a * a); }
   return 0.f;
+}
+
+// ---------------------------------------------------------------------------------------------
+// Eigen::umeyama (no scaling), the rotation of every ICP iteration (icp.cu) from the cross-covariance sigma (row-major
+// 3x3): one-sided Jacobi SVD in f64, then R = U diag(1, 1, d) V^T; same operation order as the oracle's restatement.
+__device__ __forceinline__ void umeyama_rotation_dev(const float sigma[9], float R[9]) {
+  double A[3][3], V[3][3] = {{1, 0, 0}, {0, 1, 0}, {0, 0, 1}};
+  for (int i = 0; i < 3; ++i)
+    for (int j = 0; j < 3; ++j) A[i][j] = (double)sigma[3 * i + j];
+  for (int sweep = 0; sweep < 60; ++sweep) {
+    bool rotated = false;
+    for (int p = 0; p < 2; ++p)
+      for (int q = p + 1; q < 3; ++q) {
+        double alpha = 0, beta = 0, gamma = 0;
+        for (int i = 0; i < 3; ++i) { alpha += A[i][p] * A[i][p]; beta += A[i][q] * A[i][q]; gamma += A[i][p] * A[i][q]; }
+        if (gamma == 0.0 || fabs(gamma) <= 1e-17 * sqrt(alpha * beta)) continue;
+        rotated = true;
+        const double zeta = (beta - alpha) / (2.0 * gamma);
+        const double t = (zeta >= 0.0 ? 1.0 : -1.0) / (fabs(zeta) + sqrt(1.0 + zeta * zeta));
+        const double c = 1.0 / sqrt(1.0 + t * t), sn = c * t;
+        for (int i = 0; i < 3; ++i) {
+          const double ap = A[i][p], aq = A[i][q];
+          A[i][p] = c * ap - sn * aq; A[i][q] = sn * ap + c * aq;
+          const double vp = V[i][p], vq = V[i][q];
+          V[i][p] = c * vp - sn * vq; V[i][q] = sn * vp + c * vq;
+        }
+      }
+    if (!rotated) break;
+  }
+  double sv[3], U[3][3];
+  for (int j = 0; j < 3; ++j) sv[j] = sqrt(A[0][j] * A[0][j] + A[1][j] * A[1][j] + A[2][j] * A[2][j]);
+  int lo = 0;
+  if (sv[1] < sv[lo]) lo = 1;
+  if (sv[2] < sv[lo]) lo = 2;
+  const int a = (lo + 1) % 3, b = (lo + 2) % 3;
+  for (int j = 0; j < 3; ++j)
+    for (int i = 0; i < 3; ++i) U[i][j] = sv[j] > 0.0 ? A[i][j] / sv[j] : 0.0;
+  if (!(sv[lo] > 1e-12 * (sv[a] > sv[b] ? sv[a] : sv[b]))) {  // rank-deficient: complete U right-handed
+    U[0][lo] = U[1][a] * U[2][b] - U[2][a] * U[1][b];
+    U[1][lo] = U[2][a] * U[0][b] - U[0][a] * U[2][b];
+    U[2][lo] = U[0][a] * U[1][b] - U[1][a] * U[0][b];
+  }
+  const double detU = U[0][0] * (U[1][1] * U[2][2] - U[1][2] * U[2][1]) - U[0][1] * (U[1][0] * U[2][2] - U[1][2] * U[2][0]) +
+                      U[0][2] * (U[1][0] * U[2][1] - U[1][1] * U[2][0]);
+  const double detV = V[0][0] * (V[1][1] * V[2][2] - V[1][2] * V[2][1]) - V[0][1] * (V[1][0] * V[2][2] - V[1][2] * V[2][0]) +
+                      V[0][2] * (V[1][0] * V[2][1] - V[1][1] * V[2][0]);
+  const double d = detU * detV < 0.0 ? -1.0 : 1.0;
+  for (int i = 0; i < 3; ++i)
+    for (int j = 0; j < 3; ++j) {
+      const double r = U[i][a] * V[j][a] + U[i][b] * V[j][b] + d * (U[i][lo] * V[j][lo]);
+      R[3 * i + j] = (float)r;
+    }
 }
 
 }  // namespace liogpu

@@ -1,6 +1,6 @@
 // s2m_fused.cuh — the whole loop of scan2MapOptimization (mapOptmization.cpp:1848-1859) as ONE persistent
-// cooperative launch per registration.  Included by s2m.cu (same translation unit: it reuses the search, plane-fit
-// and 6x6 routines defined there).
+// cooperative launch per registration.  Included by s2m.cu (same translation unit: it reuses the search and plane-fit
+// routines defined there and the 6x6 tail of lm_tail.cuh).
 //
 // Grid: every CTA slot of the GPU (occupancy x SM count), co-resident by cooperative launch.  CTA `gridDim.x - 1`
 // is a service CTA (iteration 0's eigen-decomposition / matP, off the critical path); the others loop:
@@ -203,28 +203,7 @@ __device__ __forceinline__ void fz_warp_transform(const int lane, const float po
 __device__ __forceinline__ void fz_matp_warp(LmDevState* st, FinSmem& m, const int lane) {
   for (int e = lane; e < 36; e += 32) m.AtA[e] = __ldcg(st->AtA0 + e);
   __syncwarp();
-  warp_eigen6(m, lane);
-  for (int e = lane; e < 36; e += 32) m.V2[e] = m.V[e];
-  __syncwarp();
-  int deg = 0;
-  if (lane == 0) {
-    for (int i = 5; i >= 0; --i) {
-      if (m.W[i] < 100.f) {
-        for (int j = 0; j < 6; ++j) m.V2[i * 6 + j] = 0.f;
-        deg = 1;
-      } else {
-        break;
-      }
-    }
-  }
-  __syncwarp();
-  warp_inv6_lu(m, lane);
-  for (int e = lane; e < 36; e += 32) {
-    const int i = e / 6, j = e % 6;
-    double acc = 0;
-    for (int k = 0; k < 6; ++k) acc += (double)m.Vi[i * 6 + k] * (double)m.V2[k * 6 + j];
-    st->matP[e] = (float)acc;
-  }
+  const int deg = lm_eigen_matp(m, lane, st->matP);
   if (lane == 0) {
     if (deg) st->cert_mismatch = 1;
     st->eig_pending = 0;

@@ -324,6 +324,16 @@ void SYM(qr53_solve)(const float* A15, const float* b5, float* x3) {
   std::memcpy(A, A15, sizeof(A));
   qr53_solve(A, b5, x3);
 }
+// surfOptimization's per-point plane fit and weight (MO:1641-1684) on given neighbours; returns the accept flag.
+int SYM(plane_residual)(const float* ori4, const float* sel4, const float* nbr20, float d2_4, float* coeff4) {
+  P4 nb[5], c;
+  std::memcpy(nb, nbr20, sizeof(nb));
+  const bool ok = plane_residual(*(const P4*)ori4, *(const P4*)sel4, nb, d2_4, c);
+  std::memcpy(coeff4, &c, sizeof(c));
+  return ok ? 1 : 0;
+}
+// Eigen::umeyama's rotation (no scaling) from the 3x3 cross-covariance, row-major.
+void SYM(umeyama_rotation)(const float* sigma9, float* R9) { umeyama_rotation(sigma9, R9); }
 
 struct s2m_result {
   int iterations, converged, n_sel, is_degenerate, tie_queries;

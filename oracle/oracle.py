@@ -283,6 +283,22 @@ class Oracle:
         self._f("qr53_solve")(_p(A, C.c_float), _p(b, C.c_float), _p(x, C.c_float))
         return x
 
+    def plane_residual(self, ori, sel, nbr, d2_4: float = 0.0):
+        """surfOptimization's plane fit for one point (MO:1641-1684) -> (flag, coeff (4,)); coeff is zero when rejected."""
+        ori = np.ascontiguousarray(ori, np.float32).reshape(4); sel = np.ascontiguousarray(sel, np.float32).reshape(4)
+        nbr = np.ascontiguousarray(nbr, np.float32).reshape(20)
+        coeff = np.zeros(4, np.float32)
+        ok = self._f("plane_residual")(_p(ori, C.c_float), _p(sel, C.c_float), _p(nbr, C.c_float), C.c_float(d2_4),
+                                       _p(coeff, C.c_float))
+        return bool(ok), coeff
+
+    def umeyama_rotation(self, sigma):
+        """Eigen::umeyama's rotation (no scaling) of the 3x3 cross-covariance sigma -> R (3,3) float32."""
+        sigma = np.ascontiguousarray(sigma, np.float32).reshape(9)
+        R = np.zeros(9, np.float32)
+        self._f("umeyama_rotation")(_p(sigma, C.c_float), _p(R, C.c_float))
+        return R.reshape(3, 3)
+
     # -- a10 ------------------------------------------------------------------------------------
     def scan2map(self, map4, scan4, pose6, matP=None, degenerate: int = 0, max_iter: int = 30, threads: int = 1,
                  handle=None, brute: bool = False):

@@ -80,3 +80,68 @@ def test_oracle_icp_max_distance_and_no_correspondences(oracle, clouds):
     r = oracle.icp_align(src, tgt, max_correspondence_distance=5.0, threads=4)
     assert r["state"] == 5 and r["converged"] == 0 and r["iterations"] == 0
     assert np.array_equal(r["T"], np.eye(4, dtype=np.float32))
+
+
+def _kabsch(sigma):
+    """R = U diag(1, 1, d) V^T of sigma = U S V^T in f64 (the rotation Eigen::umeyama returns)"""
+    U, _, Vt = np.linalg.svd(np.asarray(sigma, np.float64))
+    d = np.sign(np.linalg.det(U) * np.linalg.det(Vt))
+    return U @ np.diag([1.0, 1.0, d]) @ Vt
+
+
+def test_oracle_umeyama_rotation_equals_numpy_kabsch(oracle):
+    """the exported rotation tail of Eigen::umeyama against an f64 Kabsch solution, on cross-covariances with a
+    unique answer: proper rotations (up to 180 degrees), reflections (det < 0 -> the nearest rotation) and coplanar
+    (rank 2) clouds; 2e-6 covers the f32 input and output roundings"""
+    rng = np.random.default_rng(5)
+    worst = 0.0
+    for t in range(400):
+        q = rng.normal(size=4)
+        if t % 50 == 0:
+            q[0] = 0.0  # 180 degrees
+        q /= np.linalg.norm(q)
+        w, x, y, z = q
+        R = np.array([[1 - 2 * (y * y + z * z), 2 * (x * y - w * z), 2 * (x * z + w * y)],
+                      [2 * (x * y + w * z), 1 - 2 * (x * x + z * z), 2 * (y * z - w * x)],
+                      [2 * (x * z - w * y), 2 * (y * z + w * x), 1 - 2 * (x * x + y * y)]])
+        src = rng.normal(size=(50, 3)) * rng.uniform(0.5, 5.0, size=3)
+        if t % 4 == 1:
+            src[:, 2] = 0.0                      # coplanar source: sigma has rank 2
+        dst = src @ R.T
+        if t % 4 == 2:
+            dst[:, 0] = -dst[:, 0]               # a reflection: det(U) det(V) < 0
+        sc, dc = src - src.mean(0), dst - dst.mean(0)
+        sigma = (dc.T @ sc / len(src)).astype(np.float32)
+        want = _kabsch(sigma)
+        got = oracle.umeyama_rotation(sigma)
+        assert abs(np.linalg.det(got.astype(np.float64)) - 1.0) < 1e-5
+        if t % 4 != 2:
+            assert np.abs(want - R).max() < 1e-5, t
+        worst = max(worst, float(np.abs(got - want).max()))
+        assert np.abs(got - want).max() <= 2e-6, (t, got, want)
+    print(f"umeyama_rotation vs f64 Kabsch: max |dR| = {worst:.3g} over 400 cross-covariances")
+
+
+def test_oracle_plane_residual_export(oracle):
+    """the exported per-point plane fit: its plane is qr53_solve's, the points' residuals decide the flag, and a
+    neighbour set farther than 1 m (d2_4 >= 1) is rejected before any fit"""
+    rng = np.random.default_rng(9)
+    for t in range(200):
+        n = rng.normal(size=3); n /= np.linalg.norm(n)
+        d = rng.uniform(0.5, 20.0)
+        pts = rng.normal(size=(5, 3)) * 0.3
+        pts -= np.outer(pts @ n, n)
+        pts += (d * n) + rng.normal(size=(5, 3)) * (0.001 if t % 2 else 0.3)
+        nbr = np.concatenate([pts, np.zeros((5, 1))], 1).astype(np.float32)
+        sel = np.array([*(d * n + rng.normal(size=3) * 0.05), 0], np.float32)
+        ori = np.array([*rng.normal(size=3) * 10, 0], np.float32)
+        ok, coeff = oracle.plane_residual(ori, sel, nbr)
+        x = oracle.qr53_solve(nbr[:, :3], -np.ones(5, np.float32))
+        pn = x / np.float32(np.sqrt(np.float32(x @ x)))
+        r = np.abs(nbr[:, :3].astype(np.float64) @ pn.astype(np.float64) + 1.0 / np.linalg.norm(x.astype(np.float64)))
+        if r.max() > 0.2 + 1e-4:
+            assert not ok
+        if ok:
+            assert np.allclose(coeff[:3] / np.linalg.norm(coeff[:3]), pn, atol=1e-5)
+        far_ok, far_coeff = oracle.plane_residual(ori, sel, nbr, d2_4=1.0)
+        assert not far_ok and not far_coeff.any()
